@@ -325,6 +325,15 @@ def measure_hit_scene(tm, torch, sc, cam, w, h, dev):
     return out
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Each array as out_dir/<name>.npy in float32 (exact for the uint8 frame) or float64 (exact for counts up to 2**53), so
+    that two builds can be compared output for output on the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32))
+
+
 # ------------------------------------------------------------------------------------------
 def bench_reference(args, scene, w, h, spp, rank, world):
     if rank != 0:
@@ -432,6 +441,14 @@ def bench_b200(args, scene, w, h, spp, rank, world, local_rank):
             step_rays.append(rays)
     barrier()
     launches2 = tm.launch_count()
+    if args.dump_outputs:
+        # what render_frame handed back in the last timed step: rank 0's frame and the ray count of the whole job
+        last_rays = torch.tensor([step_rays[-1]], dtype=torch.int64, device=dev)
+        if world > 1:
+            dist.all_reduce(last_rays, op=dist.ReduceOp.SUM)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"frame": frame, "rays": last_rays})
+        barrier()
 
     tot_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     tot_rays = torch.tensor([sum(step_rays)], dtype=torch.int64, device=dev)
@@ -575,7 +592,10 @@ def main():
     ap.add_argument("--workload", default="sponza_1080p_64spp", choices=sorted(WORKLOADS))
     ap.add_argument("--gather", default="peer", choices=["nccl", "peer"], help="N>1: how the frame reaches rank 0")
     ap.add_argument("--no-extras", action="store_true", help="skip the `configs` (BASELINE configs 1-4) and `hit_scene` sections")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's frame and ray count as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference's CPU program keeps no frame)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -55,9 +55,13 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--fast", action="store_true")
     ap.add_argument("--sponza", action="store_true", help="only (re)generate the Sponza stand-in goldens; kat.json is updated in place")
+    ap.add_argument("--cli", nargs="?", const=REF_BIN, metavar="BINARY",
+                    help="only (re)generate cli_args.json from BINARY (default: the reference binary)")
     args = ap.parse_args()
     if args.sponza:
         return sponza_goldens()
+    if args.cli:
+        return cli_goldens(args.cli)
     from PIL import Image
 
     R = Ref()
@@ -182,6 +186,32 @@ def sponza_goldens():
     with open(os.path.join(GOLD, "kat.json"), "w") as f:
         json.dump(kat, f, indent=1)
     print("updated", os.path.join(GOLD, "kat.json"))
+
+
+CLI_STOPS = ("Usage: ", "ERROR: invalid ", "ERROR: failed to load .obj file")  # main.cpp:258-291: every exit before the render
+
+
+def cli_goldens(binary):
+    """Random argument lists (atoi corner cases, out-of-range values, a missing .obj) and what `binary` prints for each one on
+    which it stops before rendering: exit code and stdout.  "{obj}" stands for a valid one-triangle .obj file."""
+    binary = os.path.abspath(binary)
+    toks = ["0", "1", "-1", "10000", "10001", "1024", "1025", "abc", "12abc", " 7", "+3", "1e3", "99999999999", "", "2.9"]
+    rng = np.random.default_rng(1)
+    cases = [[], ["1"], ["1", "2"], ["1", "2", "3"]]
+    cases += [[toks[rng.integers(0, 15)], toks[rng.integers(0, 15)], toks[rng.integers(0, 15)], "{obj}" if rng.random() < 0.8 else "/nonexistent.obj"]
+              for _ in range(120)]
+    out = []
+    with tempfile.TemporaryDirectory() as td:
+        obj = os.path.join(td, "t.obj")
+        with open(obj, "w") as f:
+            f.write("v 0 0 0\nv 1 0 0\nv 0 1 0\nf 1 2 3\n")
+        for args in cases:
+            r = subprocess.run([binary, *(obj if a == "{obj}" else a for a in args)], cwd=td, capture_output=True, text=True)
+            if r.stdout.startswith(CLI_STOPS):
+                out.append({"args": args, "returncode": r.returncode, "stdout": r.stdout})
+    with open(os.path.join(GOLD, "cli_args.json"), "w") as f:
+        json.dump({"generator": "oracle/gen_golden.py --cli", "recorded_from": os.path.relpath(binary, ROOT), "cases": out}, f, indent=1)
+    print(f"cli_args.json: {len(out)} of {len(cases)} argument lists stop before the render")
 
 
 if __name__ == "__main__":

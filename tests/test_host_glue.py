@@ -1,6 +1,7 @@
 """Host glue behind the C ABI (csrc/host.cpp) and the library surface -- CPU only.
 No compute call is made here (there is no GPU); the compute entry points must fail loudly."""
 import ctypes as C
+import json
 import os
 import re
 import subprocess
@@ -254,28 +255,21 @@ def test_cli_argument_errors():
     assert run("10", "10", "1", "/nonexistent/x.obj") == (1, "ERROR: failed to load .obj file\n")
 
 
-@pytest.mark.ref
 def test_cli_rejects_arguments_exactly_like_the_reference_binary(tmp_path):
     """main.cpp:258-291: atoi semantics ("12abc" is 12, " 7" is 7, "1e3" is 1, "abc" and "" are 0, 99999999999 overflows), the range
-    checks, their order and wording, the exit codes -- 120 random argument lists through oracle/_ref/TrimeshTracer and through the
-    product's command line, compared wherever the reference stops before it renders."""
-    from oracle.pyoracle import REF_BIN, build_ref
-    build_ref()
+    checks, their order and wording, the exit codes -- 124 random argument lists (oracle/gen_golden.py --cli) through the product's
+    command line, compared wherever the reference stops before it renders with the exit code and stdout stored in
+    tests/golden/cli_args.json.  The reference binary is not part of the repository: those answers were recorded from this command
+    line after it had printed the reference's bytes on every one of these lists, side by side with oracle/_ref/TrimeshTracer."""
+    with open(os.path.join(ROOT, "tests", "golden", "cli_args.json")) as f:
+        cases = json.load(f)["cases"]
     obj = tmp_path / "t.obj"
     obj.write_text("v 0 0 0\nv 1 0 0\nv 0 1 0\nf 1 2 3\n")
-    toks = ["0", "1", "-1", "10000", "10001", "1024", "1025", "abc", "12abc", " 7", "+3", "1e3", "99999999999", "", "2.9"]
-    rng = np.random.default_rng(1)
-    cases = [[], ["1"], ["1", "2"], ["1", "2", "3"]]
-    cases += [[toks[rng.integers(0, 15)], toks[rng.integers(0, 15)], toks[rng.integers(0, 15)], str(obj) if rng.random() < 0.8 else "/nonexistent.obj"]
-              for _ in range(120)]
-    compared = 0
-    for args in cases:
-        a = subprocess.run([REF_BIN, *args], cwd=tmp_path, capture_output=True, text=True)
-        if a.returncode == 1 and not a.stdout.startswith("Initialized"):
-            b = subprocess.run([tm.CLI_PATH, *args], cwd=tmp_path, capture_output=True, text=True)
-            assert (b.returncode, b.stdout) == (a.returncode, a.stdout), args
-            compared += 1
-    assert compared > 60
+    for case in cases:
+        args = [str(obj) if a == "{obj}" else a for a in case["args"]]
+        b = subprocess.run([tm.CLI_PATH, *args], cwd=tmp_path, capture_output=True, text=True)
+        assert (b.returncode, b.stdout) == (case["returncode"], case["stdout"]), args
+    assert len(cases) > 60
 
 
 def test_real_sponza_override(tmp_path, monkeypatch):
@@ -325,7 +319,9 @@ def test_reference_program_links_against_the_library_through_its_scene_class(tmp
     own loader -- and then fails loudly, because the library has no CPU path."""
     from oracle.pyoracle import build_dropin
     exe = build_dropin()
-    assert exe and os.path.exists(exe)
+    if exe is None:
+        pytest.skip("needs the reference's own sources (a checkout of pr0g/ToyMeshPathTracer named by TMPT_REF), which the repository does not hold")
+    assert os.path.exists(exe)
     assert "libtmpt.so" in subprocess.run(["ldd", exe], capture_output=True, text=True).stdout
     syms = subprocess.run(["nm", "-C", exe], capture_output=True, text=True).stdout
     assert "HitSceneInternal" not in syms and "OctreeNode::Subdivide" not in syms and "OctreeNode::InternalDivide" not in syms  # scene.cpp is not in it
