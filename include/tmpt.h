@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define TMPT_ABI_VERSION 2
+#define TMPT_ABI_VERSION 3
 
 typedef enum tmpt_status {
     TMPT_OK = 0,
@@ -131,6 +131,31 @@ int tmpt_hit_scene(const tmpt_scene* scene, const float* rays6, int64_t nRays, f
 int tmpt_render(const tmpt_scene* scene, const tmpt_camera* camera, int width, int height, int spp,
                 int mem, uint8_t* rgba, uint64_t* rayCount, double* seconds, void* stream);
 
+/* Beyond the reference: the linear radiance and first-hit AOVs ("arbitrary output variables") of a frame, for denoisers,
+ * tone mapping, compositing and picking.  Each pointer may be NULL (not produced); at least one must be set.  All buffers
+ * are [height][width] with row 0 = bottom (as tmpt_render's rgba), in the memory space `mem` names. */
+typedef struct tmpt_outputs {
+    uint8_t* rgba;      /* width*height*4 bytes: tmpt_render's frame, byte for byte                                        */
+    float* radiance;    /* width*height*4: the linear per-pixel mean BEFORE sqrt / quantise, sum * (1/spp); A = 1.0f        */
+    float* normal;      /* width*height*4: xyz = sum over the samples of the camera ray's first-hit geometric normal (as
+                           tmpt_hit_scene's outNormal3) * (1/spp); w = hits * (1/spp), the coverage.  Albedo is 0.7 at
+                           every hit (main.cpp:48), so 0.7 * w is the albedo AOV                                            */
+    float* depth;       /* width*height: sum of the first-hit t / hits (IEEE division); +INFINITY where no sample hit        */
+    int32_t* triangle;  /* width*height: ORIGINAL index of the triangle that sample 0's camera ray hits, -1 for the sky     */
+} tmpt_outputs;
+
+/* One frame of tmpt_render with the outputs `out` names.  The paths do not change: RNG streams, rays, rayCount and rgba
+ * are those of tmpt_render with the same arguments; the AOVs are recorded from the camera rays the integrator traces
+ * anyway.  Summation order (what makes every buffer bit-exact against a serial restatement): inside a chunk the colour and
+ * the AOV sums run in sample order from +0.0f, a sample whose camera ray misses adds nothing to the AOV sums; the chunk
+ * sums are then added in chunk order from +0.0f; the divisions by spp are multiplications by the float 1/spp.  NaN stays
+ * NaN: `radiance` keeps a NaN the reference arithmetic makes (such pixels are 0 in rgba); nothing is sanitised.
+ * TMPT_HOST: each requested buffer is staged in device scratch owned by the scene; `seconds` covers the kernels and every
+ * device-to-host copy.  Errors: TMPT_ERR_ARG for a NULL `out`, no buffer requested, a bad `mem`, or the range checks of
+ * tmpt_render.  Single GPU. */
+int tmpt_render_outputs(const tmpt_scene* scene, const tmpt_camera* camera, int width, int height, int spp, int mem,
+                        const tmpt_outputs* out, uint64_t* rayCount, double* seconds, void* stream);
+
 /* Progressive rendering (beyond the reference, SURVEY.md 8(f) rank 4): the frame converges over calls.
  * tmpt_progressive_begin fixes the frame size and clears the running per-pixel sums kept with the scene; every
  * tmpt_progressive_pass traces `nChunks` (1..128) more chunks of 8 samples per pixel with the SAME camera, adds them to
@@ -141,6 +166,11 @@ int tmpt_render(const tmpt_scene* scene, const tmpt_camera* camera, int width, i
 int tmpt_progressive_begin(tmpt_scene* scene, int width, int height);
 int tmpt_progressive_pass(tmpt_scene* scene, const tmpt_camera* camera, int nChunks, int mem, uint8_t* rgba,
                           uint64_t* rayCount, double* seconds, int* samplesSoFar, void* stream);
+/* A pass with tmpt_outputs: rgba and radiance only, both the mean over all samples so far (after P >= 32 chunks in total,
+ * radiance equals tmpt_render_outputs' at spp = 8 * P bit for bit).  A normal, depth or triangle pointer is TMPT_ERR_ARG:
+ * passes keep no running AOV sums. */
+int tmpt_progressive_pass_outputs(tmpt_scene* scene, const tmpt_camera* camera, int nChunks, int mem, const tmpt_outputs* out,
+                                  uint64_t* rayCount, double* seconds, int* samplesSoFar, void* stream);
 
 /* Multi-GPU form: this rank renders only its share of the frame and writes it packed into
  * outStripes (device memory on the scene's device, tmpt_stripe_rows(...) *

@@ -8,6 +8,7 @@ drive it through; it mirrors the reference's own interface names:
     Scene(tris)                      Scene::Scene + BuildOctree      (scene.h:19, 26)
     Scene.HitScene(rays, tMin, tMax) Scene::HitScene, batched        (scene.h:36-37)
     Scene.render(camera, w, h, spp)  TraceImageBody over all rows    (main.cpp:180-246, 329-331)
+    Scene.render_outputs(...)        the same frame plus linear radiance and first-hit AOVs (beyond the reference)
     load_scene(path)                 LoadScene                       (main.cpp:122-170)
     camera_for_scene(...)            camera placement of main()      (main.cpp:296-307)
 
@@ -39,6 +40,7 @@ ABI_SYMBOLS = [
     "tmpt_device_count", "tmpt_launch_count", "tmpt_render_stats", "tmpt_hit_scene_stats",
     "tmpt_frame_alloc", "tmpt_frame_open", "tmpt_frame_close", "tmpt_frame_free", "tmpt_render_multi",
     "tmpt_scene_refit", "tmpt_progressive_begin", "tmpt_progressive_pass", "tmpt_render_kernel_choice",
+    "tmpt_render_outputs", "tmpt_progressive_pass_outputs",
 ]
 
 
@@ -46,6 +48,25 @@ class TmptError(RuntimeError):
     def __init__(self, status, message):
         super().__init__(f"tmpt status {status}: {message}")
         self.status = status
+
+
+OUTPUTS = ("rgba", "radiance", "normal", "depth", "triangle")  # the members of tmpt_outputs, in order
+
+
+class Outputs(C.Structure):
+    """tmpt_outputs: one pointer per buffer, NULL = not produced."""
+    _fields_ = [(name, C.c_void_p) for name in OUTPUTS]
+
+
+def _output_arrays(names, width: int, height: int) -> dict:
+    """Host arrays for the named outputs: rgba [h,w,4] uint8, radiance / normal [h,w,4] float32, depth [h,w] float32,
+    triangle [h,w] int32."""
+    unknown = set(names) - set(OUTPUTS)
+    if unknown:
+        raise ValueError(f"unknown outputs {sorted(unknown)}; choose from {OUTPUTS}")
+    shapes = {"rgba": ((height, width, 4), np.uint8), "radiance": ((height, width, 4), np.float32),
+              "normal": ((height, width, 4), np.float32), "depth": ((height, width), np.float32), "triangle": ((height, width), np.int32)}
+    return {n: np.zeros(*shapes[n]) for n in OUTPUTS if n in names}
 
 
 class SceneInfo(C.Structure):
@@ -86,6 +107,9 @@ def lib() -> C.CDLL:
     L.tmpt_scene_refit.argtypes = [vp, vp, i32, C.POINTER(C.c_double)]
     L.tmpt_hit_scene.argtypes = [vp, vp, i64, f32, f32, i32, i32, vp, vp, vp, vp, vp]
     L.tmpt_render.argtypes = [vp, vp, i32, i32, i32, i32, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
+    L.tmpt_render_outputs.argtypes = [vp, vp, i32, i32, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
+    L.tmpt_progressive_pass_outputs.argtypes = [vp, vp, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double),
+                                                C.POINTER(i32), vp]
     L.tmpt_progressive_begin.argtypes = [vp, i32, i32]
     L.tmpt_progressive_pass.argtypes = [vp, vp, i32, i32, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double), C.POINTER(i32), vp]
     L.tmpt_render_stripes.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]
@@ -274,6 +298,27 @@ class Scene:
         _check(lib().tmpt_render(self._h, _ptr(cam), width, height, spp, HOST, _ptr(rgba), C.byref(rays), C.byref(sec), None))
         return rgba, rays.value, sec.value
 
+    def render_outputs(self, camera, width: int, height: int, spp: int, outputs=OUTPUTS):
+        """One frame with the named outputs (tmpt_render_outputs) -> ({name: host array}, rayCount, seconds).  rgba is
+        render()'s frame; radiance the linear mean before sqrt / quantise; normal / depth / triangle the camera rays' first
+        hits (include/tmpt.h)."""
+        cam = _f32(camera).reshape(22)
+        arrays = _output_arrays(outputs, width, height)
+        out = Outputs(**{n: a.ctypes.data for n, a in arrays.items()})
+        rays, sec = C.c_uint64(0), C.c_double(0.0)
+        _check(lib().tmpt_render_outputs(self._h, _ptr(cam), width, height, spp, HOST, C.byref(out), C.byref(rays), C.byref(sec), None))
+        return arrays, rays.value, sec.value
+
+    def render_outputs_device(self, camera, width: int, height: int, spp: int, rgba_ptr: int = 0, radiance_ptr: int = 0,
+                              normal_ptr: int = 0, depth_ptr: int = 0, triangle_ptr: int = 0, stream: int = 0):
+        """tmpt_render_outputs into device buffers (raw addresses, e.g. torch ``data_ptr()``; 0 = not produced) -> (rayCount, seconds)."""
+        cam = _f32(camera).reshape(22)
+        out = Outputs(rgba_ptr or None, radiance_ptr or None, normal_ptr or None, depth_ptr or None, triangle_ptr or None)
+        rays, sec = C.c_uint64(0), C.c_double(0.0)
+        _check(lib().tmpt_render_outputs(self._h, _ptr(cam), width, height, spp, DEVICE, C.byref(out), C.byref(rays), C.byref(sec),
+                                         stream or None))
+        return rays.value, sec.value
+
     def progressive_begin(self, width: int, height: int):
         """Start (or restart) a progressive render of a width x height frame (tmpt_progressive_begin)."""
         _check(lib().tmpt_progressive_begin(self._h, width, height))
@@ -287,6 +332,18 @@ class Scene:
         rays, sec, spp = C.c_uint64(0), C.c_double(0.0), C.c_int32(0)
         _check(lib().tmpt_progressive_pass(self._h, _ptr(cam), n_chunks, HOST, _ptr(rgba), C.byref(rays), C.byref(sec), C.byref(spp), None))
         return rgba, rays.value, sec.value, spp.value
+
+    def progressive_pass_outputs(self, camera, n_chunks: int = 1, radiance: bool = True):
+        """A progressive pass that also returns the linear mean so far -> ({"rgba", "radiance"}, rays of this pass, seconds,
+        samples so far)."""
+        width, height = self._prog
+        cam = _f32(camera).reshape(22)
+        arrays = _output_arrays(("rgba", "radiance") if radiance else ("rgba",), width, height)
+        out = Outputs(**{n: a.ctypes.data for n, a in arrays.items()})
+        rays, sec, spp = C.c_uint64(0), C.c_double(0.0), C.c_int32(0)
+        _check(lib().tmpt_progressive_pass_outputs(self._h, _ptr(cam), n_chunks, HOST, C.byref(out), C.byref(rays), C.byref(sec),
+                                                   C.byref(spp), None))
+        return arrays, rays.value, sec.value, spp.value
 
     def render_into(self, camera, width: int, height: int, spp: int, host_ptr: int):
         """One frame into caller-owned HOST memory (w*h*4 bytes, e.g. a pinned buffer) -> (rayCount, seconds): tmpt_render as a

@@ -78,21 +78,31 @@ TMPT_HD uchar4 resolve_pixel(ex::V3 sum, float sppRecip) {
     return px;
 }
 
+// What the camera ray of one sample hit (AOV = true): the depth-0 HitScene answer.  id = -1 for the sky; t / normal are
+// valid for hits only (normal = hit_payload's geometric normal, as tmpt_hit_scene reports it).
+struct FirstHit {
+    int id;
+    float t;
+    ex::V3 normal;
+};
+
 // One whole pixel, serially: the straightforward form used by the host emulation and by the
 // first (non-wavefront) render kernel.  kk[] holds the per-bounce sun term (0 for a
-// shadowed bounce).
-template <bool STATS = false, bool FAR = true, class Stack, class Scene>
+// shadowed bounce).  AOV: `first` receives the camera ray's hit; the path is the same.
+template <bool STATS = false, bool FAR = true, bool AOV = false, class Stack, class Scene>
 TMPT_HD ex::V3 trace_path(Stack& stack, const Scene& sc, const Camera& cam, ex::V3 o, ex::V3 d, ex::V3 lightDir, uint32_t& rng,
-                          unsigned long long& rays, bvh::TravStats* stats = nullptr) {
+                          unsigned long long& rays, bvh::TravStats* stats = nullptr, FirstHit* first = nullptr) {
     float kk[kMaxDepth];
     int depth = 0;
     ex::V3 color = ex::v3(0.0f, 0.0f, 0.0f);
+    if (AOV) first->id = -1;
     while (depth < kMaxDepth) {
         ++rays;
         const bvh::HitRec h = bvh::traverse_with<false, STATS, FAR>(stack, sc, o, d, kMinT, kMaxT, stats);
         if (h.id < 0) { color = sky(d); break; }
         ex::V3 pos, normal;
         bvh::hit_payload(sc, h.id, h.u, h.v, pos, normal);
+        if (AOV && depth == 0) { first->id = h.id; first->t = h.t; first->normal = normal; }
         ++rays;
         // the shadow ray (main.cpp:59): through the sun grid when the scene has one (sungrid.cuh), else through the tree
 #if defined(TMPT_SUN_ONLY) && TMPT_SUN_ONLY  // (experiment: what the tree fallback in the same kernel costs)
@@ -126,30 +136,68 @@ TMPT_HD int chunk_len(int spp) {
 }
 TMPT_HD int chunk_count(int spp) { const int c = chunk_len(spp); return (spp + c - 1) / c; }
 
+// AOV sums of one chunk or pixel (AOV = true), each from +0 in sample order, chunk sums added in chunk order like the colour:
+// over the samples whose camera ray hits, the hit count, the sum of their normals and of their t.  id0 = the camera-ray hit of
+// the first sample (tmpt_outputs.triangle reports chunk 0's).
+struct AovSums {
+    ex::V3 normal;
+    float t, hits;
+    int id0;
+};
+TMPT_HD void aov_clear(AovSums& a) { a.normal = ex::v3(0.0f, 0.0f, 0.0f); a.t = 0.0f; a.hits = 0.0f; a.id0 = -1; }
+TMPT_HD void aov_add_hit(AovSums& a, ex::V3 normal, float t) { a.normal = ex::add(a.normal, normal); a.t = ex::add(a.t, t); a.hits = ex::add(a.hits, 1.0f); }
+
+// The float outputs of a pixel (include/tmpt.h, tmpt_outputs) from its sums: radiance = colour sum * (1/spp) with A = 1 (the
+// value resolve_pixel takes the square root of), normal = (normal sum, hit count) * (1/spp), depth = t sum / hit count, +inf
+// where no camera ray hit.  NaN stays NaN.
+TMPT_HD float4 radiance_of(ex::V3 sum, float sppRecip) {
+    const ex::V3 c = ex::muls(sum, sppRecip);
+    return make_float4(c.x, c.y, c.z, 1.0f);
+}
+TMPT_HD float4 normal_of(ex::V3 normalSum, float hits, float sppRecip) {
+    const ex::V3 n = ex::muls(normalSum, sppRecip);
+    return make_float4(n.x, n.y, n.z, ex::mul(hits, sppRecip));
+}
+TMPT_HD float depth_of(float tSum, float hits) { return hits > 0.0f ? ex::divf(tSum, hits) : ex::u2f(0x7F800000u); }
+
 // `len` = samples per chunk: chunk_len(spp) for a one-shot frame, kMaxChunkSamples for a progressive pass
-template <bool STATS = false, bool FAR = true, class Stack, class Scene>
+template <bool STATS = false, bool FAR = true, bool AOV = false, class Stack, class Scene>
 TMPT_HD ex::V3 render_chunk(Stack& stack, const Scene& sc, const Camera& cam, int x, int y, int chunk, int width, int height, int spp, int len, ex::V3 lightDir,
-                            unsigned long long& rays, bvh::TravStats* stats = nullptr) {
+                            unsigned long long& rays, bvh::TravStats* stats = nullptr, AovSums* aov = nullptr) {
     const float invW = ex::divf(1.0f, (float)width), invH = ex::divf(1.0f, (float)height);
     uint32_t rng = ex::chunk_seed((uint32_t)chunk, (uint32_t)y * (uint32_t)width + (uint32_t)x, (uint32_t)width * (uint32_t)height);
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f);
     const int s0 = chunk * len, s1 = s0 + len < spp ? s0 + len : spp;
+    if (AOV) aov_clear(*aov);
     for (int s = s0; s < s1; ++s) {
         ex::V3 o, d;
         primary_ray(cam, x, y, invW, invH, rng, o, d);
-        sum = ex::add(sum, trace_path<STATS, FAR>(stack, sc, cam, o, d, lightDir, rng, rays, stats));
+        FirstHit fh;
+        sum = ex::add(sum, trace_path<STATS, FAR, AOV>(stack, sc, cam, o, d, lightDir, rng, rays, stats, &fh));
+        if (AOV) {
+            if (s == s0) aov->id0 = fh.id;
+            if (fh.id >= 0) aov_add_hit(*aov, fh.normal, fh.t);
+        }
     }
     return sum;
 }
 
-// One whole pixel, serially (host emulation; the kernels spread the chunks over lanes).
-template <bool STATS = false, class Scene>
+// One whole pixel, serially (host emulation; the kernels spread the chunks over lanes).  AOV: `aov` receives the pixel's sums.
+template <bool STATS = false, bool AOV = false, class Scene>
 TMPT_HD uchar4 render_pixel(const Scene& sc, const Camera& cam, int x, int y, int width, int height, int spp, ex::V3 lightDir,
-                            unsigned long long& rays, ex::V3* outLinear = nullptr, bvh::TravStats* stats = nullptr) {
+                            unsigned long long& rays, ex::V3* outLinear = nullptr, bvh::TravStats* stats = nullptr, AovSums* aov = nullptr) {
     const float sppRecip = ex::divf(1.0f, (float)spp);
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f);
     bvh::LocalStack stack;
-    for (int c = 0; c < chunk_count(spp); ++c) sum = ex::add(sum, render_chunk<STATS>(stack, sc, cam, x, y, c, width, height, spp, chunk_len(spp), lightDir, rays, stats));
+    if (AOV) aov_clear(*aov);
+    for (int c = 0; c < chunk_count(spp); ++c) {
+        AovSums ca;
+        sum = ex::add(sum, render_chunk<STATS, true, AOV>(stack, sc, cam, x, y, c, width, height, spp, chunk_len(spp), lightDir, rays, stats, &ca));
+        if (AOV) {
+            if (c == 0) aov->id0 = ca.id0;
+            aov->normal = ex::add(aov->normal, ca.normal); aov->t = ex::add(aov->t, ca.t); aov->hits = ex::add(aov->hits, ca.hits);
+        }
+    }
     if (outLinear) *outLinear = ex::muls(sum, sppRecip);
     return resolve_pixel(sum, sppRecip);
 }
