@@ -172,6 +172,40 @@ int tmpt_progressive_pass(tmpt_scene* scene, const tmpt_camera* camera, int nChu
 int tmpt_progressive_pass_outputs(tmpt_scene* scene, const tmpt_camera* camera, int nChunks, int mem, const tmpt_outputs* out,
                                   uint64_t* rayCount, double* seconds, int* samplesSoFar, void* stream);
 
+/* Adaptive progressive passes (beyond the reference): a pass traces only the pixels whose estimated error is still above a
+ * tolerance.  A session (tmpt_progressive_begin, which also clears the adaptive state) becomes uniform or adaptive with its
+ * first pass; a uniform pass in an adaptive session, or an adaptive pass in a uniform one, is TMPT_ERR_ARG.
+ * Per pixel the session keeps n (chunks so far), the colour sum and a Welford mean and M2 of the chunk-mean luminance.  For
+ * each new chunk sum S, in chunk order, with one rounding per float operation and no contraction:
+ *     Y = ((0.2126f*S.x + 0.7152f*S.y) + 0.0722f*S.z) * 0.125f;   n = n + 1;   delta = Y - mean;
+ *     mean = mean + delta / (float)n;   M2 = M2 + delta * (Y - mean)
+ * Stop rule -- the standard error of the mean luminance, taken through the sqrt display curve, in 8-bit codes, at most
+ * `tolerance` -- written without sqrt or division:
+ *     a = M2 * 65025.0f;   b = (((float)n * (float)(n - 1)) * (4.0f * fmaxf(mean, 0x1p-16f))) * (tolerance * tolerance)
+ *     converged = tolerance != 0 && n >= minChunks && !(a > b)
+ * A pixel whose state became NaN is therefore converged once n >= minChunks (more samples cannot remove a NaN from a sum).
+ * A pass: every pixel not converged under this pass's params traces exactly nChunks more 8-sample chunks, chunk indices
+ * n .. n + nChunks - 1, and updates its state as above; converged pixels are not traced.  Chunk c of a pixel is the stream a
+ * uniform pass traces as that pixel's chunk c, so every pixel equals, bit for bit in rgba and radiance, the same pixel of a
+ * uniform session after n of its chunks (and tmpt_render_outputs at spp = 8 n once n >= 32); with tolerance 0 a pass equals
+ * tmpt_progressive_pass_outputs with the same nChunks in bytes, radiance and rayCount.
+ *   out          rgba and / or radiance (other pointers: TMPT_ERR_ARG), written for the whole frame: sum * (1 / (8 n))
+ *   samples      (may be NULL) width*height int32: 8 n per pixel
+ *   rayCount     the rays traced in this pass only
+ *   activePixels (may be NULL) pixels not converged under this pass's params after the pass: 0 = the next identical pass
+ *                traces nothing
+ *   seconds      device time of select, compaction, render, resolve and copies
+ * Errors (TMPT_ERR_ARG, with a message): nChunks outside 1..128, a NULL params, a negative, NaN or infinite tolerance,
+ * minChunks outside 2..2^21, and the limits of tmpt_progressive_pass_outputs (8 x the session's most chunks of a pixel at
+ * most 2^24).  Single GPU. */
+typedef struct tmpt_adaptive {
+    float tolerance;   /* 8-bit display codes; 0 = adaptivity off (every pixel is traced) */
+    int32_t minChunks; /* no pixel stops before it has this many chunks; 2 .. 2^21 */
+} tmpt_adaptive;
+int tmpt_progressive_pass_adaptive(tmpt_scene* scene, const tmpt_camera* camera, int nChunks, const tmpt_adaptive* params, int mem,
+                                   const tmpt_outputs* out, int32_t* samples, uint64_t* rayCount, double* seconds,
+                                   int64_t* activePixels, void* stream);
+
 /* Multi-GPU form: this rank renders only its share of the frame and writes it packed into
  * outStripes (device memory on the scene's device, tmpt_stripe_rows(...) *
  * tmpt_local_width(...) * 4 bytes).  Two partitions:

@@ -40,7 +40,7 @@ ABI_SYMBOLS = [
     "tmpt_device_count", "tmpt_launch_count", "tmpt_render_stats", "tmpt_hit_scene_stats",
     "tmpt_frame_alloc", "tmpt_frame_open", "tmpt_frame_close", "tmpt_frame_free", "tmpt_render_multi",
     "tmpt_scene_refit", "tmpt_progressive_begin", "tmpt_progressive_pass", "tmpt_render_kernel_choice",
-    "tmpt_render_outputs", "tmpt_progressive_pass_outputs",
+    "tmpt_render_outputs", "tmpt_progressive_pass_outputs", "tmpt_progressive_pass_adaptive",
 ]
 
 
@@ -67,6 +67,11 @@ def _output_arrays(names, width: int, height: int) -> dict:
     shapes = {"rgba": ((height, width, 4), np.uint8), "radiance": ((height, width, 4), np.float32),
               "normal": ((height, width, 4), np.float32), "depth": ((height, width), np.float32), "triangle": ((height, width), np.int32)}
     return {n: np.zeros(*shapes[n]) for n in OUTPUTS if n in names}
+
+
+class Adaptive(C.Structure):
+    """tmpt_adaptive: the stop rule of an adaptive progressive pass."""
+    _fields_ = [("tolerance", C.c_float), ("minChunks", C.c_int32)]
 
 
 class SceneInfo(C.Structure):
@@ -110,6 +115,8 @@ def lib() -> C.CDLL:
     L.tmpt_render_outputs.argtypes = [vp, vp, i32, i32, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
     L.tmpt_progressive_pass_outputs.argtypes = [vp, vp, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double),
                                                 C.POINTER(i32), vp]
+    L.tmpt_progressive_pass_adaptive.argtypes = [vp, vp, i32, C.POINTER(Adaptive), i32, C.POINTER(Outputs), vp, C.POINTER(C.c_uint64),
+                                                 C.POINTER(C.c_double), C.POINTER(i64), vp]
     L.tmpt_progressive_begin.argtypes = [vp, i32, i32]
     L.tmpt_progressive_pass.argtypes = [vp, vp, i32, i32, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double), C.POINTER(i32), vp]
     L.tmpt_render_stripes.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]
@@ -344,6 +351,21 @@ class Scene:
         _check(lib().tmpt_progressive_pass_outputs(self._h, _ptr(cam), n_chunks, HOST, C.byref(out), C.byref(rays), C.byref(sec),
                                                    C.byref(spp), None))
         return arrays, rays.value, sec.value, spp.value
+
+    def progressive_pass_adaptive(self, camera, n_chunks: int = 1, tolerance: float = 0.5, min_chunks: int = 4, radiance: bool = True):
+        """An adaptive progressive pass (tmpt_progressive_pass_adaptive): only pixels whose estimated error is above `tolerance`
+        8-bit codes trace n_chunks more chunks -> ({"rgba", ["radiance"], "samples"}, rays of this pass, seconds, pixels still
+        active after the pass)."""
+        width, height = self._prog
+        cam = _f32(camera).reshape(22)
+        arrays = _output_arrays(("rgba", "radiance") if radiance else ("rgba",), width, height)
+        out = Outputs(**{n: a.ctypes.data for n, a in arrays.items()})
+        arrays["samples"] = np.zeros((height, width), np.int32)
+        params = Adaptive(tolerance, min_chunks)
+        rays, sec, active = C.c_uint64(0), C.c_double(0.0), C.c_int64(0)
+        _check(lib().tmpt_progressive_pass_adaptive(self._h, _ptr(cam), n_chunks, C.byref(params), HOST, C.byref(out),
+                                                    _ptr(arrays["samples"]), C.byref(rays), C.byref(sec), C.byref(active), None))
+        return arrays, rays.value, sec.value, active.value
 
     def render_into(self, camera, width: int, height: int, spp: int, host_ptr: int):
         """One frame into caller-owned HOST memory (w*h*4 bytes, e.g. a pinned buffer) -> (rayCount, seconds): tmpt_render as a

@@ -182,6 +182,26 @@ TMPT_HD ex::V3 render_chunk(Stack& stack, const Scene& sc, const Camera& cam, in
     return sum;
 }
 
+// Adaptive progressive passes (include/tmpt.h, tmpt_progressive_pass_adaptive): a pixel's chunk count n and the Welford mean / M2
+// of its chunk-mean luminance, updated per chunk sum in chunk order.  One rounding per operation, no contraction.
+TMPT_HD void adaptive_add_chunk(ex::V3 chunkSum, uint32_t& n, float& mean, float& m2) {
+    const float y = ex::mul(ex::add(ex::add(ex::mul(0.2126f, chunkSum.x), ex::mul(0.7152f, chunkSum.y)), ex::mul(0.0722f, chunkSum.z)), 0.125f);
+    n += 1u;
+    const float delta = ex::sub(y, mean);
+    mean = ex::add(mean, ex::divf(delta, (float)n));
+    m2 = ex::add(m2, ex::mul(delta, ex::sub(y, mean)));
+}
+// The stop rule: the standard error of the mean luminance, through the sqrt display curve, in 8-bit codes, is at most
+// `tolerance` -- se = sqrt(M2 / (n (n-1))), codes = 255 * se / (2 sqrt(mean)) -- squared and multiplied out (no sqrt, no division).
+// NaN state compares false, so such a pixel stops at minChunks.  Tolerance 0 stops nothing: the explicit test keeps a pixel with
+// M2 = 0 (then a = b = 0) tracing.
+TMPT_HD bool adaptive_converged(uint32_t n, float mean, float m2, float tolerance, int minChunks) {
+    if (tolerance == 0.0f || n < (uint32_t)minChunks) return false;
+    const float a = ex::mul(m2, 65025.0f);
+    const float b = ex::mul(ex::mul(ex::mul((float)n, (float)(n - 1u)), ex::mul(4.0f, fmaxf(mean, 0x1p-16f))), ex::mul(tolerance, tolerance));
+    return !(a > b);
+}
+
 // One whole pixel, serially (host emulation; the kernels spread the chunks over lanes).  AOV: `aov` receives the pixel's sums.
 template <bool STATS = false, bool AOV = false, class Scene>
 TMPT_HD uchar4 render_pixel(const Scene& sc, const Camera& cam, int x, int y, int width, int height, int spp, ex::V3 lightDir,

@@ -107,6 +107,17 @@ struct tmpt_scene {
     void* d_outs[4] = {};          // tmpt_render_outputs(TMPT_HOST): radiance, normal, depth, triangle staged on the device
     size_t outsBytes[4] = {};
     int progW = 0, progH = 0, progChunks = -1;  // -1: no progressive render begun
+    int progAdaptive = -1;         // the session's kind, fixed by its first pass: -1 none yet, 0 uniform, 1 adaptive
+    // adaptive passes (tmpt_progressive_pass_adaptive), allocated by a session's first adaptive pass: per pixel the chunk count
+    // and (mean, M2) of the chunk-mean luminance; the select flags, their exclusive scan and scan totals; the active list
+    uint32_t* d_adN = nullptr;
+    float2* d_adStat = nullptr;
+    uint32_t *d_adFlags = nullptr, *d_adOffs = nullptr, *d_adTotals = nullptr;  // d_adTotals: scan totals, then the grand total
+    uint2* d_adList = nullptr;
+    unsigned int* d_adActive = nullptr;  // [0] pixels left active by the pass, [1] the session's largest chunk count n
+    size_t adPixels = 0;           // capacity of the per-pixel buffers above (tile-padded frame)
+    int32_t* d_samples = nullptr;  // tmpt_progressive_pass_adaptive(TMPT_HOST): samples staged on the device
+    size_t samplesBytes = 0;
     // staging of tmpt_hit_scene(TMPT_HOST): one device and one pinned host buffer per scene, grown on demand and reused (the
     // entry point is called in a loop by batched-query users: five cudaMalloc / cudaFree pairs and pageable copies per call
     // cost more than the kernel for batches under a million rays)
@@ -662,6 +673,8 @@ struct RenderParams {
     uint32_t* tileCounter;
     unsigned long long* laneCounter;  // k_render_regen: next lane item
     unsigned long long* stats;  // instrumented pass only
+    const uint2* list;   // LIST kernels (adaptive passes): the band's entries of the active list, {x | y << 16, first chunk n_i}
+    int listLen;         // entries in the band; accum = [chunks][listLen]
 };
 
 __device__ __forceinline__ int owned_row_to_global(int r, int stripeRows, int rank, int world) {
@@ -719,7 +732,8 @@ constexpr int kSStack = TMPT_SSTACK;
 // exact all-triangle scan.  Only the 256-thread configuration has that instantiation (a camera sixteen scene sizes away sees
 // a few pixels of scene).
 // AOV = the frame has AOV outputs (tmpt_outputs normal / depth / triangle): the same paths, plus each sample's camera-ray hit.
-template <bool STATS, int THREADS, int MINB, int SSTACK, bool FAR = false, bool AOV = false>
+// LIST = an adaptive pass: work item (list tile t, k) is entry list[t * 32 + lane] of the band, its chunk n_i + k of 8 samples.
+template <bool STATS, int THREADS, int MINB, int SSTACK, bool FAR = false, bool AOV = false, bool LIST = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_render(const RenderParams p) {
     const int lane = threadIdx.x & 31;
     unsigned long long rays = 0;
@@ -732,6 +746,16 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render(const RenderParams p) 
         if (tile >= (uint32_t)p.numTiles * (uint32_t)p.chunks) break;
         const int chunk = (int)(tile / (uint32_t)p.numTiles);
         tile -= (uint32_t)chunk * (uint32_t)p.numTiles;
+        if (LIST) {
+            const uint32_t e = tile * 32u + (uint32_t)lane;
+            if (e < (uint32_t)p.listLen) {
+                const uint2 en = p.list[e];
+                const ex::V3 sum = integ::render_chunk<STATS, FAR>(stack, p.sc, p.cam, (int)(en.x & 0xFFFFu), (int)(en.x >> 16), (int)en.y + chunk, p.width,
+                                                                   p.height, 0x7FFFFFFF, integ::kMaxChunkSamples, p.lightDir, rays, &ts);
+                __stcs(&p.accum[(size_t)chunk * p.listLen + e], make_float4(sum.x, sum.y, sum.z, 0.0f));
+            }
+            continue;
+        }
         const int tx = (int)(tile % (uint32_t)p.tilesX), ty = (int)(tile / (uint32_t)p.tilesX);
         const int xl = tx * 8 + (lane & 7), rb = ty * 4 + (lane >> 3), r = p.bandRow0 + rb;
         int x, y;
@@ -893,7 +917,8 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
 // tracing.  Work item = one (pixel, chunk) per lane; consecutive items are the pixels of one 8x4 tile, so a warp starts with a
 // whole tile.  The per-lane arithmetic and its order are those of integ::render_chunk: the frame is byte-identical to k_render's.
 // AOV (as in k_render): the camera ray's hit of each sample is added to nsum / tsum and counted in cl's top byte.
-template <int THREADS, int MINB, int GATE, bool AOV = false>
+// LIST (as in k_render): item (list tile t, k, lane) is entry list[t * 32 + lane], chunk n_i + k; loc holds the entry index.
+template <int THREADS, int MINB, int GATE, bool AOV = false, bool LIST = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderParams p) {
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -920,7 +945,9 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             bool wantItem = !havePath && !done && (cl & 0xFFu) == 0u;
             if (wantItem && hasItem) {
                 const int xl = (int)(loc & 0xFFFFu), rb = (int)(loc >> 16);
-                if (p.useAccum) {
+                if (LIST) {
+                    __stcs(&p.accum[(size_t)(cl >> 8) * p.listLen + loc], make_float4(sum.x, sum.y, sum.z, 0.0f));
+                } else if (p.useAccum) {
                     const size_t a = ((size_t)(AOV ? (cl >> 8) & 0xFFFFu : cl >> 8) * p.bandRows + rb) * p.localWidth + xl;
                     __stcs(&p.accum[a], make_float4(sum.x, sum.y, sum.z, AOV ? (float)(cl >> 24) : 0.0f));
                     if (AOV) __stcs(&p.accum[a + (size_t)p.chunks * p.bandRows * p.localWidth], make_float4(nsum.x, nsum.y, nsum.z, tsum));
@@ -946,6 +973,21 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
                         const uint32_t wi = (uint32_t)(item >> 5), li = (uint32_t)item & 31u;
                         const int chunk = (int)(wi / (uint32_t)p.numTiles);
                         const uint32_t tile = wi - (uint32_t)chunk * (uint32_t)p.numTiles;
+                        if (LIST) {
+                            const uint32_t e = tile * 32u + li;
+                            if (e < (uint32_t)p.listLen) {
+                                const uint2 en = p.list[e];
+                                rng = ex::chunk_seed(en.y + (uint32_t)chunk, (en.x >> 16) * (uint32_t)p.width + (en.x & 0xFFFFu),
+                                                     (uint32_t)p.width * (uint32_t)p.height);
+                                pix = en.x;
+                                loc = e;
+                                cl = ((uint32_t)chunk << 8) | (uint32_t)integ::kMaxChunkSamples;
+                                sum = ex::v3(0.0f, 0.0f, 0.0f);
+                                hasItem = true;
+                                wantItem = false;
+                            }
+                            continue;
+                        }
                         const int tx = (int)(tile % (uint32_t)p.tilesX), ty = (int)(tile / (uint32_t)p.tilesX);
                         const int xl = tx * 8 + (int)(li & 7u), rb = ty * 4 + (int)(li >> 3);
                         const int r = p.bandRow0 + rb;
@@ -1194,6 +1236,77 @@ __global__ void k_resolve(const RenderParams p, int bandRows) {
         if (p.normal) p.normal[pix] = integ::normal_of(nsum, hits, sppRecip);
         if (p.depth) p.depth[pix] = integ::depth_of(tsum, hits);
     }
+}
+
+// ---- K8: adaptive progressive passes (tmpt_progressive_pass_adaptive) ------------------------------------------------------------
+// The active list is in tile order: slot i = tile (i >> 5) of the frame's 8x4 tiles in row-major tile order, lane i & 31 =
+// (x & 7) + 8 (y & 3).  flags[i] = 1 for a pixel of the frame that the pass's params do not call converged; k_scan_* turn the flags
+// into list positions and k_adaptive_compact writes each active pixel's entry {x | y << 16, n_i} there.  With every pixel of a
+// frame whose size is a multiple of 8 x 4 active, list tile t is frame tile t: a LIST kernel's warp traces what k_render's does.
+__global__ void k_adaptive_select(const uint32_t* __restrict__ n, const float2* __restrict__ stat, int width, int height, int tilesX,
+                                  long long slots, float tolerance, int minChunks, uint32_t* __restrict__ flags) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= slots) return;
+    const int tile = (int)(i >> 5), lane = (int)(i & 31);
+    const int x = (tile % tilesX) * 8 + (lane & 7), y = (tile / tilesX) * 4 + (lane >> 3);
+    uint32_t f = 0u;
+    if (x < width && y < height) {
+        const size_t pix = (size_t)y * width + x;
+        const float2 st = stat[pix];
+        f = integ::adaptive_converged(n[pix], st.x, st.y, tolerance, minChunks) ? 0u : 1u;
+    }
+    flags[i] = f;
+}
+__global__ void k_adaptive_compact(const uint32_t* __restrict__ flags, const uint32_t* __restrict__ offs, const uint32_t* __restrict__ n,
+                                   int width, int tilesX, long long slots, uint2* __restrict__ list) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= slots || !flags[i]) return;
+    const int tile = (int)(i >> 5), lane = (int)(i & 31);
+    const int x = (tile % tilesX) * 8 + (lane & 7), y = (tile / tilesX) * 4 + (lane >> 3);
+    list[offs[i]] = make_uint2((uint32_t)x | ((uint32_t)y << 16), n[(size_t)y * width + x]);
+}
+// The band's chunk sums ([chunks][listLen]) into each entry's pixel in chunk order: the colour sum, n and the Welford state, then
+// the pixels left unconverged under the pass's params are counted (the others were converged before the pass and are unchanged)
+// into counters[0], and counters[1] keeps the session's largest n.
+__global__ void k_resolve_adaptive(const RenderParams p, float4* __restrict__ sumBuf, uint32_t* __restrict__ n, float2* __restrict__ stat,
+                                   float tolerance, int minChunks, unsigned int* __restrict__ counters) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    bool open = false;
+    uint32_t nn = 0u;
+    if (e < p.listLen) {
+        const uint2 en = p.list[e];
+        const size_t pix = (size_t)(en.x >> 16) * p.width + (en.x & 0xFFFFu);
+        const float4 s0 = sumBuf[pix];
+        ex::V3 sum = ex::v3(s0.x, s0.y, s0.z);
+        nn = n[pix];
+        float2 st = stat[pix];
+        for (int c = 0; c < p.chunks; ++c) {
+            const float4 v = __ldcs(&p.accum[(size_t)c * p.listLen + e]);
+            const ex::V3 cs = ex::v3(v.x, v.y, v.z);
+            sum = ex::add(sum, cs);
+            integ::adaptive_add_chunk(cs, nn, st.x, st.y);
+        }
+        sumBuf[pix] = make_float4(sum.x, sum.y, sum.z, 0.0f);
+        n[pix] = nn;
+        stat[pix] = st;
+        open = !integ::adaptive_converged(nn, st.x, st.y, tolerance, minChunks);
+    }
+    const unsigned b = __ballot_sync(0xffffffffu, open), mx = __reduce_max_sync(0xffffffffu, nn);
+    if ((threadIdx.x & 31) == 0 && b) atomicAdd(&counters[0], (unsigned)__popc(b));
+    if ((threadIdx.x & 31) == 0 && mx) atomicMax(&counters[1], mx);
+}
+// The whole frame after an adaptive pass: every pixel is its mean over its own 8 n_i samples (as k_resolve resolves a uniform pass).
+__global__ void k_adaptive_write(const float4* __restrict__ sumBuf, const uint32_t* __restrict__ n, long long pixels, uchar4* __restrict__ frame,
+                                 float4* __restrict__ radiance, int32_t* __restrict__ samples) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= pixels) return;
+    const float4 v = sumBuf[i];
+    const ex::V3 sum = ex::v3(v.x, v.y, v.z);
+    const int spp = (int)n[i] * integ::kMaxChunkSamples;
+    const float sppRecip = ex::divf(1.0f, (float)spp);
+    frame[i] = integ::resolve_pixel(sum, sppRecip);
+    if (radiance) radiance[i] = integ::radiance_of(sum, sppRecip);
+    if (samples) samples[i] = spp;
 }
 
 // K5: rank 0 scatters the gathered, rank-major packed stripes into the frame
@@ -1656,6 +1769,8 @@ extern "C" void tmpt_scene_destroy(tmpt_scene* s) {
     cudaFree(s->d_tris9); cudaFree(s->d_nodes); cudaFree(s->d_qnodes); cudaFree(s->d_status);  // (d_tris, d_hitdata live inside d_nodes)
     cudaFree(s->d_tileCounter); cudaFree(s->d_rayCount); cudaFree(s->d_fetchCounter); cudaFree(s->d_frame); cudaFree(s->d_accum); cudaFree(s->d_sum);
     for (void* o : s->d_outs) cudaFree(o);
+    cudaFree(s->d_adN); cudaFree(s->d_adStat); cudaFree(s->d_adFlags); cudaFree(s->d_adOffs); cudaFree(s->d_adTotals); cudaFree(s->d_adList);
+    cudaFree(s->d_adActive); cudaFree(s->d_samples);
     cudaFree(s->d_stage);
     cudaFree(s->d_probe);
     cudaFree(s->d_sunStart); cudaFree(s->d_sunCount); cudaFree(s->d_sunEntries);
@@ -1793,12 +1908,13 @@ static int host_chunk_len(int spp) {
 static int host_chunk_count(int spp) { const int c = host_chunk_len(spp); return (spp + c - 1) / c; }
 
 // planes = 2 for a frame with AOV outputs (a second set of chunk planes: normal and t sums), so its bands have half the rows.
+// An adaptive pass bands its active list instead: "rows" of width 1 = list entries, in multiples of granule = 32 (whole list tiles).
 static int prepare_render_chunks(tmpt_scene* s, int width, int chunks, bool forceAccum, int ownedRows, cudaStream_t st, int* outBandRows,
-                                 int planes = 1) {
+                                 int planes = 1, int granule = 4) {
     int bandRows = ownedRows;
     if ((chunks > 1 || forceAccum) && ownedRows > 0) {
         const size_t rowBytes = (size_t)width * chunks * planes * sizeof(float4), budget = (size_t)4 << 30;
-        bandRows = (int)std::min<size_t>((size_t)ownedRows, std::max<size_t>(4, (budget / rowBytes) & ~(size_t)3));
+        bandRows = (int)std::min<size_t>((size_t)ownedRows, std::max<size_t>(granule, (budget / rowBytes) & ~(size_t)(granule - 1)));
         const size_t need = (size_t)bandRows * rowBytes;
         if (s->accumBytes < need) {
             CU_TRY(cudaStreamSynchronize(st));
@@ -1814,10 +1930,19 @@ static int prepare_render(tmpt_scene* s, int width, int spp, int ownedRows, cuda
     return prepare_render_chunks(s, width, host_chunk_count(spp), false, ownedRows, st, outBandRows);
 }
 
-// One pass of a progressive render: chunks [chunk0, chunk0 + nChunks) of kMaxChunkSamples samples, added to `sum`.
+// One pass of a progressive render: chunks [chunk0, chunk0 + nChunks) of kMaxChunkSamples samples, added to `sum`.  An adaptive
+// pass (adaptive != nullptr) traces chunks [n_i, n_i + nChunks) of the pixels on its active list instead (chunk0 unused).
+struct AdaptivePass {
+    float tolerance;
+    int minChunks;
+    int32_t* samples;  // device buffer of the frame's samples per pixel, or null
+    int listLen;       // active pixels: set by the select step of render_frame
+    unsigned int counters[2];  // after the pass: pixels left unconverged, the session's largest n
+};
 struct ProgressivePass {
     int chunk0, nChunks;
     float4* sum;
+    AdaptivePass* adaptive = nullptr;
 };
 
 // The float outputs of a single-GPU frame (tmpt_outputs, device pointers; null = not produced).
@@ -1904,9 +2029,14 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     p.laneCounter = s->d_fetchCounter;
     p.stats = statsDev;
     p.accum = nullptr;
-    if (p.ownedRows == 0) return TMPT_OK;
+    p.list = nullptr;
+    p.listLen = 0;
+    const AdaptivePass* ad = prog ? prog->adaptive : nullptr;  // LIST kernels over the active list, banded by list entries
+    const int units = ad ? ad->listLen : p.ownedRows;
+    if (units == 0) return TMPT_OK;  // (an adaptive pass with an empty list traces nothing: the kernel choice stays the last frame's)
     int bandRows = 0;
-    const int prc = prepare_render_chunks(s, p.localWidth, p.chunks, p.useAccum != 0, p.ownedRows, st, &bandRows, aov ? 2 : 1);
+    const int prc = ad ? prepare_render_chunks(s, 1, p.chunks, true, units, st, &bandRows, 1, 32)
+                       : prepare_render_chunks(s, p.localWidth, p.chunks, p.useAccum != 0, p.ownedRows, st, &bandRows, aov ? 2 : 1);
     if (prc != TMPT_OK) return prc;
     p.accum = s->d_accum;
     // 32 warps per SM at 64 registers (sweep in profiles/r1_tuning_sweeps.txt: 24 warps at 77 registers is 10 % slower, 40
@@ -1921,20 +2051,25 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
 #endif
     if (aov && (statsDev || rk > 0 || (TMPT_TUNE_CFG && cfgEnv >= 4)))
         return tmpt::fail(TMPT_ERR_ARG, "render: AOV outputs need the shipped render kernels (no instrumented pass, TMPT_RENDER_KERNEL or tuning configuration)");
+    if (ad && (rk > 0 || (TMPT_TUNE_CFG && cfgEnv >= 4)))
+        return tmpt::fail(TMPT_ERR_ARG, "render: adaptive passes need the shipped render kernels (no TMPT_RENDER_KERNEL or tuning configuration)");
     // the shared-memory part of the traversal stacks: kSStack entries x 8 bytes per thread (dynamic shared memory)
     constexpr size_t smemPerThread = (size_t)kSStack * sizeof(unsigned long long);
     if (smemPerThread * 256 > 48 * 1024) {  // (function attributes are per device: set on every launch path, it costs microseconds)
         CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
         CU_TRY(cudaFuncSetAttribute(k_render<true, 256, 4, kSStack>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
         CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
+        CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
     }
     if (smemPerThread * 512 > 48 * 1024) {
         CU_TRY(cudaFuncSetAttribute(k_render<false, 512, 2, kSStack>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 512)));
         CU_TRY(cudaFuncSetAttribute(k_render<false, 512, 2, kSStack, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 512)));
+        CU_TRY(cudaFuncSetAttribute(k_render<false, 512, 2, kSStack, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 512)));
     }
     if (smemPerThread * 1024 > 48 * 1024) {
         CU_TRY(cudaFuncSetAttribute(k_render<false, 1024, 1, kSStack>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 1024)));
         CU_TRY(cudaFuncSetAttribute(k_render<false, 1024, 1, kSStack, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 1024)));
+        CU_TRY(cudaFuncSetAttribute(k_render<false, 1024, 1, kSStack, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 1024)));
     }
     // (lens offsets are at most lensRadius from the origin: add it to the test)
     const bool farCamera = s->view.farLimit > 0.0f &&
@@ -1943,6 +2078,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     if (farCamera && smemPerThread * 256 > 48 * 1024) {
         CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
         CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
+        CU_TRY(cudaFuncSetAttribute(k_render<false, 256, 4, kSStack, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smemPerThread * 256)));
     }
     bool usePaths = false;  // (the instrumented pass and far cameras stay with k_render)
     if (!statsDev && !farCamera && rk == 0 && cfgEnv == 0) {
@@ -1977,10 +2113,17 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM256, k_render<false, 256, 4, kSStack>, 256, smemPerThread * 256));
     CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM512, k_render<false, 512, 2, kSStack>, 512, smemPerThread * 512));
     CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM1024, k_render<false, 1024, 1, kSStack>, 1024, smemPerThread * 1024));
-    for (p.bandRow0 = 0; p.bandRow0 < p.ownedRows; p.bandRow0 += bandRows) {
-        const int rowsHere = std::min(bandRows, p.ownedRows - p.bandRow0);
-        p.bandRows = rowsHere;
-        p.numTiles = p.tilesX * div_up(rowsHere, 4);
+    for (int b0 = 0; b0 < units; b0 += bandRows) {
+        const int rowsHere = std::min(bandRows, units - b0);
+        if (ad) {
+            p.list = s->d_adList + b0;
+            p.listLen = rowsHere;
+            p.numTiles = div_up(rowsHere, 32);
+        } else {
+            p.bandRow0 = b0;
+            p.bandRows = rowsHere;
+            p.numTiles = p.tilesX * div_up(rowsHere, 4);
+        }
         const long long items = (long long)p.numTiles * p.chunks;
         if (items >= 0xFFFFFFFFll) return tmpt::fail(TMPT_ERR_ARG, "render: too many work items in one band");
         CU_TRY(cudaMemsetAsync(s->d_tileCounter, 0, sizeof(uint32_t), st));
@@ -2016,11 +2159,19 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
             const bool big = items >= (long long)s->smCount * 32 * 8 && perSMp1024 > 0;
             const int t = big ? 1024 : 256;
             const int gridP = (int)std::min<long long>((long long)s->smCount * std::max(big ? perSMp1024 : perSMp256, 1), (items * 32 + t - 1) / t);
-            if (aov) {
+            if (ad) {
+                if (big) LAUNCH((k_render_paths<1024, 1, 8, false, true>), gridP, 1024, 0, st, p);
+                else LAUNCH((k_render_paths<256, 4, 8, false, true>), gridP, 256, 0, st, p);
+            } else if (aov) {
                 if (big) LAUNCH((k_render_paths<1024, 1, 8, true>), gridP, 1024, 0, st, p);
                 else LAUNCH((k_render_paths<256, 4, 8, true>), gridP, 256, 0, st, p);
             } else if (big) LAUNCH((k_render_paths<1024, 1, 8>), gridP, 1024, 0, st, p);
             else LAUNCH((k_render_paths<256, 4, 8>), gridP, 256, 0, st, p);
+        } else if (ad) {  // (the same configurations as below, over the active list; never instrumented)
+            if (farCamera) LAUNCH((k_render<false, 256, 4, kSStack, true, false, true>), grid, 256, smemPerThread * 256, st, p);
+            else if (cfg == 3) LAUNCH((k_render<false, 1024, 1, kSStack, false, false, true>), grid, 1024, smemPerThread * 1024, st, p);
+            else if (cfg == 2) LAUNCH((k_render<false, 512, 2, kSStack, false, false, true>), grid, 512, smemPerThread * 512, st, p);
+            else LAUNCH((k_render<false, 256, 4, kSStack, false, false, true>), grid, 256, smemPerThread * 256, st, p);
         } else if (aov) {  // (the same configurations as below, with AOV outputs; never instrumented)
             if (farCamera) LAUNCH((k_render<false, 256, 4, kSStack, true, true>), grid, 256, smemPerThread * 256, st, p);
             else if (cfg == 3) LAUNCH((k_render<false, 1024, 1, kSStack, false, true>), grid, 1024, smemPerThread * 1024, st, p);
@@ -2031,7 +2182,8 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         else if (cfg == 3) LAUNCH((k_render<false, 1024, 1, kSStack>), grid, 1024, smemPerThread * 1024, st, p);
         else if (cfg == 2) LAUNCH((k_render<false, 512, 2, kSStack>), grid, 512, smemPerThread * 512, st, p);
         else LAUNCH((k_render<false, 256, 4, kSStack>), grid, 256, smemPerThread * 256, st, p);
-        if (p.useAccum && aov) LAUNCH(k_resolve<true>, div_up((long long)rowsHere * p.localWidth, 256), 256, 0, st, p, rowsHere);
+        if (ad) LAUNCH(k_resolve_adaptive, div_up(rowsHere, 256), 256, 0, st, p, prog->sum, s->d_adN, s->d_adStat, ad->tolerance, ad->minChunks, s->d_adActive);
+        else if (p.useAccum && aov) LAUNCH(k_resolve<true>, div_up((long long)rowsHere * p.localWidth, 256), 256, 0, st, p, rowsHere);
         else if (p.useAccum) LAUNCH(k_resolve<false>, div_up((long long)rowsHere * p.localWidth, 256), 256, 0, st, p, rowsHere);
     }
     CU_TRY(cudaGetLastError());
@@ -2097,16 +2249,46 @@ static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int
             }
     FrameOutputs f;
     f.radiance = (float4*)dev[1]; f.normal = (float4*)dev[2]; f.depth = (float*)dev[3]; f.triangle = (int32_t*)dev[4];
+    AdaptivePass* ad = prog ? prog->adaptive : nullptr;
+    int32_t* userSamples = ad ? ad->samples : nullptr;
+    if (userSamples && mem == TMPT_HOST) {
+        const int rc = grow_scratch((void**)&s->d_samples, &s->samplesBytes, pixels * sizeof(int32_t));
+        if (rc != TMPT_OK) return rc;
+        ad->samples = s->d_samples;
+    }
     const int chunks = prog ? prog->nChunks : host_chunk_count(spp);
-    int rc = prepare_render_chunks(s, width, chunks, prog || f.accum(), height, st, nullptr, f.aov() ? 2 : 1);  // (scratch allocation stays outside the timed window)
+    // (scratch allocation stays outside the timed window; an adaptive pass allocates for a list of every pixel)
+    int rc = ad ? prepare_render_chunks(s, 1, chunks, true, (int)pixels, st, nullptr, 1, 32)
+                : prepare_render_chunks(s, width, chunks, prog || f.accum(), height, st, nullptr, f.aov() ? 2 : 1);
     if (rc != TMPT_OK) return rc;
     CU_TRY(cudaEventRecord(s->ev0, st));
     CU_TRY(cudaMemsetAsync(s->d_rayCount, 0, sizeof(unsigned long long), st));
+    if (ad) {  // select + compact: the active list and its length (one small copy)
+        const int tilesX = div_up(width, 8);
+        const long long slots = (long long)tilesX * div_up(height, 4) * 32;
+        const int nBlocks = div_up(slots, kScanBlock);
+        LAUNCH(k_adaptive_select, div_up(slots, 256), 256, 0, st, s->d_adN, s->d_adStat, width, height, tilesX, slots, ad->tolerance, ad->minChunks,
+               s->d_adFlags);
+        LAUNCH(k_scan_totals, nBlocks, kScanBlock, 0, st, s->d_adFlags, slots, s->d_adTotals);
+        LAUNCH(k_scan_of_totals, 1, kScanBlock, 0, st, s->d_adTotals, nBlocks, s->d_adTotals + nBlocks);
+        LAUNCH(k_scan_apply, nBlocks, kScanBlock, 0, st, s->d_adFlags, slots, s->d_adTotals, s->d_adTotals + nBlocks, s->d_adOffs);
+        LAUNCH(k_adaptive_compact, div_up(slots, 256), 256, 0, st, s->d_adFlags, s->d_adOffs, s->d_adN, width, tilesX, slots, s->d_adList);
+        CU_TRY(cudaMemsetAsync(s->d_adActive, 0, sizeof(unsigned int), st));
+        uint32_t listLen = 0;
+        CU_TRY(cudaMemcpyAsync(&listLen, s->d_adTotals + nBlocks, sizeof listLen, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        ad->listLen = (int)listLen;
+    }
     rc = launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, (uint8_t*)dev[0], s->d_rayCount, st, nullptr, prog, &f);
     if (rc != TMPT_OK) return rc;
-    if (mem == TMPT_HOST)
+    if (ad) LAUNCH(k_adaptive_write, div_up((long long)pixels, 256), 256, 0, st, prog->sum, s->d_adN, (long long)pixels, (uchar4*)dev[0], f.radiance,
+                   ad->samples);
+    if (mem == TMPT_HOST) {
         for (int k = 0; k < 5; ++k)
             if (user[k]) CU_TRY(cudaMemcpyAsync(user[k], dev[k], bytes[k], cudaMemcpyDeviceToHost, st));
+        if (userSamples) CU_TRY(cudaMemcpyAsync(userSamples, s->d_samples, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    }
+    if (ad) CU_TRY(cudaMemcpyAsync(ad->counters, s->d_adActive, sizeof ad->counters, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaEventRecord(s->ev1, st));
     unsigned long long rays = 0;
     CU_TRY(cudaMemcpyAsync(&rays, s->d_rayCount, sizeof rays, cudaMemcpyDeviceToHost, st));
@@ -2157,7 +2339,7 @@ extern "C" int tmpt_progressive_begin(tmpt_scene* s, int width, int height) {
     }
     CU_TRY(cudaMemsetAsync(s->d_sum, 0, need, s->stream));
     CU_TRY(cudaStreamSynchronize(s->stream));
-    s->progW = width; s->progH = height; s->progChunks = 0;
+    s->progW = width; s->progH = height; s->progChunks = 0; s->progAdaptive = -1;
     return TMPT_OK;
 }
 
@@ -2170,6 +2352,7 @@ extern "C" int tmpt_progressive_pass_outputs(tmpt_scene* s, const tmpt_camera* c
         return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_pass_outputs: passes produce rgba and radiance only (no running AOV sums)");
     if (s->progChunks < 0) return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_pass_outputs: call tmpt_progressive_begin first");
     std::lock_guard<std::mutex> lock(s->hostCallMutex);
+    if (s->progAdaptive == 1) return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_pass_outputs: this session's passes are adaptive (tmpt_progressive_begin starts a new one)");
     if (nChunks < 1 || nChunks > 128 || (long long)(s->progChunks + nChunks) * integ::kMaxChunkSamples > (1 << 24))
         return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_pass_outputs: %d chunks after %d", nChunks, s->progChunks);
     DeviceGuard guard(s->device);
@@ -2179,7 +2362,70 @@ extern "C" int tmpt_progressive_pass_outputs(tmpt_scene* s, const tmpt_camera* c
     rc = render_frame(s, camera, s->progW, s->progH, 0, mem, out, &pass, st, rayCount, seconds);
     if (rc != TMPT_OK) return rc;
     s->progChunks += nChunks;
+    s->progAdaptive = 0;
     if (samplesSoFar) *samplesSoFar = s->progChunks * integ::kMaxChunkSamples;
+    return check_status(s, st);
+}
+
+// The per-pixel state of adaptive passes, for a progW x progH session: zeroed with the session's first adaptive pass.
+static int begin_adaptive(tmpt_scene* s, cudaStream_t st) {
+    const int tilesX = div_up(s->progW, 8);
+    const size_t slots = (size_t)tilesX * div_up(s->progH, 4) * 32, pixels = (size_t)s->progW * s->progH;
+    if (s->adPixels < slots) {
+        CU_TRY(cudaStreamSynchronize(st));
+        cudaFree(s->d_adN); cudaFree(s->d_adStat); cudaFree(s->d_adFlags); cudaFree(s->d_adOffs); cudaFree(s->d_adTotals); cudaFree(s->d_adList);
+        cudaFree(s->d_adActive);
+        s->d_adN = nullptr; s->d_adStat = nullptr; s->d_adFlags = s->d_adOffs = s->d_adTotals = nullptr; s->d_adList = nullptr; s->d_adActive = nullptr;
+        s->adPixels = 0;
+        CU_TRY(cudaMalloc((void**)&s->d_adN, slots * sizeof(uint32_t)));
+        CU_TRY(cudaMalloc((void**)&s->d_adStat, slots * sizeof(float2)));
+        CU_TRY(cudaMalloc((void**)&s->d_adFlags, slots * sizeof(uint32_t)));
+        CU_TRY(cudaMalloc((void**)&s->d_adOffs, (slots + 1) * sizeof(uint32_t)));
+        CU_TRY(cudaMalloc((void**)&s->d_adTotals, (slots / kScanBlock + 2) * sizeof(uint32_t)));
+        CU_TRY(cudaMalloc((void**)&s->d_adList, slots * sizeof(uint2)));
+        CU_TRY(cudaMalloc((void**)&s->d_adActive, 2 * sizeof(unsigned int)));
+        s->adPixels = slots;
+    }
+    CU_TRY(cudaMemsetAsync(s->d_adN, 0, pixels * sizeof(uint32_t), st));
+    CU_TRY(cudaMemsetAsync(s->d_adStat, 0, pixels * sizeof(float2), st));
+    CU_TRY(cudaMemsetAsync(s->d_adActive, 0, 2 * sizeof(unsigned int), st));
+    return TMPT_OK;
+}
+
+extern "C" int tmpt_progressive_pass_adaptive(tmpt_scene* s, const tmpt_camera* camera, int nChunks, const tmpt_adaptive* params, int mem,
+                                              const tmpt_outputs* out, int32_t* samples, uint64_t* rayCount, double* seconds,
+                                              int64_t* activePixels, void* stream) {
+    static const char* fn = "tmpt_progressive_pass_adaptive";
+    if (!s || !camera) return tmpt::fail(TMPT_ERR_ARG, "%s: NULL scene / camera", fn);
+    int rc = check_outputs(fn, out, mem);
+    if (rc != TMPT_OK) return rc;
+    if (out->normal || out->depth || out->triangle) return tmpt::fail(TMPT_ERR_ARG, "%s: passes produce rgba and radiance only (no running AOV sums)", fn);
+    if (!params) return tmpt::fail(TMPT_ERR_ARG, "%s: params is NULL", fn);
+    if (!(params->tolerance >= 0.0f && params->tolerance <= 3.4028235e38f))
+        return tmpt::fail(TMPT_ERR_ARG, "%s: tolerance %g is not a finite value >= 0", fn, (double)params->tolerance);
+    if (params->minChunks < 2 || params->minChunks > (1 << 21)) return tmpt::fail(TMPT_ERR_ARG, "%s: minChunks %d out of range 2..2^21", fn, params->minChunks);
+    if (nChunks < 1 || nChunks > 128) return tmpt::fail(TMPT_ERR_ARG, "%s: nChunks %d out of range 1..128", fn, nChunks);
+    if (s->progChunks < 0) return tmpt::fail(TMPT_ERR_ARG, "%s: call tmpt_progressive_begin first", fn);
+    std::lock_guard<std::mutex> lock(s->hostCallMutex);
+    if (s->progAdaptive == 0) return tmpt::fail(TMPT_ERR_ARG, "%s: this session's passes are uniform (tmpt_progressive_begin starts a new one)", fn);
+    // progChunks = the session's largest n (a pixel is traced at most once per pass)
+    if ((long long)(s->progChunks + nChunks) * integ::kMaxChunkSamples > (1 << 24))
+        return tmpt::fail(TMPT_ERR_ARG, "%s: %d chunks after %d", fn, nChunks, s->progChunks);
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "%s: cudaSetDevice(%d) failed", fn, s->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (s->progAdaptive < 0) {
+        rc = begin_adaptive(s, st);
+        if (rc != TMPT_OK) return rc;
+    }
+    AdaptivePass ad{params->tolerance, params->minChunks, samples, 0, {0u, 0u}};
+    ProgressivePass pass{0, nChunks, s->d_sum};
+    pass.adaptive = &ad;
+    rc = render_frame(s, camera, s->progW, s->progH, 0, mem, out, &pass, st, rayCount, seconds);
+    if (rc != TMPT_OK) return rc;
+    s->progAdaptive = 1;
+    if (ad.listLen > 0) s->progChunks = (int)ad.counters[1];
+    if (activePixels) *activePixels = (int64_t)ad.counters[0];
     return check_status(s, st);
 }
 
