@@ -206,6 +206,53 @@ int tmpt_progressive_pass_adaptive(tmpt_scene* scene, const tmpt_camera* camera,
                                    const tmpt_outputs* out, int32_t* samples, uint64_t* rayCount, double* seconds,
                                    int64_t* activePixels, void* stream);
 
+/* Denoising (beyond the reference): an edge-avoiding a-trous wavelet filter (Dammertz et al. 2010) with the variance-guided
+ * luminance weights of SVGF's spatial filter (Schied et al. 2017) over a frame's linear radiance, guided by its first-hit normal,
+ * coverage and depth.  Bit-exact against a serial restatement: one rounding per float operation, no contraction, every sum in
+ * the order below from +0.0f, and e^(-x) is expneg (binary64 with unfused operations, one rounding to binary32, within 1 ulp of
+ * the correctly rounded value; 1 for x <= 0; 0 for x >= 104, +inf and NaN).
+ * Per pixel p: c = radiance.xyz, N = normal.xyz, z = depth; l(c) = ((0.2126f c.x + 0.7152f c.y) + 0.0722f c.z).
+ *   class      p is a hit pixel if normal.w > 0, else sky; pixels of different classes never mix
+ *   valid      all three channels of p's current colour are finite; an invalid pixel is never a tap, so a NaN pixel becomes the
+ *              weighted mean of its valid neighbours (it keeps its input if it has none)
+ *   prologue   n_p = N * (1 / sqrt(dot(N, N))) for a hit pixel with dot(N, N) finite and > 0, else 0.
+ *              (gx, gy): (z[x+1] - z[x-1]) * 0.5 over in-frame hit neighbours, z[x+1] - z or z - z[x-1] where only one is,
+ *              0 where none is (likewise in y with the rows above and below); 0 for sky.
+ *              var_p: over the valid pixels of p's class in the 3 x 3 window (dy outer, dx inner), count and sum of l, then
+ *              mean = sum / count and var = (sum of (l - mean) * (l - mean)) / count; 0 if none qualifies.  State = (c, var).
+ *   iteration  i = 0 .. iterations - 1 with step s = 2^i, each from the previous state into a new one:
+ *              v_p = (sum k var_q) / (sum k) over the valid pixels of p's class in the 3 x 3 window at spacing 1, k =
+ *                    g[dx] * g[dy] with g = {1/4, 1/2, 1/4}; 0 if none qualifies
+ *              taps q = p + s (dx, dy), dy outer and dx inner over -2..2, counted if in the frame, valid and of p's class:
+ *                h   = h1[dx] * h1[dy], h1 = {1/16, 1/4, 3/8, 1/4, 1/16}
+ *                w_n = |dot(n_p, n_q)| squared normalPowerLog2 times (hit); 1 (sky)
+ *                e_z = |z_p - z_q| / (sigmaDepth * (|gx dx + gy dy| * s + 0.01f z_p)) (hit); 0 (sky)
+ *                e_c = 16 |cov_p - cov_q| with cov = normal.w (hit): silhouette pixels, blends of surface and sky, are
+ *                      filtered with pixels of like coverage and left out of the interior's sums; 0 (sky)
+ *                e_l = |l_p - l_q| / (sigmaLuminance * sqrt(v_p) + 1e-10f) for a valid p; 0 for an invalid one
+ *                w   = (h * w_n) * expneg((e_z + e_c) + e_l)
+ *              W = sum w, C = sum w c_q per channel, V = sum (w w) var_q; new state (C / W, V / (W W)), or the old one if W == 0
+ *   outputs    rgba = quantise(sqrt(c)) per channel as tmpt_render (NaN -> 0), A = 255; radiance = (c, 1.0f).  With
+ *              iterations = 0 both come straight from the input: rgba is tmpt_render's frame for the same radiance, byte for byte.
+ *   in         tmpt_render_outputs' buffers: radiance, normal and depth are required; rgba and triangle are not read.  The guides
+ *              may come from a frame at another spp than the radiance: e.g. normal and depth from tmpt_render_outputs at spp 8,
+ *              radiance from an adaptive session (tmpt_progressive_pass_adaptive) of the same camera and size.
+ *   out        rgba and / or radiance (other pointers: TMPT_ERR_ARG); out->radiance may be in->radiance (filters in place).
+ *   mem / stream / seconds as tmpt_render_outputs: with TMPT_HOST the inputs and outputs are staged in device scratch owned by
+ *              the scene; seconds = device time of the kernels and copies.  The scene supplies the device, the stream, its
+ *              host-call lock and scratch (4 x 16 bytes per pixel); its triangles are not read.  Single GPU.
+ * Errors (TMPT_ERR_ARG, with a message, before any device work): a NULL scene, in, params or out; a missing in->radiance,
+ * in->normal or in->depth; no output requested or an AOV pointer in `out`; a bad mem; width or height outside 1..10000;
+ * iterations outside 0..8, normalPowerLog2 outside 0..8, or a sigma that is not a finite value > 0. */
+typedef struct tmpt_denoise_params {
+    int32_t iterations;      /* 0..8 a-trous passes; pass i's taps are 2^i pixels apart; 0 = the output is the input     */
+    float sigmaLuminance;    /* > 0, finite: luminance edge-stop in units of the local standard deviation (SVGF: 4)     */
+    float sigmaDepth;        /* > 0, finite: depth edge-stop (SVGF: 1)                                                   */
+    int32_t normalPowerLog2; /* 0..8: the normal weight is |n_p . n_q|^(2^k) (SVGF's 128 = 7)                           */
+} tmpt_denoise_params;
+int tmpt_denoise(tmpt_scene* scene, int width, int height, int mem, const tmpt_outputs* in, const tmpt_denoise_params* params,
+                 const tmpt_outputs* out, double* seconds, void* stream);
+
 /* Multi-GPU form: this rank renders only its share of the frame and writes it packed into
  * outStripes (device memory on the scene's device, tmpt_stripe_rows(...) *
  * tmpt_local_width(...) * 4 bytes).  Two partitions:

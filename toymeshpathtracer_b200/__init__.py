@@ -9,6 +9,7 @@ drive it through; it mirrors the reference's own interface names:
     Scene.HitScene(rays, tMin, tMax) Scene::HitScene, batched        (scene.h:36-37)
     Scene.render(camera, w, h, spp)  TraceImageBody over all rows    (main.cpp:180-246, 329-331)
     Scene.render_outputs(...)        the same frame plus linear radiance and first-hit AOVs (beyond the reference)
+    Scene.denoise(...)               an a-trous filter over the radiance, guided by the AOVs (beyond the reference)
     load_scene(path)                 LoadScene                       (main.cpp:122-170)
     camera_for_scene(...)            camera placement of main()      (main.cpp:296-307)
 
@@ -40,7 +41,7 @@ ABI_SYMBOLS = [
     "tmpt_device_count", "tmpt_launch_count", "tmpt_render_stats", "tmpt_hit_scene_stats",
     "tmpt_frame_alloc", "tmpt_frame_open", "tmpt_frame_close", "tmpt_frame_free", "tmpt_render_multi",
     "tmpt_scene_refit", "tmpt_progressive_begin", "tmpt_progressive_pass", "tmpt_render_kernel_choice",
-    "tmpt_render_outputs", "tmpt_progressive_pass_outputs", "tmpt_progressive_pass_adaptive",
+    "tmpt_render_outputs", "tmpt_progressive_pass_outputs", "tmpt_progressive_pass_adaptive", "tmpt_denoise",
 ]
 
 
@@ -72,6 +73,11 @@ def _output_arrays(names, width: int, height: int) -> dict:
 class Adaptive(C.Structure):
     """tmpt_adaptive: the stop rule of an adaptive progressive pass."""
     _fields_ = [("tolerance", C.c_float), ("minChunks", C.c_int32)]
+
+
+class DenoiseParams(C.Structure):
+    """tmpt_denoise_params: the a-trous filter's iterations and edge-stopping parameters."""
+    _fields_ = [("iterations", C.c_int32), ("sigmaLuminance", C.c_float), ("sigmaDepth", C.c_float), ("normalPowerLog2", C.c_int32)]
 
 
 class SceneInfo(C.Structure):
@@ -117,6 +123,7 @@ def lib() -> C.CDLL:
                                                 C.POINTER(i32), vp]
     L.tmpt_progressive_pass_adaptive.argtypes = [vp, vp, i32, C.POINTER(Adaptive), i32, C.POINTER(Outputs), vp, C.POINTER(C.c_uint64),
                                                  C.POINTER(C.c_double), C.POINTER(i64), vp]
+    L.tmpt_denoise.argtypes = [vp, i32, i32, i32, C.POINTER(Outputs), C.POINTER(DenoiseParams), C.POINTER(Outputs), C.POINTER(C.c_double), vp]
     L.tmpt_progressive_begin.argtypes = [vp, i32, i32]
     L.tmpt_progressive_pass.argtypes = [vp, vp, i32, i32, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double), C.POINTER(i32), vp]
     L.tmpt_render_stripes.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp]
@@ -366,6 +373,36 @@ class Scene:
         _check(lib().tmpt_progressive_pass_adaptive(self._h, _ptr(cam), n_chunks, C.byref(params), HOST, C.byref(out),
                                                     _ptr(arrays["samples"]), C.byref(rays), C.byref(sec), C.byref(active), None))
         return arrays, rays.value, sec.value, active.value
+
+    def denoise(self, radiance, normal, depth, iterations: int = 5, sigma_luminance: float = 4.0, sigma_depth: float = 1.0,
+                normal_power_log2: int = 7, outputs=("rgba", "radiance")):
+        """tmpt_denoise on host arrays: radiance / normal [h,w,4] float32 and depth [h,w] float32 as render_outputs returns them (the
+        guides may come from a frame at another spp) -> ({"rgba", "radiance"} as named in `outputs`, seconds)."""
+        radiance, normal, depth = _f32(radiance), _f32(normal), _f32(depth)
+        height, width = depth.shape
+        if radiance.shape != (height, width, 4) or normal.shape != (height, width, 4):
+            raise ValueError(f"radiance {radiance.shape} and normal {normal.shape} must be {(height, width, 4)} for depth {depth.shape}")
+        if set(outputs) - {"rgba", "radiance"}:
+            raise ValueError(f"denoise outputs are rgba and radiance, not {sorted(set(outputs) - {'rgba', 'radiance'})}")
+        arrays = _output_arrays(outputs, width, height)
+        inp = Outputs(radiance=radiance.ctypes.data, normal=normal.ctypes.data, depth=depth.ctypes.data)
+        out = Outputs(**{n: a.ctypes.data for n, a in arrays.items()})
+        params = DenoiseParams(iterations, sigma_luminance, sigma_depth, normal_power_log2)
+        sec = C.c_double(0.0)
+        _check(lib().tmpt_denoise(self._h, width, height, HOST, C.byref(inp), C.byref(params), C.byref(out), C.byref(sec), None))
+        return arrays, sec.value
+
+    def denoise_device(self, width: int, height: int, radiance_ptr: int, normal_ptr: int, depth_ptr: int, rgba_out_ptr: int = 0,
+                       radiance_out_ptr: int = 0, iterations: int = 5, sigma_luminance: float = 4.0, sigma_depth: float = 1.0,
+                       normal_power_log2: int = 7, stream: int = 0) -> float:
+        """tmpt_denoise on device buffers (raw addresses, e.g. torch ``data_ptr()``; an output 0 = not produced; radiance_out_ptr may
+        be radiance_ptr) -> seconds."""
+        inp = Outputs(radiance=radiance_ptr, normal=normal_ptr, depth=depth_ptr)
+        out = Outputs(rgba=rgba_out_ptr or None, radiance=radiance_out_ptr or None)
+        params = DenoiseParams(iterations, sigma_luminance, sigma_depth, normal_power_log2)
+        sec = C.c_double(0.0)
+        _check(lib().tmpt_denoise(self._h, width, height, DEVICE, C.byref(inp), C.byref(params), C.byref(out), C.byref(sec), stream or None))
+        return sec.value
 
     def render_into(self, camera, width: int, height: int, spp: int, host_ptr: int):
         """One frame into caller-owned HOST memory (w*h*4 bytes, e.g. a pinned buffer) -> (rayCount, seconds): tmpt_render as a

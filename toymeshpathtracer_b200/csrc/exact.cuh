@@ -179,6 +179,45 @@ TMPT_HD void sincos_spec(float a, float& s, float& c) {
     c = d2f(cv);
 }
 
+// "Exp spec": e^(-x) for the denoiser's edge-stopping weights (denoise.cuh), written like sincos_spec: binary64 with unfused
+// multiply / add and one final rounding to binary32, so the host restatement gives identical bits; within 1 ulp of the
+// correctly rounded value.  x <= 0 (and -0) gives 1, so a weight never exceeds its kernel weight; x >= 104 (where e^(-x) is
+// below half the smallest subnormal), +inf and NaN give 0, so a bad weight drops out of a sum instead of poisoning it.
+// Reduction: x = k ln2 + r with ln2 split Cody-Waite style (k <= 150, so k * LN2_HI is exact), |r| <= ln2 / 2; e^(-r) is the
+// degree-13 Taylor polynomial (truncation below 1e-17) in Horner form, scaled by 2^-k exactly (the double has the range).
+TMPT_HD float expneg_spec(float x) {
+    if (!(x < 104.0f)) return 0.0f;
+    if (x <= 0.0f) return 1.0f;
+    const double INV_LN2 = 1.44269504088896338700e+00;
+    const double LN2_HI = 6.93147180369123816490e-01;  // 0x3FE62E42FEE00000
+    const double LN2_LO = 1.90821492927058770002e-10;  // 0x3DEA39EF35793C76
+    const double xd = (double)x;
+    const double kd = floor(dadd(dmul(xd, INV_LN2), 0.5));
+    const double y = -dsub(dsub(xd, dmul(kd, LN2_HI)), dmul(kd, LN2_LO));  // -r
+    double p = 1.0 / 6227020800.0;                                          // 1/13!
+    p = dadd(dmul(p, y), 1.0 / 479001600.0);
+    p = dadd(dmul(p, y), 1.0 / 39916800.0);
+    p = dadd(dmul(p, y), 1.0 / 3628800.0);
+    p = dadd(dmul(p, y), 1.0 / 362880.0);
+    p = dadd(dmul(p, y), 1.0 / 40320.0);
+    p = dadd(dmul(p, y), 1.0 / 5040.0);
+    p = dadd(dmul(p, y), 1.0 / 720.0);
+    p = dadd(dmul(p, y), 1.0 / 120.0);
+    p = dadd(dmul(p, y), 1.0 / 24.0);
+    p = dadd(dmul(p, y), 1.0 / 6.0);
+    p = dadd(dmul(p, y), 0.5);
+    p = dadd(dmul(p, y), 1.0);
+    p = dadd(dmul(p, y), 1.0);
+    const uint64_t bits = (uint64_t)(1023 - (int)kd) << 52;  // 2^-k
+    double scale;
+#ifdef __CUDA_ARCH__
+    scale = __longlong_as_double((long long)bits);
+#else
+    memcpy(&scale, &bits, 8);
+#endif
+    return d2f(dmul(p, scale));
+}
+
 // maths.cpp:30-38
 TMPT_HD V3 random_unit_vector(uint32_t& state) {
     const float kPI = 3.1415926f;  // maths.h:14

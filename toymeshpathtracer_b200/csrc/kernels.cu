@@ -10,6 +10,7 @@
 //   K5  share gather   k_unpack_stripes       (rank 0 after the multi-GPU gather; the default multi-GPU path has no gather:
 //                                              every rank's k_render stores its pixels into rank 0's frame over NVLink)
 //   K6  refit          k_refit_pending, k_refit_wide  (tmpt_scene_refit: moved vertices, same topology)
+//   K9  denoise        k_denoise_prep, k_denoise_atrous, k_denoise_copy  (tmpt_denoise: a-trous filter over the radiance and AOVs)
 //
 // There is no CPU fallback in this file: every entry point needs a CUDA device.
 #include <cooperative_groups.h>
@@ -29,6 +30,7 @@
 
 #include "build_logic.cuh"
 #include "common.h"
+#include "denoise.cuh"
 #include "integrator.cuh"
 // The render kernel with per-lane ray regeneration (k_render_regen: measured in rounds 1 and 2, 31 % slower, DESIGN.md 5) is
 // compiled only with -DTMPT_EXPERIMENTS=1; the shipped library does not contain it.  (Round 1's three experimental HitScene
@@ -118,6 +120,8 @@ struct tmpt_scene {
     size_t adPixels = 0;           // capacity of the per-pixel buffers above (tile-padded frame)
     int32_t* d_samples = nullptr;  // tmpt_progressive_pass_adaptive(TMPT_HOST): samples staged on the device
     size_t samplesBytes = 0;
+    float4* d_denoise = nullptr;   // tmpt_denoise: [4][pixels] float4: two state buffers (ping-pong), guideA, guideB (denoise.cuh)
+    size_t denoiseBytes = 0;
     // staging of tmpt_hit_scene(TMPT_HOST): one device and one pinned host buffer per scene, grown on demand and reused (the
     // entry point is called in a loop by batched-query users: five cudaMalloc / cudaFree pairs and pageable copies per call
     // cost more than the kernel for batches under a million rays)
@@ -1309,6 +1313,47 @@ __global__ void k_adaptive_write(const float4* __restrict__ sumBuf, const uint32
     if (samples) samples[i] = spp;
 }
 
+// ---- K9: denoiser (tmpt_denoise) -----------------------------------------------------------------------------------------------
+// One thread per pixel over 32 x 8 blocks, through denoise.cuh's per-pixel functions.  A warp is one row segment of 32 pixels, so
+// every tap's loads are 32 consecutive float4s at any step; no shared-memory tile: from step 2 on the 5 x 5 taps reach 2 .. 128
+// pixels away, far outside any tile of a 256-thread block, and at step 1 the overlapping windows of a block are L1 hits.
+constexpr int kDenoiseBX = 32, kDenoiseBY = 8;
+__global__ void __launch_bounds__(kDenoiseBX * kDenoiseBY) k_denoise_prep(const float4* __restrict__ radiance, const float4* __restrict__ normal,
+                                                                        const float* __restrict__ depth, int width, int height,
+                                                                        float4* __restrict__ state, float4* __restrict__ guideA,
+                                                                        float4* __restrict__ guideB) {
+    const int x = blockIdx.x * kDenoiseBX + threadIdx.x, y = blockIdx.y * kDenoiseBY + threadIdx.y;
+    if (x >= width || y >= height) return;
+    const size_t p = (size_t)y * width + x;
+    float4 st, a, b;
+    dn::prep_pixel(radiance, normal, depth, width, height, x, y, st, a, b);
+    state[p] = st;
+    guideA[p] = a;
+    guideB[p] = b;
+}
+// One iteration: state `in` -> `out`; the LAST one writes the outputs instead of a state (the epilogue fused).
+template <bool LAST>
+__global__ void __launch_bounds__(kDenoiseBX * kDenoiseBY) k_denoise_atrous(const float4* __restrict__ in, float4* __restrict__ out,
+                                                                          const float4* __restrict__ guideA, const float4* __restrict__ guideB,
+                                                                          int width, int height, int step, dn::Params prm,
+                                                                          uchar4* __restrict__ rgba, float4* __restrict__ radiance) {
+    const int x = blockIdx.x * kDenoiseBX + threadIdx.x, y = blockIdx.y * kDenoiseBY + threadIdx.y;
+    if (x >= width || y >= height) return;
+    const size_t p = (size_t)y * width + x;
+    const float4 s = dn::atrous_pixel(in, guideA, guideB, width, height, x, y, step, prm);
+    if (!LAST) { out[p] = s; return; }
+    if (rgba) rgba[p] = dn::rgba_of(s);
+    if (radiance) radiance[p] = dn::radiance_of(s);
+}
+// No iteration: the outputs of the input radiance (radiance out may be radiance in: each thread reads its pixel before it writes it).
+__global__ void k_denoise_copy(const float4* radianceIn, long long pixels, uchar4* __restrict__ rgba, float4* radiance) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= pixels) return;
+    const float4 c = radianceIn[i];
+    if (rgba) rgba[i] = dn::rgba_of(c);
+    if (radiance) radiance[i] = dn::radiance_of(c);
+}
+
 // K5: rank 0 scatters the gathered, rank-major packed stripes into the frame
 __global__ void k_unpack_stripes(const uchar4* __restrict__ gathered, int width, int height, int stripeRows, int world, int maxRowsPerRank,
                                  uchar4* __restrict__ frame) {
@@ -1770,7 +1815,7 @@ extern "C" void tmpt_scene_destroy(tmpt_scene* s) {
     cudaFree(s->d_tileCounter); cudaFree(s->d_rayCount); cudaFree(s->d_fetchCounter); cudaFree(s->d_frame); cudaFree(s->d_accum); cudaFree(s->d_sum);
     for (void* o : s->d_outs) cudaFree(o);
     cudaFree(s->d_adN); cudaFree(s->d_adStat); cudaFree(s->d_adFlags); cudaFree(s->d_adOffs); cudaFree(s->d_adTotals); cudaFree(s->d_adList);
-    cudaFree(s->d_adActive); cudaFree(s->d_samples);
+    cudaFree(s->d_adActive); cudaFree(s->d_samples); cudaFree(s->d_denoise);
     cudaFree(s->d_stage);
     cudaFree(s->d_probe);
     cudaFree(s->d_sunStart); cudaFree(s->d_sunCount); cudaFree(s->d_sunEntries);
@@ -2438,6 +2483,87 @@ extern "C" int tmpt_progressive_pass(tmpt_scene* s, const tmpt_camera* camera, i
 }
 
 // One process, several devices: stripes of rank i on scenes[i], pixels stored into device 0's frame by peer access.
+// The denoiser (beyond the reference): include/tmpt.h documents the filter; denoise.cuh holds its arithmetic.
+extern "C" int tmpt_denoise(tmpt_scene* s, int width, int height, int mem, const tmpt_outputs* in, const tmpt_denoise_params* params,
+                            const tmpt_outputs* out, double* seconds, void* stream) {
+    static const char* fn = "tmpt_denoise";
+    if (!s) return tmpt::fail(TMPT_ERR_ARG, "%s: NULL scene", fn);
+    if (!in) return tmpt::fail(TMPT_ERR_ARG, "%s: in is NULL", fn);
+    if (!params) return tmpt::fail(TMPT_ERR_ARG, "%s: params is NULL", fn);
+    if (!out) return tmpt::fail(TMPT_ERR_ARG, "%s: out is NULL", fn);
+    if (!in->radiance || !in->normal || !in->depth) return tmpt::fail(TMPT_ERR_ARG, "%s: in->radiance, in->normal and in->depth are required", fn);
+    if (!out->rgba && !out->radiance) return tmpt::fail(TMPT_ERR_ARG, "%s: no output requested", fn);
+    if (out->normal || out->depth || out->triangle) return tmpt::fail(TMPT_ERR_ARG, "%s: out takes rgba and radiance only", fn);
+    if (mem != TMPT_HOST && mem != TMPT_DEVICE) return tmpt::fail(TMPT_ERR_ARG, "%s: mem %d", fn, mem);
+    if (width < 1 || width > 10000 || height < 1 || height > 10000) return tmpt::fail(TMPT_ERR_ARG, "%s: %d x %d out of range", fn, width, height);
+    if (params->iterations < 0 || params->iterations > dn::kMaxIterations)
+        return tmpt::fail(TMPT_ERR_ARG, "%s: iterations %d out of range 0..%d", fn, params->iterations, dn::kMaxIterations);
+    if (params->normalPowerLog2 < 0 || params->normalPowerLog2 > dn::kMaxNormalPowerLog2)
+        return tmpt::fail(TMPT_ERR_ARG, "%s: normalPowerLog2 %d out of range 0..%d", fn, params->normalPowerLog2, dn::kMaxNormalPowerLog2);
+    if (!(params->sigmaLuminance > 0.0f && params->sigmaLuminance <= 3.4028235e38f))
+        return tmpt::fail(TMPT_ERR_ARG, "%s: sigmaLuminance %g is not a finite value > 0", fn, (double)params->sigmaLuminance);
+    if (!(params->sigmaDepth > 0.0f && params->sigmaDepth <= 3.4028235e38f))
+        return tmpt::fail(TMPT_ERR_ARG, "%s: sigmaDepth %g is not a finite value > 0", fn, (double)params->sigmaDepth);
+    std::lock_guard<std::mutex> lock(s->hostCallMutex);
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "%s: cudaSetDevice(%d) failed", fn, s->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    const size_t pixels = (size_t)width * height;
+    const size_t bytes[3] = {pixels * sizeof(float4), pixels * sizeof(float4), pixels * sizeof(float)};  // radiance, normal, depth
+    const void* user[3] = {in->radiance, in->normal, in->depth};
+    const void* dev[3] = {in->radiance, in->normal, in->depth};
+    uchar4* rgba = (uchar4*)out->rgba;
+    float4* radiance = (float4*)out->radiance;
+    // (scratch allocation stays outside the timed window)
+    if (mem == TMPT_HOST) {
+        for (int k = 0; k < 3; ++k) {
+            const int rc = grow_scratch(&s->d_outs[k], &s->outsBytes[k], bytes[k]);  // tmpt_render_outputs' staging of the same buffers
+            if (rc != TMPT_OK) return rc;
+            dev[k] = s->d_outs[k];
+        }
+        if (rgba) {
+            const int rc = grow_scratch((void**)&s->d_frame, &s->frameBytes, pixels * 4);
+            if (rc != TMPT_OK) return rc;
+            rgba = (uchar4*)s->d_frame;
+        }
+        if (radiance) radiance = (float4*)s->d_outs[0];  // the staged input: read by the prologue (or the copy) before this is written
+    }
+    if (params->iterations > 0) {
+        const int rc = grow_scratch((void**)&s->d_denoise, &s->denoiseBytes, 4 * pixels * sizeof(float4));
+        if (rc != TMPT_OK) return rc;
+    }
+    CU_TRY(cudaEventRecord(s->ev0, st));
+    if (mem == TMPT_HOST)
+        for (int k = 0; k < 3; ++k) CU_TRY(cudaMemcpyAsync((void*)dev[k], user[k], bytes[k], cudaMemcpyHostToDevice, st));
+    const float4* rin = (const float4*)dev[0];
+    if (params->iterations == 0) {
+        LAUNCH(k_denoise_copy, div_up((long long)pixels, 256), 256, 0, st, rin, (long long)pixels, rgba, radiance);
+    } else {
+        float4 *state[2] = {s->d_denoise, s->d_denoise + pixels}, *guideA = s->d_denoise + 2 * pixels, *guideB = s->d_denoise + 3 * pixels;
+        const dim3 grid(div_up(width, kDenoiseBX), div_up(height, kDenoiseBY)), block(kDenoiseBX, kDenoiseBY);
+        const dn::Params prm{params->iterations, params->sigmaLuminance, params->sigmaDepth, params->normalPowerLog2};
+        LAUNCH(k_denoise_prep, grid, block, 0, st, rin, (const float4*)dev[1], (const float*)dev[2], width, height, state[0], guideA, guideB);
+        for (int i = 0; i < params->iterations; ++i) {
+            if (i + 1 < params->iterations)
+                LAUNCH(k_denoise_atrous<false>, grid, block, 0, st, state[i & 1], state[(i + 1) & 1], guideA, guideB, width, height, 1 << i, prm,
+                       nullptr, nullptr);
+            else
+                LAUNCH(k_denoise_atrous<true>, grid, block, 0, st, state[i & 1], nullptr, guideA, guideB, width, height, 1 << i, prm, rgba, radiance);
+        }
+    }
+    CU_TRY(cudaGetLastError());
+    if (mem == TMPT_HOST) {
+        if (out->rgba) CU_TRY(cudaMemcpyAsync(out->rgba, rgba, pixels * 4, cudaMemcpyDeviceToHost, st));
+        if (out->radiance) CU_TRY(cudaMemcpyAsync(out->radiance, radiance, bytes[0], cudaMemcpyDeviceToHost, st));
+    }
+    CU_TRY(cudaEventRecord(s->ev1, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    float ms = 0.0f;
+    CU_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    if (seconds) *seconds = (double)ms * 1.0e-3;
+    return TMPT_OK;
+}
+
 extern "C" int tmpt_render_multi(tmpt_scene* const* scenes, int nScenes, const tmpt_camera* camera, int width, int height, int spp, uint8_t* rgba,
                                  uint64_t* rayCount, double* seconds) {
     if (!scenes || nScenes < 1 || nScenes > 64) return tmpt::fail(TMPT_ERR_ARG, "tmpt_render_multi: bad scene list");
