@@ -85,6 +85,52 @@ extern "C" int tmpt_device_count(void) {
 static inline int div_up(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 // ------------------------------------------------------------------------------------------
+// owned memory: every device and pinned host allocation of a scene or a call
+// ------------------------------------------------------------------------------------------
+namespace {
+struct DeviceMem {
+    static cudaError_t alloc(void** p, size_t bytes) { return cudaMalloc(p, bytes); }
+    static void free(void* p) { cudaFree(p); }
+};
+struct PinnedMem {  // page-locked host memory: asynchronous copies to and from it
+    static cudaError_t alloc(void** p, size_t bytes) { return cudaHostAlloc(p, bytes, cudaHostAllocDefault); }
+    static void free(void* p) { cudaFreeHost(p); }
+};
+// n elements of T: freed by the destructor, grown (not shrunk) on demand and reused, contents not preserved.
+template <class T, class Mem = DeviceMem>
+struct DevBuf {
+    T* p = nullptr;
+    size_t cap = 0;  // elements
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) { reset(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    void reset() { if (p) Mem::free(p); p = nullptr; cap = 0; }
+    // Room for at least n elements (at least 1).  Growing first waits for `st`, where work may still use the old memory, and
+    // allocates max(n, allocN) elements.  A failed allocation leaves the buffer empty, so the next call tries again.
+    cudaError_t grow(size_t n, cudaStream_t st, size_t allocN = 0) {
+        n = std::max<size_t>(n, 1);
+        if (cap >= n) return cudaSuccess;
+        if (p) {
+            const cudaError_t e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) return e;
+        }
+        reset();
+        n = std::max(n, allocN);
+        const cudaError_t e = Mem::alloc((void**)&p, n * sizeof(T));
+        if (e != cudaSuccess) { p = nullptr; return e; }
+        cap = n;
+        return cudaSuccess;
+    }
+};
+template <class T>
+using PinnedBuf = DevBuf<T, PinnedMem>;
+}  // namespace
+
+// ------------------------------------------------------------------------------------------
 // the scene object behind tmpt_scene*
 // ------------------------------------------------------------------------------------------
 struct tmpt_scene {
@@ -92,60 +138,56 @@ struct tmpt_scene {
     int triCount = 0;
     int smCount = 148;
     cudaStream_t stream = nullptr;
-    float* d_tris9 = nullptr;      // caller's triangles, original order
-    float4* d_nodes = nullptr;     // wide nodes, 7 x float4 each: what the walk reads
-    uint4* d_qnodes = nullptr;     // wide nodes, quantised: only in a -DTMPT_QNODES=1 build (an experiment, not the default)
+    DevBuf<float> d_tris9;         // caller's triangles, original order
+    DevBuf<float4> d_nodes;        // wide nodes, 7 x float4 each: what the walk reads; then the views below
+    DevBuf<uint4> d_qnodes;        // wide nodes, quantised: only in a -DTMPT_QNODES=1 build (an experiment, not the default)
     float4* d_tris = nullptr;      // leaf-ordered MT slots
     float4* d_hitdata = nullptr;   // per original triangle: vertices + precomputed normal
     uint32_t* d_parent = nullptr;  // per wide node: parent index (refit)
     uint32_t* d_pending = nullptr; // per wide node: inner children not yet refitted (refit scratch)
     uint32_t* d_bounds = nullptr;  // scene bounds as ordered uints (refit scratch)
-    uint32_t* d_status = nullptr;  // [0] status bits
+    DevBuf<uint32_t> d_status;     // [0] status bits
     // render scratch
-    uint32_t* d_tileCounter = nullptr;
-    unsigned long long* d_rayCount = nullptr;
-    unsigned long long* d_fetchCounter = nullptr;  // ray queue head of the persistent HitScene kernel
-    uint8_t* d_frame = nullptr;
-    size_t frameBytes = 0;
-    float4* d_accum = nullptr;     // chunk sums of the band being rendered
-    size_t accumBytes = 0;
-    float4* d_sum = nullptr;       // progressive render: running per-pixel sums
-    size_t sumBytes = 0;
-    void* d_outs[4] = {};          // tmpt_render_outputs(TMPT_HOST): radiance, normal, depth, triangle staged on the device
-    size_t outsBytes[4] = {};
+    DevBuf<uint32_t> d_tileCounter;
+    DevBuf<unsigned long long> d_rayCount;
+    DevBuf<unsigned long long> d_fetchCounter;  // ray queue head of the persistent HitScene kernel
+    // rgba, radiance, normal, depth, triangle staged on the device (indexed like Staging::user): tmpt_render_outputs(TMPT_HOST)
+    // and tmpt_denoise(TMPT_HOST); [0] is also the frame of a call that asks for none, and tmpt_render_multi's frame
+    DevBuf<char> staged[5];
+    DevBuf<float4> d_accum;        // chunk sums of the band being rendered
+    DevBuf<float4> d_sum;          // progressive render: running per-pixel sums
     int progW = 0, progH = 0, progChunks = -1;  // -1: no progressive render begun
     int progAdaptive = -1;         // the session's kind, fixed by its first pass: -1 none yet, 0 uniform, 1 adaptive
-    // adaptive passes (tmpt_progressive_pass_adaptive), allocated by a session's first adaptive pass: per pixel the chunk count
-    // and (mean, M2) of the chunk-mean luminance; the select flags, their exclusive scan and scan totals; the active list
-    uint32_t* d_adN = nullptr;
-    float2* d_adStat = nullptr;
-    uint32_t *d_adFlags = nullptr, *d_adOffs = nullptr, *d_adTotals = nullptr;  // d_adTotals: scan totals, then the grand total
-    uint2* d_adList = nullptr;
-    unsigned int* d_adActive = nullptr;  // [0] pixels left active by the pass, [1] the session's largest chunk count n
-    size_t adPixels = 0;           // capacity of the per-pixel buffers above (tile-padded frame)
-    int32_t* d_samples = nullptr;  // tmpt_progressive_pass_adaptive(TMPT_HOST): samples staged on the device
-    size_t samplesBytes = 0;
-    float4* d_denoise = nullptr;   // tmpt_denoise: [4][pixels] float4: two state buffers (ping-pong), guideA, guideB (denoise.cuh)
-    size_t denoiseBytes = 0;
+    // adaptive passes (tmpt_progressive_pass_adaptive), allocated by a session's first adaptive pass: per pixel (tile-padded
+    // frame) the chunk count and (mean, M2) of the chunk-mean luminance; the select flags, their exclusive scan and scan totals;
+    // the active list
+    DevBuf<uint32_t> d_adN;
+    DevBuf<float2> d_adStat;
+    DevBuf<uint32_t> d_adFlags, d_adOffs, d_adTotals;  // d_adTotals: scan totals, then the grand total
+    DevBuf<uint2> d_adList;
+    DevBuf<unsigned int> d_adActive;  // [0] pixels left active by the pass, [1] the session's largest chunk count n
+    DevBuf<int32_t> d_samples;     // tmpt_progressive_pass_adaptive(TMPT_HOST): samples staged on the device
+    DevBuf<float4> d_denoise;      // tmpt_denoise: [4][pixels] float4: two state buffers (ping-pong), guideA, guideB (denoise.cuh)
     // staging of tmpt_hit_scene(TMPT_HOST): one device and one pinned host buffer per scene, grown on demand and reused (the
     // entry point is called in a loop by batched-query users: five cudaMalloc / cudaFree pairs and pageable copies per call
     // cost more than the kernel for batches under a million rays)
-    char* d_stage = nullptr;
-    char* h_stage = nullptr;
-    size_t stageBytes = 0;
-    std::mutex hostCallMutex;      // serialises the entry points that use per-scene scratch (staging, frame, accum, counters)
-    uint32_t *d_sunStart = nullptr, *d_sunCount = nullptr;  // sun grid (sungrid.cuh): cell offsets; counts / fill cursors + scan scratch
-    uint2* d_sunEntries = nullptr;
-    uint32_t sunEntriesCap = 0, sunEntries = 0;
+    DevBuf<char> d_stage;
+    PinnedBuf<char> h_stage;
+    // serialises the entry points that use or reallocate per-scene scratch (staging, frame, accum, progressive sums, sun grid,
+    // counters) or the timing events ev0 / ev1
+    std::mutex hostCallMutex;
+    DevBuf<uint32_t> d_sunStart, d_sunCount;  // sun grid (sungrid.cuh): cell offsets; counts / fill cursors + scan scratch
+    DevBuf<uint2> d_sunEntries;
+    uint32_t sunEntries = 0;
     uint64_t sunBytes = 0;
-    size_t sunStartCap = 0, sunCountCap = 0;
     // render-kernel choice (k_render vs k_render_paths), cached per camera / frame size: see k_probe_paths
     tmpt_camera probeCam{};
     int probeW = 0, probeH = 0, probeUsePaths = -1;  // -1: no decision yet
     int lastUsedPaths = -1;                           // what the last frame ran (tmpt_render_kernel_choice)
     bool probePending = false;                        // a probe is in flight: h_probe is valid once probeDone has passed
     float probeEscape = 0.0f;
-    unsigned int *d_probe = nullptr, *h_probe = nullptr;  // device counters / their pinned copy
+    DevBuf<unsigned int> d_probe;  // device counters
+    PinnedBuf<unsigned int> h_probe;  // their pinned copy
     cudaEvent_t probeDone = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bvh::SceneView view{};
@@ -1391,12 +1433,6 @@ float bvh_far_limit(const tmpt_scene_info& info) {
     for (int k = 0; k < 3; ++k) m = std::max(m, std::max(std::fabs(info.bounds_min[k]), std::fabs(info.bounds_max[k])));
     return 16.0f * m;
 }
-template <class T>
-struct DevBuf {
-    T* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t alloc(size_t n) { return cudaMalloc((void**)&p, (n ? n : 1) * sizeof(T)); }
-};
 
 constexpr int kTreeTooDeep = -100;  // internal: tmpt_scene_create falls back to the depth-bounded default builder
 
@@ -1425,13 +1461,13 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
                             {&pHi, N * 16}, {&primFinal, N * 4}, {&nodeCounter, 4}, {&tqA, N * sizeof(SahTask)}, {&tqB, N * sizeof(SahTask)}};
         size_t total = 0;
         for (const Req& r : reqs) total += (r.bytes + 255) & ~(size_t)255;
-        CU_TRY(arena.alloc(total));
+        CU_TRY(arena.grow(total, st));
         size_t off = 0;
         for (const Req& r : reqs) { r.a->p = arena.p + off; off += (r.bytes + 255) & ~(size_t)255; }
     }
     // nodes, slots and hit payload share one allocation (each cudaMalloc costs as much as a build kernel)
-    CU_TRY(cudaMalloc((void**)&s->d_nodes, (size_t)n * (bvh::NODE_F4 + 3 + 3) * sizeof(float4) + ((size_t)n * 2 + 8) * sizeof(uint32_t)));
-    s->d_tris = s->d_nodes + (size_t)n * bvh::NODE_F4;
+    CU_TRY(s->d_nodes.grow((size_t)n * (bvh::NODE_F4 + 3 + 3) + div_up((long long)n * 2 + 8, sizeof(float4) / sizeof(uint32_t)), st));
+    s->d_tris = s->d_nodes.p + (size_t)n * bvh::NODE_F4;
     s->d_hitdata = s->d_tris + (size_t)n * 3;
     s->d_parent = (uint32_t*)(s->d_hitdata + (size_t)n * 3);
     s->d_pending = s->d_parent + n;
@@ -1452,19 +1488,19 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
     CU_TRY(cudaMemsetAsync(d_parent, 0xFF, 2 * (size_t)n * sizeof(int), st));
 
     const int B = 256, G = div_up(n, B);
-    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9, n, d_bounds);
-    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9, n, s->d_hitdata);
+    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9.p, n, d_bounds);
+    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9.p, n, s->d_hitdata);
     bld::BinTree t{n, d_keysA, d_left, d_right, d_parent, d_lo, d_hi, d_first, d_visits};
     bld::SahParams sp{cInner, cTri, maxLeaf};
     const uint32_t* primOrder = d_primA;
     int rootIsLeaf = (n == 1);
     if (flags & TMPT_BUILD_LBVH) {
-        LAUNCH(k_morton, G, B, 0, st, s->d_tris9, n, d_bounds, d_keysA, d_primA);
+        LAUNCH(k_morton, G, B, 0, st, s->d_tris9.p, n, d_bounds, d_keysA, d_primA);
         const int passes = 16;  // 63-bit keys, 4 bits per pass; an even count leaves the result in A
         const int sortSmem = 16 * SORT_THREADS * (int)sizeof(uint32_t);
         CU_TRY(cudaFuncSetAttribute(k_radix_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, sortSmem));
         LAUNCH(k_radix_sort, 1, SORT_THREADS, sortSmem, st, d_keysA, d_primA, d_keysB, d_primB, n, passes);
-        LAUNCH(k_leaf_boxes, G, B, 0, st, s->d_tris9, d_primA, n, d_bounds, cTri, d_lo, d_hi, d_first);
+        LAUNCH(k_leaf_boxes, G, B, 0, st, s->d_tris9.p, d_primA, n, d_bounds, cTri, d_lo, d_hi, d_first);
         if (n > 1) {
             LAUNCH(k_karras, div_up(n - 1, B), B, 0, st, t);
             LAUNCH(k_refit, G, B, 0, st, t, sp);
@@ -1475,7 +1511,7 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         float4* const d_pLo = (float4*)pLo.p; float4* const d_pHi = (float4*)pHi.p;
         uint32_t* const d_primFinal = (uint32_t*)primFinal.p; uint32_t* const d_nodeCounter = (uint32_t*)nodeCounter.p;
         SahTask* const d_tqA = (SahTask*)tqA.p; SahTask* const d_tqB = (SahTask*)tqB.p;
-        LAUNCH(k_prim_boxes, G, B, 0, st, s->d_tris9, n, d_bounds, d_pLo, d_pHi, d_primA);
+        LAUNCH(k_prim_boxes, G, B, 0, st, s->d_tris9.p, n, d_bounds, d_pLo, d_pHi, d_primA);
         const SahTask rootTask{0, 0, n, 0};
         const uint32_t one = 1, zero = 0;
         CU_TRY(cudaMemcpyAsync(d_tqA, &rootTask, sizeof rootTask, cudaMemcpyHostToDevice, st));
@@ -1493,7 +1529,7 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
             uint32_t* countsP = d_qCount; uint32_t* nodeCounterP = d_nodeCounter; uint32_t* primFinalP = d_primFinal;
             const float4* pLoP = d_pLo; const float4* pHiP = d_pHi;
             int maxLevels = 4096;
-            uint32_t* statusP = s->d_status + 1;
+            uint32_t* statusP = s->d_status.p + 1;
             void* args[] = {&t, &pLoP, &pHiP, &idxA, &idxB, &primFinalP, &qA, &qB, &countsP, &nodeCounterP, &sp, &maxLevels, &statusP};
             // (a refused cooperative launch -- e.g. the device is shared and the grid cannot be co-resident -- is not an error:
             //  nothing has run yet, the per-level loop below does the same work)
@@ -1523,12 +1559,12 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         CU_TRY(cudaMemcpyAsync(d_primA, d_primFinal, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
         s->info.builder = TMPT_BUILD_DEFAULT;
     }
-    bld::WideOut w{s->d_nodes, s->d_tris, s->d_tris9, primOrder, d_counters, d_sah, s->d_parent};
+    bld::WideOut w{s->d_nodes.p, s->d_tris, s->d_tris9.p, primOrder, d_counters, d_sah, s->d_parent};
     if (n > 1) {
         float4 rootHi;
         uint32_t bst = 0;
         CU_TRY(cudaMemcpyAsync(&rootHi, d_hi, sizeof rootHi, cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaMemcpyAsync(&bst, s->d_status + 1, 4, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaMemcpyAsync(&bst, s->d_status.p + 1, 4, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         if (bst & 2u) return tmpt::fail(TMPT_ERR_CUDA, "SAH build did not terminate");
         int c; memcpy(&c, &rootHi.w, 4);
@@ -1598,8 +1634,8 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
     }
     if ((int)hc[1] != n) return tmpt::fail(TMPT_ERR_CUDA, "BVH build lost triangles: %u slots for %d triangles", hc[1], n);
 #if TMPT_QNODES
-    CU_TRY(cudaMalloc((void**)&s->d_qnodes, ((size_t)hc[0] * bvh::QNODE_STRIDE) * sizeof(uint4)));
-    LAUNCH(k_quantize_nodes, div_up((int)hc[0], 128), 128, 0, st, s->d_nodes, s->d_qnodes, hc[0]);
+    CU_TRY(s->d_qnodes.grow((size_t)hc[0] * bvh::QNODE_STRIDE, st));
+    LAUNCH(k_quantize_nodes, div_up((int)hc[0], 128), 128, 0, st, s->d_nodes.p, s->d_qnodes.p, hc[0]);
 #endif
     // the traversal stack holds at most 3 entries per level (bvh::wide_node_step): refuse what it could not hold.  The default
     // builder cannot get here (bld::sah_must_halve bounds its depth for any input); a Morton tree over many coincident centres can.
@@ -1609,14 +1645,14 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         return kTreeTooDeep;
     }
     s->info.device_bytes = (uint64_t)n * 9 * 4 + (uint64_t)hc[0] * (bvh::NODE_F4 + (TMPT_QNODES ? bvh::QNODE_STRIDE : 0)) * 16 + (uint64_t)n * 48 + (uint64_t)n * 48;
-    s->view.nodes = s->d_nodes;
-    s->view.qnodes = s->d_qnodes;
+    s->view.nodes = s->d_nodes.p;
+    s->view.qnodes = s->d_qnodes.p;
     s->view.tris = s->d_tris;
-    s->view.tris9 = s->d_tris9;
+    s->view.tris9 = s->d_tris9.p;
     s->view.hitdata = s->d_hitdata;
     s->view.rootRef = 0u;
     s->view.triCount = n;
-    s->view.status = s->d_status;
+    s->view.status = s->d_status.p;
     s->view.farLimit = bvh_far_limit(s->info);
     return TMPT_OK;
 }
@@ -1645,49 +1681,37 @@ static int build_sun_grid(tmpt_scene* s, int n, cudaStream_t st) {  // (after th
         const long long nCells = (long long)cells * cells;
         const int nBlocks = (int)((nCells + kScanBlock - 1) / kScanBlock);
         const size_t needStart = (size_t)nCells + 1, needCount = (size_t)nCells + nBlocks + 2 + n;
-        if (s->sunStartCap < needStart) {  // (a refit finds its buffers in place)
-            cudaFree(s->d_sunStart); s->d_sunStart = nullptr; s->sunStartCap = 0;
-            CU_TRY(cudaMalloc((void**)&s->d_sunStart, needStart * sizeof(uint32_t)));
-            s->sunStartCap = needStart;
-        }
-        if (s->sunCountCap < needCount) {
-            cudaFree(s->d_sunCount); s->d_sunCount = nullptr; s->sunCountCap = 0;
-            CU_TRY(cudaMalloc((void**)&s->d_sunCount, needCount * sizeof(uint32_t)));
-            s->sunCountCap = needCount;
-        }
-        uint32_t* totals = s->d_sunCount + nCells;
+        CU_TRY(s->d_sunStart.grow(needStart, st));  // (a refit finds its buffers in place)
+        CU_TRY(s->d_sunCount.grow(needCount, st));
+        uint32_t* totals = s->d_sunCount.p + nCells;
         uint32_t* grand = totals + nBlocks;
         uint32_t* bigCount = grand + 1;
         uint32_t* bigList = bigCount + 1;  // up to n slots
-        CU_TRY(cudaMemsetAsync(s->d_sunCount, 0, (size_t)(nCells + nBlocks + 2) * sizeof(uint32_t), st));
+        CU_TRY(cudaMemsetAsync(s->d_sunCount.p, 0, (size_t)(nCells + nBlocks + 2) * sizeof(uint32_t), st));
         const int binGrid = (int)(((long long)n * 32 + 255) / 256), bigGrid = s->smCount * 8;
-        LAUNCH((k_sun_bin<false>), binGrid, 256, 0, st, g, s->d_tris, s->d_tris9, n, s->d_sunCount, nullptr, nullptr, bigList, bigCount);
-        LAUNCH((k_sun_bin_big<false>), bigGrid, 256, 0, st, g, s->d_tris, s->d_tris9, s->d_sunCount, nullptr, nullptr, bigList, bigCount);
-        LAUNCH(k_scan_totals, nBlocks, kScanBlock, 0, st, s->d_sunCount, nCells, totals);
+        LAUNCH((k_sun_bin<false>), binGrid, 256, 0, st, g, s->d_tris, s->d_tris9.p, n, s->d_sunCount.p, nullptr, nullptr, bigList, bigCount);
+        LAUNCH((k_sun_bin_big<false>), bigGrid, 256, 0, st, g, s->d_tris, s->d_tris9.p, s->d_sunCount.p, nullptr, nullptr, bigList, bigCount);
+        LAUNCH(k_scan_totals, nBlocks, kScanBlock, 0, st, s->d_sunCount.p, nCells, totals);
         LAUNCH(k_scan_of_totals, 1, kScanBlock, 0, st, totals, nBlocks, grand);
-        LAUNCH(k_scan_apply, nBlocks, kScanBlock, 0, st, s->d_sunCount, nCells, totals, grand, s->d_sunStart);
+        LAUNCH(k_scan_apply, nBlocks, kScanBlock, 0, st, s->d_sunCount.p, nCells, totals, grand, s->d_sunStart.p);
         uint32_t total = 0;
         const double t2 = now();
         CU_TRY(cudaMemcpyAsync(&total, grand, sizeof total, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         const double t3 = now();
         if ((unsigned long long)total > kSunMaxEntries) continue;  // halve the grid
-        if (s->sunEntriesCap < total) {
-            cudaFree(s->d_sunEntries); s->d_sunEntries = nullptr; s->sunEntriesCap = 0;
-            CU_TRY(cudaMalloc((void**)&s->d_sunEntries, (size_t)std::max<uint32_t>(total, 1u) * sizeof(uint2)));
-            s->sunEntriesCap = std::max<uint32_t>(total, 1u);
-        }
-        CU_TRY(cudaMemsetAsync(s->d_sunCount, 0, (size_t)nCells * sizeof(uint32_t), st));
-        LAUNCH((k_sun_bin<true>), binGrid, 256, 0, st, g, s->d_tris, s->d_tris9, n, s->d_sunCount, s->d_sunStart, s->d_sunEntries, bigList, bigCount);
-        LAUNCH((k_sun_bin_big<true>), bigGrid, 256, 0, st, g, s->d_tris, s->d_tris9, s->d_sunCount, s->d_sunStart, s->d_sunEntries, bigList, bigCount);
-        LAUNCH(k_sun_sort, (int)((nCells + 127) / 128), 128, 0, st, s->d_sunStart, nCells, s->d_sunEntries);
+        CU_TRY(s->d_sunEntries.grow(total, st));
+        CU_TRY(cudaMemsetAsync(s->d_sunCount.p, 0, (size_t)nCells * sizeof(uint32_t), st));
+        LAUNCH((k_sun_bin<true>), binGrid, 256, 0, st, g, s->d_tris, s->d_tris9.p, n, s->d_sunCount.p, s->d_sunStart.p, s->d_sunEntries.p, bigList, bigCount);
+        LAUNCH((k_sun_bin_big<true>), bigGrid, 256, 0, st, g, s->d_tris, s->d_tris9.p, s->d_sunCount.p, s->d_sunStart.p, s->d_sunEntries.p, bigList, bigCount);
+        LAUNCH(k_sun_sort, (int)((nCells + 127) / 128), 128, 0, st, s->d_sunStart.p, nCells, s->d_sunEntries.p);
         if (trace) {
             CU_TRY(cudaStreamSynchronize(st));
             fprintf(stderr, "[sun grid] n %d entries %u: host setup %.2f ms, alloc + count launches %.2f ms, wait for the stream %.2f ms, alloc + fill + sort %.2f ms\n",
                     cells, total, t1 - t0, t2 - t1, t3 - t2, now() - t3);
         }
-        g.cellStart = s->d_sunStart;
-        g.entries = s->d_sunEntries;
+        g.cellStart = s->d_sunStart.p;
+        g.entries = s->d_sunEntries.p;
         s->view.sun = g;
         s->sunBytes = (uint64_t)(nCells + 1) * 4 + (uint64_t)total * 8;
         s->info.device_bytes += s->sunBytes;
@@ -1736,28 +1760,28 @@ extern "C" int tmpt_scene_create(const float* tris9, int triCount, int device, u
         CU_TRY(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
         CU_TRY(cudaEventCreate(&s->ev0));
         CU_TRY(cudaEventCreate(&s->ev1));
-        CU_TRY(cudaMalloc((void**)&s->d_status, 4 * sizeof(uint32_t)));
-        CU_TRY(cudaMemsetAsync(s->d_status, 0, 4 * sizeof(uint32_t), s->stream));
-        CU_TRY(cudaMalloc((void**)&s->d_tileCounter, sizeof(uint32_t)));
-        CU_TRY(cudaMalloc((void**)&s->d_rayCount, sizeof(unsigned long long)));
-        CU_TRY(cudaMalloc((void**)&s->d_fetchCounter, sizeof(unsigned long long)));
+        CU_TRY(s->d_status.grow(4, s->stream));
+        CU_TRY(cudaMemsetAsync(s->d_status.p, 0, 4 * sizeof(uint32_t), s->stream));
+        CU_TRY(s->d_tileCounter.grow(1, s->stream));
+        CU_TRY(s->d_rayCount.grow(1, s->stream));
+        CU_TRY(s->d_fetchCounter.grow(1, s->stream));
         CU_TRY(cudaEventRecord(s->ev0, s->stream));
         if (triCount > 0) {
-            CU_TRY(cudaMalloc((void**)&s->d_tris9, (size_t)triCount * 9 * sizeof(float)));
-            CU_TRY(cudaMemcpyAsync(s->d_tris9, tris9, (size_t)triCount * 9 * sizeof(float), cudaMemcpyHostToDevice, s->stream));
+            CU_TRY(s->d_tris9.grow((size_t)triCount * 9, s->stream));
+            CU_TRY(cudaMemcpyAsync(s->d_tris9.p, tris9, (size_t)triCount * 9 * sizeof(float), cudaMemcpyHostToDevice, s->stream));
             int brc = build_bvh(s, flags);
             if (brc == kTreeTooDeep && (flags & TMPT_BUILD_LBVH)) {
                 // a Morton tree can be arbitrarily deep (many coincident centres); the SAH builder bounds its depth for any input
                 CU_TRY(cudaStreamSynchronize(s->stream));
-                cudaFree(s->d_nodes); s->d_nodes = nullptr;
-                cudaFree(s->d_qnodes); s->d_qnodes = nullptr;
+                s->d_nodes.reset();
+                s->d_qnodes.reset();
                 brc = build_bvh(s, flags & ~(unsigned)TMPT_BUILD_LBVH);
             }
             if (brc != TMPT_OK) return brc == kTreeTooDeep ? TMPT_ERR_ARG : brc;
             brc = build_sun_grid(s, triCount, s->stream);
             if (brc != TMPT_OK) return brc;
         } else {
-            s->view = bvh::SceneView{nullptr, nullptr, nullptr, nullptr, bvh::NONE, 0, s->d_status, nullptr, 0.0f};
+            s->view = bvh::SceneView{nullptr, nullptr, nullptr, nullptr, bvh::NONE, 0, s->d_status.p, nullptr, 0.0f};
         }
         CU_TRY(cudaEventRecord(s->ev1, s->stream));
         CU_TRY(cudaStreamSynchronize(s->stream));
@@ -1780,20 +1804,21 @@ extern "C" int tmpt_scene_refit(tmpt_scene* s, const float* tris9, int triCount,
     if (triCount != s->triCount) return tmpt::fail(TMPT_ERR_ARG, "tmpt_scene_refit: %d triangles, the scene was built with %d", triCount, s->triCount);
     if (seconds) *seconds = 0.0;
     if (triCount == 0) return TMPT_OK;
+    std::lock_guard<std::mutex> lock(s->hostCallMutex);
     DeviceGuard guard(s->device);
     if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "tmpt_scene_refit: cudaSetDevice(%d) failed", s->device);
     cudaStream_t st = s->stream;
     const int n = triCount, B = 256, G = div_up(n, B), nodes = s->info.node_count;
     CU_TRY(cudaEventRecord(s->ev0, st));
-    CU_TRY(cudaMemcpyAsync(s->d_tris9, tris9, (size_t)n * 9 * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(s->d_tris9.p, tris9, (size_t)n * 9 * sizeof(float), cudaMemcpyHostToDevice, st));
     const uint32_t initBounds[6] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0u, 0u, 0u};
     CU_TRY(cudaMemcpyAsync(s->d_bounds, initBounds, sizeof initBounds, cudaMemcpyHostToDevice, st));
-    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9, n, s->d_bounds);
-    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9, n, s->d_hitdata);
-    LAUNCH(k_refit_pending, div_up(nodes, 128), 128, 0, st, s->d_nodes, (uint32_t)nodes, s->d_pending);
-    LAUNCH(k_refit_wide, div_up(nodes, 128), 128, 0, st, s->d_nodes, s->d_tris, s->d_tris9, s->d_parent, s->d_pending, (uint32_t)nodes, s->d_bounds);
+    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9.p, n, s->d_bounds);
+    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9.p, n, s->d_hitdata);
+    LAUNCH(k_refit_pending, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, (uint32_t)nodes, s->d_pending);
+    LAUNCH(k_refit_wide, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, s->d_tris, s->d_tris9.p, s->d_parent, s->d_pending, (uint32_t)nodes, s->d_bounds);
 #if TMPT_QNODES
-    LAUNCH(k_quantize_nodes, div_up(nodes, 128), 128, 0, st, s->d_nodes, s->d_qnodes, (uint32_t)nodes);
+    LAUNCH(k_quantize_nodes, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, s->d_qnodes.p, (uint32_t)nodes);
 #endif
     uint32_t hb[6];
     CU_TRY(cudaMemcpyAsync(hb, s->d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
@@ -1822,21 +1847,11 @@ extern "C" void tmpt_scene_destroy(tmpt_scene* s) {
     if (!s) return;
     DeviceGuard guard(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
-    cudaFree(s->d_tris9); cudaFree(s->d_nodes); cudaFree(s->d_qnodes); cudaFree(s->d_status);  // (d_tris, d_hitdata live inside d_nodes)
-    cudaFree(s->d_tileCounter); cudaFree(s->d_rayCount); cudaFree(s->d_fetchCounter); cudaFree(s->d_frame); cudaFree(s->d_accum); cudaFree(s->d_sum);
-    for (void* o : s->d_outs) cudaFree(o);
-    cudaFree(s->d_adN); cudaFree(s->d_adStat); cudaFree(s->d_adFlags); cudaFree(s->d_adOffs); cudaFree(s->d_adTotals); cudaFree(s->d_adList);
-    cudaFree(s->d_adActive); cudaFree(s->d_samples); cudaFree(s->d_denoise);
-    cudaFree(s->d_stage);
-    cudaFree(s->d_probe);
-    cudaFree(s->d_sunStart); cudaFree(s->d_sunCount); cudaFree(s->d_sunEntries);
-    if (s->h_probe) cudaFreeHost(s->h_probe);
     if (s->probeDone) cudaEventDestroy(s->probeDone);
-    if (s->h_stage) cudaFreeHost(s->h_stage);
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
     if (s->stream) cudaStreamDestroy(s->stream);
-    delete s;
+    delete s;  // (its buffers free their memory while the guard holds the scene's device)
 }
 
 extern "C" int tmpt_scene_get_info(const tmpt_scene* s, tmpt_scene_info* out) {
@@ -1847,7 +1862,7 @@ extern "C" int tmpt_scene_get_info(const tmpt_scene* s, tmpt_scene_info* out) {
 
 static int check_status(const tmpt_scene* s, cudaStream_t st) {
     uint32_t status = 0;
-    CU_TRY(cudaMemcpyAsync(&status, s->d_status, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&status, s->d_status.p, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     if (status & bvh::STACK_OVERFLOW) return tmpt::fail(TMPT_ERR_CUDA, "traversal stack overflow (BVH depth %d)", s->info.max_depth);
     return TMPT_OK;
@@ -1877,17 +1892,9 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
     if (mem == TMPT_HOST) {
         lock.lock();
         tmpt_scene* ms = const_cast<tmpt_scene*>(s);  // scratch only
-        if (ms->stageBytes < total) {
-            CU_TRY(cudaStreamSynchronize(ms->stream));
-            cudaFree(ms->d_stage); ms->d_stage = nullptr;
-            if (ms->h_stage) { cudaFreeHost(ms->h_stage); ms->h_stage = nullptr; }
-            ms->stageBytes = 0;
-            const size_t cap = total + total / 4;
-            CU_TRY(cudaMalloc((void**)&ms->d_stage, cap));
-            CU_TRY(cudaHostAlloc((void**)&ms->h_stage, cap, cudaHostAllocDefault));
-            ms->stageBytes = cap;
-        }
-        char* h = ms->h_stage; char* d = ms->d_stage;
+        CU_TRY(ms->d_stage.grow(total, ms->stream, total + total / 4));
+        CU_TRY(ms->h_stage.grow(total, ms->stream, total + total / 4));
+        char* h = ms->h_stage.p; char* d = ms->d_stage.p;
         memcpy(h, rays6, 6 * n * 4);
         if (outT) memcpy(h + offT, outT, n * 4);
         if (outPos3) memcpy(h + offPos, outPos3, 3 * n * 4);
@@ -1904,13 +1911,13 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
 #if TMPT_EXPERIMENTS
     static const int refillGate = getenv("TMPT_HIT_REFILL") ? atoi(getenv("TMPT_HIT_REFILL")) : 0;
     if (refillGate > 0 && mode != TMPT_HIT_BRUTE) {
-        CU_TRY(cudaMemsetAsync(s->d_fetchCounter, 0, sizeof(unsigned long long), st));
+        CU_TRY(cudaMemsetAsync(s->d_fetchCounter.p, 0, sizeof(unsigned long long), st));
         int perSM = 0;
 #define REFILL_CASE(M, GT)                                                                                                     \
         if (mode == M && refillGate == GT) {                                                                                   \
             CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_hit_scene_refill<M, GT>, B, 0));                    \
             const int GP = (int)std::min<long long>(div_up(nRays, B), (long long)s->smCount * std::max(perSM, 1));            \
-            LAUNCH((k_hit_scene_refill<M, GT>), GP, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, s->d_fetchCounter); \
+            LAUNCH((k_hit_scene_refill<M, GT>), GP, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, s->d_fetchCounter.p); \
         } else
         REFILL_CASE(TMPT_HIT_CLOSEST, 1) REFILL_CASE(TMPT_HIT_CLOSEST, 4) REFILL_CASE(TMPT_HIT_CLOSEST, 8) REFILL_CASE(TMPT_HIT_CLOSEST, 16)
         REFILL_CASE(TMPT_HIT_ANY, 1) REFILL_CASE(TMPT_HIT_ANY, 4) REFILL_CASE(TMPT_HIT_ANY, 8) REFILL_CASE(TMPT_HIT_ANY, 16)
@@ -1924,7 +1931,7 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
     else LAUNCH((k_hit_scene<TMPT_HIT_BRUTE, false>), G, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
     CU_TRY(cudaGetLastError());
     if (mem == TMPT_HOST) {
-        const char* d = s->d_stage; char* h = s->h_stage;
+        const char* d = s->d_stage.p; char* h = s->h_stage.p;
         CU_TRY(cudaMemcpyAsync(h + offID, d + offID, total - offID, cudaMemcpyDeviceToHost, st));  // id | t | pos | normal in one copy
         CU_TRY(cudaStreamSynchronize(st));
         memcpy(outID, h + offID, n * 4);
@@ -2025,12 +2032,7 @@ static int prepare_accum(tmpt_scene* s, const RenderPlan& pl, cudaStream_t st, i
         const size_t unitBytes = (size_t)pl.unitWidth * pl.chunks * pl.planes * sizeof(float4), budget = (size_t)4 << 30;
         band = (int)std::min<size_t>((size_t)pl.units, std::max<size_t>(pl.granule, (budget / unitBytes) & ~(size_t)(pl.granule - 1)));
         const size_t need = (size_t)band * unitBytes;
-        if (s->accumBytes < need) {
-            CU_TRY(cudaStreamSynchronize(st));
-            cudaFree(s->d_accum); s->d_accum = nullptr; s->accumBytes = 0;
-            CU_TRY(cudaMalloc((void**)&s->d_accum, need));
-            s->accumBytes = need;
-        }
+        CU_TRY(s->d_accum.grow(need / sizeof(float4), st));
     }
     if (outBandUnits) *outBandUnits = band;
     return TMPT_OK;
@@ -2047,21 +2049,21 @@ static int choose_render_kernel(tmpt_scene* s, const tmpt_camera* camera, const 
     static const int pathsEnv = getenv("TMPT_RENDER_PATHS") ? atoi(getenv("TMPT_RENDER_PATHS")) : -1;
     *usePaths = pathsEnv > 0;
     if (pathsEnv >= 0 || s->triCount == 0) return TMPT_OK;
-    if (!s->d_probe) {
-        CU_TRY(cudaMalloc((void**)&s->d_probe, 4 * sizeof(unsigned int)));
-        CU_TRY(cudaMallocHost((void**)&s->h_probe, 4 * sizeof(unsigned int)));
+    if (!s->probeDone) {
+        CU_TRY(s->d_probe.grow(4, st));
+        CU_TRY(s->h_probe.grow(4, st));
         CU_TRY(cudaEventCreateWithFlags(&s->probeDone, cudaEventDisableTiming));
     }
     auto consume = [&]() {
-        s->probeEscape = s->h_probe[1] ? (float)s->h_probe[2] / (float)s->h_probe[1] : 1.0f;  // (no camera ray hits anything: open)
+        s->probeEscape = s->h_probe.p[1] ? (float)s->h_probe.p[2] / (float)s->h_probe.p[1] : 1.0f;  // (no camera ray hits anything: open)
         s->probeUsePaths = s->probeEscape > kOpenFrame ? 1 : 0;
         s->probePending = false;
     };
     if (s->probePending && cudaEventQuery(s->probeDone) == cudaSuccess) consume();
     if (!s->probePending && (s->probeUsePaths < 0 || s->probeW != width || s->probeH != height || memcmp(&s->probeCam, camera, sizeof(tmpt_camera)) != 0)) {
-        CU_TRY(cudaMemsetAsync(s->d_probe, 0, 4 * sizeof(unsigned int), st));
-        LAUNCH(k_probe_paths, 32, 128, 0, st, s->view, cam, width, height, s->d_probe);
-        CU_TRY(cudaMemcpyAsync(s->h_probe, s->d_probe, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaMemsetAsync(s->d_probe.p, 0, 4 * sizeof(unsigned int), st));
+        LAUNCH(k_probe_paths, 32, 128, 0, st, s->view, cam, width, height, s->d_probe.p);
+        CU_TRY(cudaMemcpyAsync(s->h_probe.p, s->d_probe.p, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaEventRecord(s->probeDone, st));
         s->probeCam = *camera; s->probeW = width; s->probeH = height;
         s->probePending = true;
@@ -2138,8 +2140,8 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     p.outStripes = (uchar4*)outStripes;
     p.frame = (uchar4*)frame;
     p.rayCount = rayCountDev;
-    p.tileCounter = s->d_tileCounter;
-    p.laneCounter = s->d_fetchCounter;
+    p.tileCounter = s->d_tileCounter.p;
+    p.laneCounter = s->d_fetchCounter.p;
     p.stats = statsDev;
     p.accum = nullptr;
     p.list = nullptr;
@@ -2147,7 +2149,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     if (pl.units == 0) return TMPT_OK;  // (an adaptive pass with an empty list traces nothing: the kernel choice stays the last frame's)
     int band = 0;
     TRY(prepare_accum(s, pl, st, &band));
-    p.accum = s->d_accum;
+    p.accum = s->d_accum.p;
     // 32 warps per SM at 64 registers (sweep in profiles/r1_tuning_sweeps.txt: 24 warps at 77 registers is 10 % slower, 40
     // warps at 48 registers spills and is 3 % slower), as ONE 1024-thread CTA per SM when the band has work for every SM
     // several times over (+1.6 % over four 256-thread CTAs: 5016 vs 4937 Mrays/s), as 256-thread CTAs for small frames, whose
@@ -2173,7 +2175,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     for (int b0 = 0; b0 < pl.units; b0 += band) {
         const int here = std::min(band, pl.units - b0);
         if (pl.mode == OutMode::List) {
-            p.list = s->d_adList + b0;
+            p.list = s->d_adList.p + b0;
             p.listLen = here;
             p.numTiles = div_up(here, 32);
         } else {
@@ -2183,7 +2185,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         }
         const long long items = (long long)p.numTiles * p.chunks;
         if (items >= 0xFFFFFFFFll) return tmpt::fail(TMPT_ERR_ARG, "render: too many work items in one band");
-        CU_TRY(cudaMemsetAsync(s->d_tileCounter, 0, sizeof(uint32_t), st));
+        CU_TRY(cudaMemsetAsync(s->d_tileCounter.p, 0, sizeof(uint32_t), st));
 #if TMPT_TUNE_CFG
         if (cfgEnv >= 4 && cfgEnv <= 8) {  // tuning only (-DTMPT_TUNE_CFG=1): other resident-warp / register-budget points
             if (cfgEnv == 4) LAUNCH((k_render<false, 768, 1, 0>), s->smCount, 768, 0, st, p);           // 24 warps, 85 registers
@@ -2195,7 +2197,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
 #endif
 #if TMPT_EXPERIMENTS
         if (rk > 0 && !statsDev) {
-            CU_TRY(cudaMemsetAsync(s->d_fetchCounter, 0, sizeof(unsigned long long), st));
+            CU_TRY(cudaMemsetAsync(s->d_fetchCounter.p, 0, sizeof(unsigned long long), st));
             int perSMr = 0;
 #define REGEN_CASE(V, TA, TB)                                                                                        \
             if (rk == V) {                                                                                           \
@@ -2226,7 +2228,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
             }
             const RenderKernel k = render_kernel(pl.mode, usePaths, cfg, farCamera, statsDev != nullptr);
             TRY(render_blocks_per_sm(k, &perSM[cfg]));
-            if (usePaths) CU_TRY(cudaMemsetAsync(s->d_fetchCounter, 0, sizeof(unsigned long long), st));  // one (pixel, chunk) item per lane
+            if (usePaths) CU_TRY(cudaMemsetAsync(s->d_fetchCounter.p, 0, sizeof(unsigned long long), st));  // one (pixel, chunk) item per lane
             // every SM's resident CTAs, or fewer when a warp per (tile, chunk) item (k_render) or a lane per (pixel, chunk) item
             // (k_render_paths, 32 per tile) needs fewer
             const int warps = k.threads / 32;
@@ -2234,8 +2236,8 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
             LAUNCH(k.fn, grid, k.threads, k.smem, st, p);
         }
         if (pl.mode == OutMode::List)
-            LAUNCH(k_resolve_adaptive, div_up(here, 256), 256, 0, st, p, prog->sum, s->d_adN, s->d_adStat, prog->adaptive->tolerance,
-                   prog->adaptive->minChunks, s->d_adActive);
+            LAUNCH(k_resolve_adaptive, div_up(here, 256), 256, 0, st, p, prog->sum, s->d_adN.p, s->d_adStat.p, prog->adaptive->tolerance,
+                   prog->adaptive->minChunks, s->d_adActive.p);
         else if (p.useAccum && pl.mode == OutMode::Aov) LAUNCH(k_resolve<true>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p, here);
         else if (p.useAccum) LAUNCH(k_resolve<false>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p, here);
     }
@@ -2278,14 +2280,6 @@ static int check_outputs(const char* fn, const tmpt_outputs* out, int mem) {
     return TMPT_OK;
 }
 
-static int grow_scratch(void** p, size_t* cap, size_t need) {
-    if (*cap >= need) return TMPT_OK;
-    cudaFree(*p); *p = nullptr; *cap = 0;
-    CU_TRY(cudaMalloc(p, need));
-    *cap = need;
-    return TMPT_OK;
-}
-
 // The buffers rgba, radiance, normal, depth, triangle of a call as the kernels see them.  With TMPT_HOST each buffer the caller gave
 // is staged in the scene's device scratch (one buffer per kind, kept with the scene), and the caller copies it in or out inside its
 // timed window; with TMPT_DEVICE the kernels use the caller's buffers.
@@ -2294,15 +2288,14 @@ struct Staging {
     void* dev[5] = {};
     size_t bytes[5] = {};
     // frame: the kernels write an RGBA frame even when the caller asks for none (into the scene's scratch frame)
-    int stage(tmpt_scene* s, size_t pixels, int mem, bool frame) {
+    int stage(tmpt_scene* s, size_t pixels, int mem, bool frame, cudaStream_t st) {
         const size_t sizes[5] = {pixels * 4, pixels * sizeof(float4), pixels * sizeof(float4), pixels * sizeof(float), pixels * sizeof(int32_t)};
         for (int k = 0; k < 5; ++k) {
             dev[k] = user[k];
             bytes[k] = sizes[k];
             if ((mem == TMPT_HOST && user[k]) || (k == 0 && frame && !user[k])) {
-                void** p = k == 0 ? (void**)&s->d_frame : &s->d_outs[k - 1];
-                TRY(grow_scratch(p, k == 0 ? &s->frameBytes : &s->outsBytes[k - 1], sizes[k]));
-                dev[k] = *p;
+                CU_TRY(s->staged[k].grow(sizes[k], st));
+                dev[k] = s->staged[k].p;
             }
         }
         return TMPT_OK;
@@ -2335,45 +2328,45 @@ static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int
                         const ProgressivePass* prog, cudaStream_t st, uint64_t* rayCount, double* seconds, AdaptiveResult* adOut = nullptr) {
     const size_t pixels = (size_t)width * height;
     Staging g{{out->rgba, out->radiance, out->normal, out->depth, out->triangle}};
-    TRY(g.stage(s, pixels, mem, true));
+    TRY(g.stage(s, pixels, mem, true, st));
     FrameOutputs f;
     f.radiance = (float4*)g.dev[1]; f.normal = (float4*)g.dev[2]; f.depth = (float*)g.dev[3]; f.triangle = (int32_t*)g.dev[4];
     const AdaptivePass* ad = prog ? prog->adaptive : nullptr;
     int32_t* samples = ad ? ad->samples : nullptr;  // (device buffer)
     if (samples && mem == TMPT_HOST) {
-        TRY(grow_scratch((void**)&s->d_samples, &s->samplesBytes, pixels * sizeof(int32_t)));
-        samples = s->d_samples;
+        CU_TRY(s->d_samples.grow(pixels, st));
+        samples = s->d_samples.p;
     }
     // (scratch allocation stays outside the timed window; an adaptive pass allocates for a list of every pixel)
     TRY(prepare_accum(s, plan_render(width, height, spp, prog, &f, (int)pixels), st, nullptr));
     CU_TRY(cudaEventRecord(s->ev0, st));
-    CU_TRY(cudaMemsetAsync(s->d_rayCount, 0, sizeof(unsigned long long), st));
+    CU_TRY(cudaMemsetAsync(s->d_rayCount.p, 0, sizeof(unsigned long long), st));
     uint32_t listLen = 0;
     if (ad) {  // select + compact: the active list and its length (one small copy)
         const int tilesX = div_up(width, 8);
         const long long slots = (long long)tilesX * div_up(height, 4) * 32;
         const int nBlocks = div_up(slots, kScanBlock);
-        LAUNCH(k_adaptive_select, div_up(slots, 256), 256, 0, st, s->d_adN, s->d_adStat, width, height, tilesX, slots, ad->tolerance, ad->minChunks,
-               s->d_adFlags);
-        LAUNCH(k_scan_totals, nBlocks, kScanBlock, 0, st, s->d_adFlags, slots, s->d_adTotals);
-        LAUNCH(k_scan_of_totals, 1, kScanBlock, 0, st, s->d_adTotals, nBlocks, s->d_adTotals + nBlocks);
-        LAUNCH(k_scan_apply, nBlocks, kScanBlock, 0, st, s->d_adFlags, slots, s->d_adTotals, s->d_adTotals + nBlocks, s->d_adOffs);
-        LAUNCH(k_adaptive_compact, div_up(slots, 256), 256, 0, st, s->d_adFlags, s->d_adOffs, s->d_adN, width, tilesX, slots, s->d_adList);
-        CU_TRY(cudaMemsetAsync(s->d_adActive, 0, sizeof(unsigned int), st));
-        CU_TRY(cudaMemcpyAsync(&listLen, s->d_adTotals + nBlocks, sizeof listLen, cudaMemcpyDeviceToHost, st));
+        LAUNCH(k_adaptive_select, div_up(slots, 256), 256, 0, st, s->d_adN.p, s->d_adStat.p, width, height, tilesX, slots, ad->tolerance, ad->minChunks,
+               s->d_adFlags.p);
+        LAUNCH(k_scan_totals, nBlocks, kScanBlock, 0, st, s->d_adFlags.p, slots, s->d_adTotals.p);
+        LAUNCH(k_scan_of_totals, 1, kScanBlock, 0, st, s->d_adTotals.p, nBlocks, s->d_adTotals.p + nBlocks);
+        LAUNCH(k_scan_apply, nBlocks, kScanBlock, 0, st, s->d_adFlags.p, slots, s->d_adTotals.p, s->d_adTotals.p + nBlocks, s->d_adOffs.p);
+        LAUNCH(k_adaptive_compact, div_up(slots, 256), 256, 0, st, s->d_adFlags.p, s->d_adOffs.p, s->d_adN.p, width, tilesX, slots, s->d_adList.p);
+        CU_TRY(cudaMemsetAsync(s->d_adActive.p, 0, sizeof(unsigned int), st));
+        CU_TRY(cudaMemcpyAsync(&listLen, s->d_adTotals.p + nBlocks, sizeof listLen, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
     }
-    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, (uint8_t*)g.dev[0], s->d_rayCount, st, nullptr, prog, &f, (int)listLen));
-    if (ad) LAUNCH(k_adaptive_write, div_up((long long)pixels, 256), 256, 0, st, prog->sum, s->d_adN, (long long)pixels, (uchar4*)g.dev[0], f.radiance,
+    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, (uint8_t*)g.dev[0], s->d_rayCount.p, st, nullptr, prog, &f, (int)listLen));
+    if (ad) LAUNCH(k_adaptive_write, div_up((long long)pixels, 256), 256, 0, st, prog->sum, s->d_adN.p, (long long)pixels, (uchar4*)g.dev[0], f.radiance,
                    samples);
     TRY(g.copy(mem, cudaMemcpyDeviceToHost, st));
     if (samples && mem == TMPT_HOST) CU_TRY(cudaMemcpyAsync(ad->samples, samples, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     if (ad) {
         adOut->listLen = (int)listLen;
-        CU_TRY(cudaMemcpyAsync(adOut->counters, s->d_adActive, sizeof adOut->counters, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaMemcpyAsync(adOut->counters, s->d_adActive.p, sizeof adOut->counters, cudaMemcpyDeviceToHost, st));
     }
     unsigned long long rays = 0;
-    TRY(end_timed_window(s, st, seconds, s->d_rayCount, &rays));
+    TRY(end_timed_window(s, st, seconds, s->d_rayCount.p, &rays));
     if (rayCount) *rayCount = rays;
     return TMPT_OK;
 }
@@ -2403,16 +2396,12 @@ extern "C" int tmpt_render(const tmpt_scene* cs, const tmpt_camera* camera, int 
 extern "C" int tmpt_progressive_begin(tmpt_scene* s, int width, int height) {
     if (!s) return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_begin: NULL scene");
     if (!frame_size_ok(width, height)) return tmpt::fail(TMPT_ERR_ARG, "tmpt_progressive_begin: %d x %d out of range", width, height);
+    std::lock_guard<std::mutex> lock(s->hostCallMutex);
     DeviceGuard guard(s->device);
     if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "tmpt_progressive_begin: cudaSetDevice(%d) failed", s->device);
-    const size_t need = (size_t)width * height * sizeof(float4);
-    if (s->sumBytes < need) {
-        CU_TRY(cudaStreamSynchronize(s->stream));
-        cudaFree(s->d_sum); s->d_sum = nullptr; s->sumBytes = 0;
-        CU_TRY(cudaMalloc((void**)&s->d_sum, need));
-        s->sumBytes = need;
-    }
-    CU_TRY(cudaMemsetAsync(s->d_sum, 0, need, s->stream));
+    const size_t pixels = (size_t)width * height;
+    CU_TRY(s->d_sum.grow(pixels, s->stream));
+    CU_TRY(cudaMemsetAsync(s->d_sum.p, 0, pixels * sizeof(float4), s->stream));
     CU_TRY(cudaStreamSynchronize(s->stream));
     s->progW = width; s->progH = height; s->progChunks = 0; s->progAdaptive = -1;
     return TMPT_OK;
@@ -2445,7 +2434,7 @@ extern "C" int tmpt_progressive_pass_outputs(tmpt_scene* s, const tmpt_camera* c
     DeviceGuard guard(s->device);
     if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "%s: cudaSetDevice(%d) failed", fn, s->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
-    const ProgressivePass pass{s->progChunks, nChunks, s->d_sum};
+    const ProgressivePass pass{s->progChunks, nChunks, s->d_sum.p};
     TRY(render_frame(s, camera, s->progW, s->progH, 0, mem, out, &pass, st, rayCount, seconds));
     s->progChunks += nChunks;
     s->progAdaptive = 0;
@@ -2457,24 +2446,16 @@ extern "C" int tmpt_progressive_pass_outputs(tmpt_scene* s, const tmpt_camera* c
 static int begin_adaptive(tmpt_scene* s, cudaStream_t st) {
     const int tilesX = div_up(s->progW, 8);
     const size_t slots = (size_t)tilesX * div_up(s->progH, 4) * 32, pixels = (size_t)s->progW * s->progH;
-    if (s->adPixels < slots) {
-        CU_TRY(cudaStreamSynchronize(st));
-        cudaFree(s->d_adN); cudaFree(s->d_adStat); cudaFree(s->d_adFlags); cudaFree(s->d_adOffs); cudaFree(s->d_adTotals); cudaFree(s->d_adList);
-        cudaFree(s->d_adActive);
-        s->d_adN = nullptr; s->d_adStat = nullptr; s->d_adFlags = s->d_adOffs = s->d_adTotals = nullptr; s->d_adList = nullptr; s->d_adActive = nullptr;
-        s->adPixels = 0;
-        CU_TRY(cudaMalloc((void**)&s->d_adN, slots * sizeof(uint32_t)));
-        CU_TRY(cudaMalloc((void**)&s->d_adStat, slots * sizeof(float2)));
-        CU_TRY(cudaMalloc((void**)&s->d_adFlags, slots * sizeof(uint32_t)));
-        CU_TRY(cudaMalloc((void**)&s->d_adOffs, (slots + 1) * sizeof(uint32_t)));
-        CU_TRY(cudaMalloc((void**)&s->d_adTotals, (slots / kScanBlock + 2) * sizeof(uint32_t)));
-        CU_TRY(cudaMalloc((void**)&s->d_adList, slots * sizeof(uint2)));
-        CU_TRY(cudaMalloc((void**)&s->d_adActive, 2 * sizeof(unsigned int)));
-        s->adPixels = slots;
-    }
-    CU_TRY(cudaMemsetAsync(s->d_adN, 0, pixels * sizeof(uint32_t), st));
-    CU_TRY(cudaMemsetAsync(s->d_adStat, 0, pixels * sizeof(float2), st));
-    CU_TRY(cudaMemsetAsync(s->d_adActive, 0, 2 * sizeof(unsigned int), st));
+    CU_TRY(s->d_adN.grow(slots, st));
+    CU_TRY(s->d_adStat.grow(slots, st));
+    CU_TRY(s->d_adFlags.grow(slots, st));
+    CU_TRY(s->d_adOffs.grow(slots + 1, st));
+    CU_TRY(s->d_adTotals.grow(slots / kScanBlock + 2, st));
+    CU_TRY(s->d_adList.grow(slots, st));
+    CU_TRY(s->d_adActive.grow(2, st));
+    CU_TRY(cudaMemsetAsync(s->d_adN.p, 0, pixels * sizeof(uint32_t), st));
+    CU_TRY(cudaMemsetAsync(s->d_adStat.p, 0, pixels * sizeof(float2), st));
+    CU_TRY(cudaMemsetAsync(s->d_adActive.p, 0, 2 * sizeof(unsigned int), st));
     return TMPT_OK;
 }
 
@@ -2494,7 +2475,7 @@ extern "C" int tmpt_progressive_pass_adaptive(tmpt_scene* s, const tmpt_camera* 
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (s->progAdaptive < 0) TRY(begin_adaptive(s, st));
     const AdaptivePass ad{params->tolerance, params->minChunks, samples};
-    const ProgressivePass pass{0, nChunks, s->d_sum, &ad};
+    const ProgressivePass pass{0, nChunks, s->d_sum.p, &ad};
     AdaptiveResult res;
     TRY(render_frame(s, camera, s->progW, s->progH, 0, mem, out, &pass, st, rayCount, seconds, &res));
     s->progAdaptive = 1;
@@ -2539,18 +2520,18 @@ extern "C" int tmpt_denoise(tmpt_scene* s, int width, int height, int mem, const
     // (scratch allocation stays outside the timed window; with TMPT_HOST an output radiance is staged where the input radiance is:
     // the prologue, or the copy, reads that before it is written)
     Staging gin{{nullptr, in->radiance, in->normal, in->depth, nullptr}}, gout{{out->rgba, out->radiance, nullptr, nullptr, nullptr}};
-    TRY(gin.stage(s, pixels, mem, false));
-    TRY(gout.stage(s, pixels, mem, false));
+    TRY(gin.stage(s, pixels, mem, false, st));
+    TRY(gout.stage(s, pixels, mem, false, st));
     uchar4* rgba = (uchar4*)gout.dev[0];
     float4* radiance = (float4*)gout.dev[1];
-    if (params->iterations > 0) TRY(grow_scratch((void**)&s->d_denoise, &s->denoiseBytes, 4 * pixels * sizeof(float4)));
+    if (params->iterations > 0) CU_TRY(s->d_denoise.grow(4 * pixels, st));
     CU_TRY(cudaEventRecord(s->ev0, st));
     TRY(gin.copy(mem, cudaMemcpyHostToDevice, st));
     const float4* rin = (const float4*)gin.dev[1];
     if (params->iterations == 0) {
         LAUNCH(k_denoise_copy, div_up((long long)pixels, 256), 256, 0, st, rin, (long long)pixels, rgba, radiance);
     } else {
-        float4 *state[2] = {s->d_denoise, s->d_denoise + pixels}, *guideA = s->d_denoise + 2 * pixels, *guideB = s->d_denoise + 3 * pixels;
+        float4 *state[2] = {s->d_denoise.p, s->d_denoise.p + pixels}, *guideA = s->d_denoise.p + 2 * pixels, *guideB = s->d_denoise.p + 3 * pixels;
         const dim3 grid(div_up(width, kDenoiseBX), div_up(height, kDenoiseBY)), block(kDenoiseBX, kDenoiseBY);
         const dn::Params prm{params->iterations, params->sigmaLuminance, params->sigmaDepth, params->normalPowerLog2};
         LAUNCH(k_denoise_prep, grid, block, 0, st, rin, (const float4*)gin.dev[2], (const float*)gin.dev[3], width, height, state[0], guideA, guideB);
@@ -2585,11 +2566,7 @@ extern "C" int tmpt_render_multi(tmpt_scene* const* scenes, int nScenes, const t
     struct Restore { int d; ~Restore() { cudaSetDevice(d); } } restore{prev};
     // the frame lives on device 0; every other device needs peer access to it
     CU_TRY(cudaSetDevice(s0->device));
-    if (s0->frameBytes < bytes) {
-        cudaFree(s0->d_frame); s0->d_frame = nullptr; s0->frameBytes = 0;
-        CU_TRY(cudaMalloc((void**)&s0->d_frame, bytes));
-        s0->frameBytes = bytes;
-    }
+    CU_TRY(s0->staged[0].grow(bytes, s0->stream));
     std::vector<unsigned long long*> counters(nScenes);
     for (int i = 0; i < nScenes; ++i) {
         CU_TRY(cudaSetDevice(scenes[i]->device));
@@ -2601,7 +2578,7 @@ extern "C" int tmpt_render_multi(tmpt_scene* const* scenes, int nScenes, const t
             if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) CU_TRY(e);
             cudaGetLastError();
         }
-        counters[i] = scenes[i]->d_rayCount;
+        counters[i] = scenes[i]->d_rayCount.p;
         CU_TRY(cudaMemsetAsync(counters[i], 0, sizeof(unsigned long long), scenes[i]->stream));
         TRY(prepare_accum(scenes[i], plan_render(tmpt_local_width(width, 0, nScenes), height, spp, nullptr, nullptr, 0), scenes[i]->stream,
                           nullptr));  // tile interleave
@@ -2613,7 +2590,7 @@ extern "C" int tmpt_render_multi(tmpt_scene* const* scenes, int nScenes, const t
     const auto t0 = std::chrono::steady_clock::now();
     for (int i = 0; i < nScenes; ++i) {
         CU_TRY(cudaSetDevice(scenes[i]->device));
-        TRY(launch_render(scenes[i], camera, width, height, spp, 0, i, nScenes, nullptr, s0->d_frame, counters[i], scenes[i]->stream));
+        TRY(launch_render(scenes[i], camera, width, height, spp, 0, i, nScenes, nullptr, (uint8_t*)s0->staged[0].p, counters[i], scenes[i]->stream));
     }
     unsigned long long total = 0;
     for (int i = nScenes - 1; i >= 0; --i) {  // device 0 last: its stream then copies the completed frame out
@@ -2623,7 +2600,7 @@ extern "C" int tmpt_render_multi(tmpt_scene* const* scenes, int nScenes, const t
         CU_TRY(cudaStreamSynchronize(scenes[i]->stream));
         total += rays;
     }
-    CU_TRY(cudaMemcpyAsync(rgba, s0->d_frame, bytes, cudaMemcpyDeviceToHost, s0->stream));
+    CU_TRY(cudaMemcpyAsync(rgba, s0->staged[0].p, bytes, cudaMemcpyDeviceToHost, s0->stream));
     CU_TRY(cudaStreamSynchronize(s0->stream));
     const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     if (rayCount) *rayCount = total;
@@ -2683,11 +2660,11 @@ extern "C" int tmpt_render_stats(const tmpt_scene* cs, const tmpt_camera* camera
     const size_t bytes = (size_t)width * height * 4;
     DevBuf<uint8_t> frame;
     DevBuf<unsigned long long> stats;
-    CU_TRY(frame.alloc(bytes));
-    CU_TRY(stats.alloc(TMPT_STATS_COUNT));
+    CU_TRY(frame.grow(bytes, st));
+    CU_TRY(stats.grow(TMPT_STATS_COUNT, st));
     CU_TRY(cudaMemsetAsync(stats.p, 0, TMPT_STATS_COUNT * sizeof(unsigned long long), st));
-    CU_TRY(cudaMemsetAsync(s->d_rayCount, 0, sizeof(unsigned long long), st));
-    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, frame.p, s->d_rayCount, st, stats.p));
+    CU_TRY(cudaMemsetAsync(s->d_rayCount.p, 0, sizeof(unsigned long long), st));
+    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, frame.p, s->d_rayCount.p, st, stats.p));
     CU_TRY(cudaMemcpyAsync(outStats, stats.p, TMPT_STATS_COUNT * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     return TMPT_OK;
@@ -2702,8 +2679,8 @@ extern "C" int tmpt_hit_scene_stats(const tmpt_scene* s, const float* rays6Dev, 
     cudaStream_t st = s->stream;
     DevBuf<unsigned long long> stats;
     DevBuf<int> ids;
-    CU_TRY(stats.alloc(TMPT_STATS_COUNT));
-    CU_TRY(ids.alloc((size_t)nRays));
+    CU_TRY(stats.grow(TMPT_STATS_COUNT, st));
+    CU_TRY(ids.grow((size_t)nRays, st));
     CU_TRY(cudaMemsetAsync(stats.p, 0, TMPT_STATS_COUNT * sizeof(unsigned long long), st));
     const int B = 128;
     const int G = (int)std::min<long long>(div_up(nRays, B), (long long)s->smCount * 64);
