@@ -135,6 +135,13 @@ TMPT_HD int chunk_len(int spp) {
     return c < 1 ? 1 : c > kMaxChunkSamples ? kMaxChunkSamples : c;
 }
 TMPT_HD int chunk_count(int spp) { const int c = chunk_len(spp); return (spp + c - 1) / c; }
+// Chunk `chunk` of pixel (x, y) with `len` samples per chunk: its samples [s0, s1) = [chunk * len, min(chunk * len + len, spp)),
+// and (returned) the seed of its stream.  render_chunk and the kernels that run their own sample loop all start a chunk here.
+TMPT_HD uint32_t chunk_start(int x, int y, int chunk, int width, int height, int spp, int len, int& s0, int& s1) {
+    s0 = chunk * len;
+    s1 = s0 + len < spp ? s0 + len : spp;
+    return ex::chunk_seed((uint32_t)chunk, (uint32_t)y * (uint32_t)width + (uint32_t)x, (uint32_t)width * (uint32_t)height);
+}
 
 // AOV sums of one chunk or pixel (AOV = true), each from +0 in sample order, chunk sums added in chunk order like the colour:
 // over the samples whose camera ray hits, the hit count, the sum of their normals and of their t.  id0 = the camera-ray hit of
@@ -165,9 +172,9 @@ template <bool STATS = false, bool FAR = true, bool AOV = false, class Stack, cl
 TMPT_HD ex::V3 render_chunk(Stack& stack, const Scene& sc, const Camera& cam, int x, int y, int chunk, int width, int height, int spp, int len, ex::V3 lightDir,
                             unsigned long long& rays, bvh::TravStats* stats = nullptr, AovSums* aov = nullptr) {
     const float invW = ex::divf(1.0f, (float)width), invH = ex::divf(1.0f, (float)height);
-    uint32_t rng = ex::chunk_seed((uint32_t)chunk, (uint32_t)y * (uint32_t)width + (uint32_t)x, (uint32_t)width * (uint32_t)height);
+    int s0, s1;
+    uint32_t rng = chunk_start(x, y, chunk, width, height, spp, len, s0, s1);
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f);
-    const int s0 = chunk * len, s1 = s0 + len < spp ? s0 + len : spp;
     if (AOV) aov_clear(*aov);
     for (int s = s0; s < s1; ++s) {
         ex::V3 o, d;

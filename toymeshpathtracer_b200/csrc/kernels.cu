@@ -712,8 +712,7 @@ struct RenderParams {
     int useAccum;        // chunk sums go through `accum` + k_resolve (more than one chunk, a progressive pass, or float outputs)
     float4* sumBuf;      // progressive: running per-pixel sums of the whole frame (null for a one-shot frame)
     int bandRow0, bandRows;  // first owned row and row count of the band being rendered (the accumulation buffer covers one band)
-    float4* accum;       // [chunks][bandRows][width] chunk sums (chunk-major planes: full-line stores, no read-modify-write in HBM); AOV
-                         // kernels: .w = the chunk's camera-ray hits, followed by [chunks][bandRows][width] (normal sum, t sum)
+    float4* accum;       // the band's chunk sums (accum_index)
     uchar4* outStripes;  // packed owned rows, or
     uchar4* frame;       // full frame (possibly peer memory)
     float4* radiance;    // tmpt_outputs' float buffers (full frame, device memory; null = not produced): written by k_resolve
@@ -725,8 +724,18 @@ struct RenderParams {
     unsigned long long* laneCounter;  // k_render_regen: next lane item
     unsigned long long* stats;  // instrumented pass only
     const uint2* list;   // LIST kernels (adaptive passes): the band's entries of the active list, {x | y << 16, first chunk n_i}
-    int listLen;         // entries in the band; accum = [chunks][listLen]
+    int listLen;         // entries in the band
 };
+
+// The 8x4-pixel tile, a warp's pixels in the render kernels and in the adaptive list: lane = (x & 7) + 8 (y & 3), tiles in
+// row-major order, `tilesX` per tile row.
+constexpr int kTileLogW = 3, kTileLogH = 2, kTileW = 1 << kTileLogW, kTileH = 1 << kTileLogH;
+static_assert(kTileW * kTileH == 32, "a tile is a warp");
+__device__ __forceinline__ void tile_pixel(uint32_t tile, uint32_t lane, int tilesX, int& x, int& y) {
+    const int tx = (int)(tile % (uint32_t)tilesX), ty = (int)(tile / (uint32_t)tilesX);
+    x = tx * kTileW + (int)(lane & (kTileW - 1));
+    y = ty * kTileH + (int)(lane >> kTileLogW);
+}
 
 __device__ __forceinline__ int owned_row_to_global(int r, int stripeRows, int rank, int world) {
     const int ls = r / stripeRows;
@@ -749,9 +758,9 @@ __device__ __forceinline__ bool local_to_global(int xl, int r, int stripeRows, i
         return true;
     }
     y = r;
-    int t0 = (rank - (r >> 2)) % world;
+    int t0 = (rank - (r >> kTileLogH)) % world;
     t0 += t0 < 0 ? world : 0;
-    x = ((t0 + (xl >> 3) * world) << 3) + (xl & 7);
+    x = ((t0 + (xl >> kTileLogW) * world) << kTileLogW) + (xl & (kTileW - 1));
     return x < width;
 }
 
@@ -782,8 +791,69 @@ constexpr int kSStack = TMPT_SSTACK;
 // What a render launch writes (one mode per instantiation of k_render and k_render_paths):
 //   Frame: the RGBA frame, or chunk sums for k_resolve (and the radiance it writes);
 //   Aov:   the frame has AOV outputs (tmpt_outputs normal / depth / triangle): the same paths, plus each sample's camera-ray hit;
-//   List:  an adaptive pass: work item (list tile t, k) is entry list[t * 32 + lane] of the band, its chunk n_i + k of 8 samples.
+//   List:  an adaptive pass: chunk sums of the band's entries of the active list (decode_item).
 enum class OutMode { Frame, Aov, List };
+
+// A render work item: one chunk of one pixel's samples.  Warp item w, lane l (k_render fetches a w per warp, k_render_paths a lane
+// item w * 32 + l per lane) is tile w % numTiles of the band and accumulation plane w / numTiles: pixel l of the tile, chunk
+// chunk0 + plane of chunkLen samples, or, List, entry tile * 32 + l of the band's list, chunk n_i + plane of 8 samples.  False: no
+// such pixel or entry.
+struct WorkItem {
+    int x, y;       // the frame pixel
+    int xl, rb, r;  // the local pixel in the band's planes, its owned row bandRow0 + rb (List: xl = the entry)
+    int chunk;      // the accumulation plane
+    int gchunk;     // the chunk of the pixel's samples (progressive passes continue the numbering)
+    int spp, len;   // integ::chunk_start's sample range arguments
+};
+template <bool LIST>
+__device__ __forceinline__ bool decode_item(const RenderParams& p, uint32_t w, uint32_t lane, WorkItem& it) {
+    const uint32_t chunk = w / (uint32_t)p.numTiles, tile = w - chunk * (uint32_t)p.numTiles;
+    if (LIST) {
+        const uint32_t e = tile * 32u + lane;
+        if (e >= (uint32_t)p.listLen) return false;
+        const uint2 en = p.list[e];
+        it = {(int)(en.x & 0xFFFFu), (int)(en.x >> 16), (int)e, 0, 0, (int)chunk, (int)(en.y + chunk), 0x7FFFFFFF, integ::kMaxChunkSamples};
+        return true;
+    }
+    it.chunk = (int)chunk; it.gchunk = p.chunk0 + (int)chunk;
+    it.spp = p.spp; it.len = p.chunkLen;
+    tile_pixel(tile, lane, p.tilesX, it.xl, it.rb);
+    it.r = p.bandRow0 + it.rb;
+    return it.xl < p.localWidth && it.r < p.ownedRows && local_to_global(it.xl, it.r, p.stripeRows, p.rank, p.world, p.width, it.x, it.y);
+}
+
+// The chunk sums of a band (RenderParams::accum): chunk-major float4 planes [plane][bandRows][localWidth], so that a warp's stores
+// and k_resolve's loads cover whole lines and nothing is read-modified-written in HBM.  Plane c holds chunk c's colour sum (Aov:
+// and its camera-ray hits in .w), Aov: plane chunks + c its (normal sum, t sum).  An adaptive pass's band: [chunk][listLen].
+__device__ __forceinline__ size_t accum_index(const RenderParams& p, int plane, int xl, int rb) {
+    return ((size_t)plane * p.bandRows + rb) * p.localWidth + xl;
+}
+__device__ __forceinline__ size_t accum_planes(const RenderParams& p, int n) { return (size_t)n * ((size_t)p.bandRows * p.localWidth); }
+__device__ __forceinline__ size_t list_accum_index(const RenderParams& p, int chunk, uint32_t e) { return (size_t)chunk * p.listLen + e; }
+
+// A finished item's chunk sum: into the planes (streaming stores: read once, by the resolve), or, with one chunk per pixel and no
+// resolve, as the resolved pixel into the frame or the packed stripes.
+template <OutMode MODE>
+__device__ __forceinline__ void store_chunk(const RenderParams& p, const WorkItem& it, ex::V3 sum, const integ::AovSums* aov = nullptr) {
+    if (MODE == OutMode::List) {
+        __stcs(&p.accum[list_accum_index(p, it.chunk, (uint32_t)it.xl)], make_float4(sum.x, sum.y, sum.z, 0.0f));
+    } else if (p.useAccum) {
+        constexpr bool AOV = MODE == OutMode::Aov;
+        const size_t a = accum_index(p, it.chunk, it.xl, it.rb);
+        __stcs(&p.accum[a], make_float4(sum.x, sum.y, sum.z, AOV ? aov->hits : 0.0f));
+        if (AOV) __stcs(&p.accum[a + accum_planes(p, p.chunks)], make_float4(aov->normal.x, aov->normal.y, aov->normal.z, aov->t));
+    } else {
+        const uchar4 px = integ::resolve_pixel(sum, ex::divf(1.0f, (float)p.spp));
+        if (p.frame) p.frame[(size_t)it.y * p.width + it.x] = px;
+        else p.outStripes[(size_t)it.r * p.localWidth + it.xl] = px;
+    }
+}
+
+// The end of a render kernel: the warp's rays, added to the launch's count with one atomic.
+__device__ __forceinline__ void flush_rays(const RenderParams& p, unsigned long long rays) {
+    for (int o = 16; o > 0; o >>= 1) rays += __shfl_xor_sync(0xffffffffu, rays, o);
+    if ((threadIdx.x & 31) == 0 && rays) atomicAdd(p.rayCount, rays);
+}
 
 // FAR = the camera stands beyond the scene's far limit (bvh.cuh: ray_is_far): rays are checked and, if far, answered by the
 // exact all-triangle scan.  Only the 256-thread configuration has that instantiation (a camera sixteen scene sizes away sees
@@ -796,43 +866,20 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render(const RenderParams p) 
     bvh::TravStats ts;
     typename RenderStack<SSTACK, THREADS>::type stack = RenderStack<SSTACK, THREADS>::make();
     for (;;) {
-        uint32_t tile = 0;
-        if (lane == 0) tile = atomicAdd(p.tileCounter, 1u);
-        tile = __shfl_sync(0xffffffffu, tile, 0);
-        if (tile >= (uint32_t)p.numTiles * (uint32_t)p.chunks) break;
-        const int chunk = (int)(tile / (uint32_t)p.numTiles);
-        tile -= (uint32_t)chunk * (uint32_t)p.numTiles;
-        if (LIST) {
-            const uint32_t e = tile * 32u + (uint32_t)lane;
-            if (e < (uint32_t)p.listLen) {
-                const uint2 en = p.list[e];
-                const ex::V3 sum = integ::render_chunk<STATS, FAR>(stack, p.sc, p.cam, (int)(en.x & 0xFFFFu), (int)(en.x >> 16), (int)en.y + chunk, p.width,
-                                                                   p.height, 0x7FFFFFFF, integ::kMaxChunkSamples, p.lightDir, rays, &ts);
-                __stcs(&p.accum[(size_t)chunk * p.listLen + e], make_float4(sum.x, sum.y, sum.z, 0.0f));
-            }
-            continue;
-        }
-        const int tx = (int)(tile % (uint32_t)p.tilesX), ty = (int)(tile / (uint32_t)p.tilesX);
-        const int xl = tx * 8 + (lane & 7), rb = ty * 4 + (lane >> 3), r = p.bandRow0 + rb;
-        int x, y;
-        if (xl < p.localWidth && r < p.ownedRows && local_to_global(xl, r, p.stripeRows, p.rank, p.world, p.width, x, y)) {
+        uint32_t item = 0;
+        if (lane == 0) item = atomicAdd(p.tileCounter, 1u);
+        item = __shfl_sync(0xffffffffu, item, 0);
+        if (item >= (uint32_t)p.numTiles * (uint32_t)p.chunks) break;
+        WorkItem it;
+        if (decode_item<LIST>(p, item, (uint32_t)lane, it)) {
             integ::AovSums aov;
-            const ex::V3 sum = integ::render_chunk<STATS, FAR, AOV>(stack, p.sc, p.cam, x, y, p.chunk0 + chunk, p.width, p.height, p.spp, p.chunkLen, p.lightDir, rays, &ts, &aov);
-            if (AOV && p.triangle && p.chunk0 + chunk == 0) p.triangle[(size_t)y * p.width + x] = aov.id0;
-            if (p.useAccum) {
-                const size_t a = ((size_t)chunk * p.bandRows + rb) * p.localWidth + xl;
-                __stcs(&p.accum[a], make_float4(sum.x, sum.y, sum.z, AOV ? aov.hits : 0.0f));  // streaming: read once, by k_resolve
-                if (AOV) __stcs(&p.accum[a + (size_t)p.chunks * p.bandRows * p.localWidth], make_float4(aov.normal.x, aov.normal.y, aov.normal.z, aov.t));
-            } else {
-                const uchar4 px = integ::resolve_pixel(sum, ex::divf(1.0f, (float)p.spp));
-                if (p.frame) p.frame[(size_t)y * p.width + x] = px;
-                else p.outStripes[(size_t)r * p.localWidth + xl] = px;
-            }
+            const ex::V3 sum = integ::render_chunk<STATS, FAR, AOV>(stack, p.sc, p.cam, it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len, p.lightDir, rays, &ts, &aov);
+            if (AOV && p.triangle && p.chunk0 + it.chunk == 0) p.triangle[(size_t)it.y * p.width + it.x] = aov.id0;
+            store_chunk<MODE>(p, it, sum, &aov);
         }
     }
     if (STATS) flush_stats(p.stats, rays, ts, 0);
-    for (int o = 16; o > 0; o >>= 1) rays += __shfl_xor_sync(0xffffffffu, rays, o);
-    if (lane == 0 && rays) atomicAdd(p.rayCount, rays);
+    flush_rays(p, rays);
 }
 
 #if TMPT_EXPERIMENTS
@@ -860,7 +907,8 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
     int state = ST_NEED_ITEM;
     bool exhausted = false;
     uint32_t rng = 0;
-    int depth = 0, s = 0, sEnd = 0, x = 0, y = 0, xl = 0, rb = 0, chunk = 0;
+    int depth = 0, s = 0, sEnd = 0;
+    WorkItem it = {};
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f), nd = ex::v3(0.0f, 0.0f, 0.0f);
     float sunk = 0.0f;
     const float invW = ex::divf(1.0f, (float)p.width), invH = ex::divf(1.0f, (float)p.height);
@@ -895,13 +943,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
                     for (int i = depth - 1; i >= 0; --i) color = integ::unwind_step(kk[i], color);
                     sum = ex::add(sum, color);
                     if (++s == sEnd) {
-                        if (p.useAccum) {
-                            __stcs(&p.accum[((size_t)chunk * p.bandRows + rb) * p.localWidth + xl], make_float4(sum.x, sum.y, sum.z, 0.0f));  // streaming: read once, by k_resolve
-                        } else {
-                            const uchar4 px = integ::resolve_pixel(sum, ex::divf(1.0f, (float)p.spp));
-                            if (p.frame) p.frame[(size_t)y * p.width + x] = px;
-                            else p.outStripes[(size_t)(p.bandRow0 + rb) * p.localWidth + xl] = px;
-                        }
+                        store_chunk<OutMode::Frame>(p, it, sum);
                         state = ST_NEED_ITEM;
                     }
                 }
@@ -920,18 +962,8 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
                             if (item >= totalItems) {
                                 state = ST_IDLE;
                             } else {
-                                const uint32_t wi = (uint32_t)(item >> 5), li = (uint32_t)item & 31u;
-                                chunk = (int)(wi / (uint32_t)p.numTiles);
-                                const uint32_t tile = wi - (uint32_t)chunk * (uint32_t)p.numTiles;
-                                const int tx = (int)(tile % (uint32_t)p.tilesX), ty = (int)(tile / (uint32_t)p.tilesX);
-                                xl = tx * 8 + (int)(li & 7u); rb = ty * 4 + (int)(li >> 3);
-                                const int r = p.bandRow0 + rb;
-                                if (xl < p.localWidth && r < p.ownedRows && local_to_global(xl, r, p.stripeRows, p.rank, p.world, p.width, x, y)) {  // (an item outside the frame is simply dropped: the lane asks again)
-                                    const int gchunk = p.chunk0 + chunk;  // progressive passes continue the chunk numbering; `chunk` stays the accum plane
-                                    rng = ex::chunk_seed((uint32_t)gchunk, (uint32_t)y * (uint32_t)p.width + (uint32_t)x, (uint32_t)p.width * (uint32_t)p.height);
-                                    const int len = p.chunkLen;
-                                    s = gchunk * len;
-                                    sEnd = s + len < p.spp ? s + len : p.spp;
+                                if (decode_item<false>(p, (uint32_t)(item >> 5), (uint32_t)item & 31u, it)) {  // (an item outside the frame is simply dropped: the lane asks again)
+                                    rng = integ::chunk_start(it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len, s, sEnd);
                                     sum = ex::v3(0.0f, 0.0f, 0.0f);
                                     state = ST_PATH_END;  // marks "has an item, needs a camera ray" for the block below
                                     depth = -1;
@@ -941,7 +973,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
                     }
                 }
                 if (state == ST_PATH_END) {  // next sample of the item
-                    integ::primary_ray(p.cam, x, y, invW, invH, rng, no, ndir);
+                    integ::primary_ray(p.cam, it.x, it.y, invW, invH, rng, no, ndir);
                     depth = 0; newRay = true; newAny = false;
                 }
             }
@@ -958,8 +990,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
         }
     }
     if (STATS) flush_stats(p.stats, rays, ts, 0);
-    for (int o = 16; o > 0; o >>= 1) rays += __shfl_xor_sync(FULL, rays, o);
-    if (lane == 0 && rays) atomicAdd(p.rayCount, rays);
+    flush_rays(p, rays);
 }
 
 #endif  // TMPT_EXPERIMENTS
@@ -973,7 +1004,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
 // tracing.  Work item = one (pixel, chunk) per lane; consecutive items are the pixels of one 8x4 tile, so a warp starts with a
 // whole tile.  The per-lane arithmetic and its order are those of integ::render_chunk: the frame is byte-identical to k_render's.
 // AOV (as in k_render): the camera ray's hit of each sample is added to nsum / tsum and counted in cl's top byte.
-// LIST (as in k_render): item (list tile t, k, lane) is entry list[t * 32 + lane], chunk n_i + k; loc holds the entry index.
+// LIST (as in k_render): loc holds the list entry.
 template <int THREADS, int MINB, int GATE, OutMode MODE = OutMode::Frame>
 __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderParams p) {
     constexpr bool AOV = MODE == OutMode::Aov, LIST = MODE == OutMode::List;
@@ -983,7 +1014,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
     float kk[integ::kMaxDepth];
     unsigned long long rays = 0;
     bool havePath = false, done = false, exhausted = false;
-    // a lane's item, packed (the kernel lives at 64 registers): pixel x | y << 16 (both < 10000), packed position xl | rb << 16,
+    // a lane's item, packed (the kernel lives at 64 registers): pixel x | y << 16 (both < 10000), local position xl | rb << 16,
     // chunk << 8 | samples left in the chunk (<= integ::kMaxChunkSamples); hasItem = the lane owes a store when `left` reaches 0.
     // AOV: camera-ray hits of the item so far << 24 (chunk < 2^16)
     uint32_t rng = 0, pix = 0, loc = 0, cl = 0;
@@ -1001,18 +1032,11 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             // (a) items that are finished: store the chunk sum, ask for a new item
             bool wantItem = !havePath && !done && (cl & 0xFFu) == 0u;
             if (wantItem && hasItem) {
-                const int xl = (int)(loc & 0xFFFFu), rb = (int)(loc >> 16);
-                if (LIST) {
-                    __stcs(&p.accum[(size_t)(cl >> 8) * p.listLen + loc], make_float4(sum.x, sum.y, sum.z, 0.0f));
-                } else if (p.useAccum) {
-                    const size_t a = ((size_t)(AOV ? (cl >> 8) & 0xFFFFu : cl >> 8) * p.bandRows + rb) * p.localWidth + xl;
-                    __stcs(&p.accum[a], make_float4(sum.x, sum.y, sum.z, AOV ? (float)(cl >> 24) : 0.0f));
-                    if (AOV) __stcs(&p.accum[a + (size_t)p.chunks * p.bandRows * p.localWidth], make_float4(nsum.x, nsum.y, nsum.z, tsum));
-                } else {
-                    const uchar4 px = integ::resolve_pixel(sum, ex::divf(1.0f, (float)p.spp));
-                    if (p.frame) p.frame[(size_t)(pix >> 16) * p.width + (pix & 0xFFFFu)] = px;
-                    else p.outStripes[(size_t)(p.bandRow0 + rb) * p.localWidth + xl] = px;
-                }
+                const int rb = (int)(loc >> 16);
+                const WorkItem it = {(int)(pix & 0xFFFFu), (int)(pix >> 16), (int)(LIST ? loc : loc & 0xFFFFu), rb, p.bandRow0 + rb,
+                                     (int)(AOV ? (cl >> 8) & 0xFFFFu : cl >> 8)};
+                const integ::AovSums aov = {nsum, tsum, (float)(cl >> 24), 0};
+                store_chunk<MODE>(p, it, sum, &aov);
                 hasItem = false;
             }
             while (__any_sync(FULL, wantItem)) {  // (a lane whose item fell outside the frame asks again)
@@ -1027,36 +1051,13 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
                     const unsigned long long item = base + (unsigned long long)__popc(want & ((1u << lane) - 1u));
                     if (item >= totalItems) { done = true; wantItem = false; }
                     else {
-                        const uint32_t wi = (uint32_t)(item >> 5), li = (uint32_t)item & 31u;
-                        const int chunk = (int)(wi / (uint32_t)p.numTiles);
-                        const uint32_t tile = wi - (uint32_t)chunk * (uint32_t)p.numTiles;
-                        if (LIST) {
-                            const uint32_t e = tile * 32u + li;
-                            if (e < (uint32_t)p.listLen) {
-                                const uint2 en = p.list[e];
-                                rng = ex::chunk_seed(en.y + (uint32_t)chunk, (en.x >> 16) * (uint32_t)p.width + (en.x & 0xFFFFu),
-                                                     (uint32_t)p.width * (uint32_t)p.height);
-                                pix = en.x;
-                                loc = e;
-                                cl = ((uint32_t)chunk << 8) | (uint32_t)integ::kMaxChunkSamples;
-                                sum = ex::v3(0.0f, 0.0f, 0.0f);
-                                hasItem = true;
-                                wantItem = false;
-                            }
-                            continue;
-                        }
-                        const int tx = (int)(tile % (uint32_t)p.tilesX), ty = (int)(tile / (uint32_t)p.tilesX);
-                        const int xl = tx * 8 + (int)(li & 7u), rb = ty * 4 + (int)(li >> 3);
-                        const int r = p.bandRow0 + rb;
-                        int x, y;
-                        if (xl < p.localWidth && r < p.ownedRows && local_to_global(xl, r, p.stripeRows, p.rank, p.world, p.width, x, y)) {
-                            const int gchunk = p.chunk0 + chunk;
-                            rng = ex::chunk_seed((uint32_t)gchunk, (uint32_t)y * (uint32_t)p.width + (uint32_t)x, (uint32_t)p.width * (uint32_t)p.height);
-                            const int s0 = gchunk * p.chunkLen;
-                            const int left = (s0 + p.chunkLen < p.spp ? s0 + p.chunkLen : p.spp) - s0;
-                            pix = (uint32_t)x | ((uint32_t)y << 16);
-                            loc = (uint32_t)xl | ((uint32_t)rb << 16);
-                            cl = ((uint32_t)chunk << 8) | (uint32_t)left;
+                        WorkItem it;
+                        if (decode_item<LIST>(p, (uint32_t)(item >> 5), (uint32_t)item & 31u, it)) {
+                            int s0, s1;
+                            rng = integ::chunk_start(it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len, s0, s1);
+                            pix = (uint32_t)it.x | ((uint32_t)it.y << 16);
+                            loc = (uint32_t)it.xl | ((uint32_t)it.rb << 16);
+                            cl = ((uint32_t)it.chunk << 8) | (uint32_t)(s1 - s0);
                             sum = ex::v3(0.0f, 0.0f, 0.0f);
                             if (AOV) { nsum = sum; tsum = 0.0f; }
                             hasItem = true;
@@ -1116,8 +1117,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             }
         }
     }
-    for (int k = 16; k > 0; k >>= 1) rays += __shfl_xor_sync(FULL, rays, k);
-    if (lane == 0 && rays) atomicAdd(p.rayCount, rays);
+    flush_rays(p, rays);
 }
 
 // ---- K7: the sun grid (sungrid.cuh), built on the device after the tree ---------------------------------------------------------
@@ -1261,15 +1261,15 @@ __global__ void __launch_bounds__(128) k_probe_paths(bvh::SceneView sc, integ::C
 // pixel = in-order sum of its chunk sums, then mean / sqrt / quantise (main.cpp:221-233), and the float outputs the frame asks
 // for (integ::radiance_of ...).  AOV: the planes hold the hit counts and the second plane set (k_render<AOV>).
 template <bool AOV>
-__global__ void k_resolve(const RenderParams p, int bandRows) {
+__global__ void k_resolve(const RenderParams p) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)bandRows * p.localWidth) return;
+    const size_t plane = accum_planes(p, 1);
+    if (i >= (long long)plane) return;
     const int rb = (int)(i / p.localWidth), xl = (int)(i - (long long)rb * p.localWidth), r = p.bandRow0 + rb;
     int x, y;
     if (!local_to_global(xl, r, p.stripeRows, p.rank, p.world, p.width, x, y)) return;
     const size_t pix = (size_t)y * p.width + x;
-    const size_t plane = (size_t)bandRows * p.localWidth;  // chunk-major planes: a warp's stores and these loads cover whole lines
-    const float4* a = p.accum + i;
+    const float4* a = p.accum + i;  // (= accum_index(p, 0, xl, rb))
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f), nsum = sum;
     float tsum = 0.0f, hits = 0.0f;
     if (p.sumBuf) { const float4 v = p.sumBuf[pix]; sum = ex::v3(v.x, v.y, v.z); }  // progressive: the chunks before this pass
@@ -1304,8 +1304,8 @@ __global__ void k_adaptive_select(const uint32_t* __restrict__ n, const float2* 
                                   long long slots, float tolerance, int minChunks, uint32_t* __restrict__ flags) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= slots) return;
-    const int tile = (int)(i >> 5), lane = (int)(i & 31);
-    const int x = (tile % tilesX) * 8 + (lane & 7), y = (tile / tilesX) * 4 + (lane >> 3);
+    int x, y;
+    tile_pixel((uint32_t)(i >> 5), (uint32_t)i & 31u, tilesX, x, y);
     uint32_t f = 0u;
     if (x < width && y < height) {
         const size_t pix = (size_t)y * width + x;
@@ -1318,8 +1318,8 @@ __global__ void k_adaptive_compact(const uint32_t* __restrict__ flags, const uin
                                    int width, int tilesX, long long slots, uint2* __restrict__ list) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= slots || !flags[i]) return;
-    const int tile = (int)(i >> 5), lane = (int)(i & 31);
-    const int x = (tile % tilesX) * 8 + (lane & 7), y = (tile / tilesX) * 4 + (lane >> 3);
+    int x, y;
+    tile_pixel((uint32_t)(i >> 5), (uint32_t)i & 31u, tilesX, x, y);
     list[offs[i]] = make_uint2((uint32_t)x | ((uint32_t)y << 16), n[(size_t)y * width + x]);
 }
 // The band's chunk sums ([chunks][listLen]) into each entry's pixel in chunk order: the colour sum, n and the Welford state, then
@@ -1338,7 +1338,7 @@ __global__ void k_resolve_adaptive(const RenderParams p, float4* __restrict__ su
         nn = n[pix];
         float2 st = stat[pix];
         for (int c = 0; c < p.chunks; ++c) {
-            const float4 v = __ldcs(&p.accum[(size_t)c * p.listLen + e]);
+            const float4 v = __ldcs(&p.accum[list_accum_index(p, c, (uint32_t)e)]);
             const ex::V3 cs = ex::v3(v.x, v.y, v.z);
             sum = ex::add(sum, cs);
             integ::adaptive_add_chunk(cs, nn, st.x, st.y);
@@ -1414,8 +1414,9 @@ __global__ void k_unpack_stripes(const uchar4* __restrict__ gathered, int width,
     if (i >= (long long)width * height) return;
     const int y = (int)(i / width), x = (int)(i - (long long)y * width);
     if (stripeRows == 0) {  // tile interleave (local_to_global): tile (tx, ty) is local tile tx / world of rank (tx + ty) % world
-        const int tx = x >> 3, ty = y >> 2, rank = (tx + ty) % world, localWidth = ((width + 7) / 8 + world - 1) / world * 8;
-        frame[i] = gathered[((size_t)rank * maxRowsPerRank + y) * localWidth + ((tx / world) << 3) + (x & 7)];
+        const int tx = x >> kTileLogW, ty = y >> kTileLogH, rank = (tx + ty) % world;
+        const int localWidth = ((width + kTileW - 1) / kTileW + world - 1) / world * kTileW;
+        frame[i] = gathered[((size_t)rank * maxRowsPerRank + y) * localWidth + ((tx / world) << kTileLogW) + (x & (kTileW - 1))];
         return;
     }
     const int gs = y / stripeRows, rank = gs % world, ls = gs / world;
@@ -1948,7 +1949,7 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
 // ------------------------------------------------------------------------------------------
 extern "C" int tmpt_local_width(int width, int stripeRows, int worldSize) {
     if (width <= 0 || stripeRows < 0 || worldSize <= 0) return 0;
-    return stripeRows > 0 ? width : ((width + 7) / 8 + worldSize - 1) / worldSize * 8;
+    return stripeRows > 0 ? width : ((width + kTileW - 1) / kTileW + worldSize - 1) / worldSize * kTileW;
 }
 extern "C" int tmpt_stripe_rows(int height, int stripeRows, int rank, int worldSize) {
     if (height <= 0 || stripeRows < 0 || worldSize <= 0 || rank < 0 || rank >= worldSize) return 0;
@@ -2017,7 +2018,7 @@ static RenderPlan plan_render(int localWidth, int ownedRows, int spp, const Prog
     pl.useAccum = pl.chunks > 1 || prog || (outs && outs->accum());
     pl.planes = pl.mode == OutMode::Aov ? 2 : 1;
     const bool list = pl.mode == OutMode::List;
-    pl.granule = list ? 32 : 4;
+    pl.granule = list ? 32 : kTileH;
     pl.units = list ? listLen : ownedRows;
     pl.unitWidth = list ? 1 : localWidth;
     return pl;
@@ -2129,7 +2130,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     p.stripeRows = stripeRows; p.rank = rank; p.world = world;
     p.ownedRows = tmpt_stripe_rows(height, stripeRows, rank, world);
     p.localWidth = tmpt_local_width(width, stripeRows, world);
-    p.tilesX = div_up(p.localWidth, 8);
+    p.tilesX = div_up(p.localWidth, kTileW);
     const RenderPlan pl = plan_render(p.localWidth, p.ownedRows, spp, prog, outs, listLen);
     p.spp = pl.spp; p.chunks = pl.chunks; p.chunk0 = pl.chunk0; p.chunkLen = pl.chunkLen; p.useAccum = pl.useAccum ? 1 : 0;
     p.radiance = outs ? outs->radiance : nullptr;
@@ -2181,7 +2182,7 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         } else {
             p.bandRow0 = b0;
             p.bandRows = here;
-            p.numTiles = p.tilesX * div_up(here, 4);
+            p.numTiles = p.tilesX * div_up(here, kTileH);
         }
         const long long items = (long long)p.numTiles * p.chunks;
         if (items >= 0xFFFFFFFFll) return tmpt::fail(TMPT_ERR_ARG, "render: too many work items in one band");
@@ -2238,8 +2239,8 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         if (pl.mode == OutMode::List)
             LAUNCH(k_resolve_adaptive, div_up(here, 256), 256, 0, st, p, prog->sum, s->d_adN.p, s->d_adStat.p, prog->adaptive->tolerance,
                    prog->adaptive->minChunks, s->d_adActive.p);
-        else if (p.useAccum && pl.mode == OutMode::Aov) LAUNCH(k_resolve<true>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p, here);
-        else if (p.useAccum) LAUNCH(k_resolve<false>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p, here);
+        else if (p.useAccum && pl.mode == OutMode::Aov) LAUNCH(k_resolve<true>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p);
+        else if (p.useAccum) LAUNCH(k_resolve<false>, div_up((long long)here * p.localWidth, 256), 256, 0, st, p);
     }
     CU_TRY(cudaGetLastError());
     return TMPT_OK;
@@ -2343,8 +2344,8 @@ static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int
     CU_TRY(cudaMemsetAsync(s->d_rayCount.p, 0, sizeof(unsigned long long), st));
     uint32_t listLen = 0;
     if (ad) {  // select + compact: the active list and its length (one small copy)
-        const int tilesX = div_up(width, 8);
-        const long long slots = (long long)tilesX * div_up(height, 4) * 32;
+        const int tilesX = div_up(width, kTileW);
+        const long long slots = (long long)tilesX * div_up(height, kTileH) * 32;
         const int nBlocks = div_up(slots, kScanBlock);
         LAUNCH(k_adaptive_select, div_up(slots, 256), 256, 0, st, s->d_adN.p, s->d_adStat.p, width, height, tilesX, slots, ad->tolerance, ad->minChunks,
                s->d_adFlags.p);
@@ -2444,8 +2445,8 @@ extern "C" int tmpt_progressive_pass_outputs(tmpt_scene* s, const tmpt_camera* c
 
 // The per-pixel state of adaptive passes, for a progW x progH session: zeroed with the session's first adaptive pass.
 static int begin_adaptive(tmpt_scene* s, cudaStream_t st) {
-    const int tilesX = div_up(s->progW, 8);
-    const size_t slots = (size_t)tilesX * div_up(s->progH, 4) * 32, pixels = (size_t)s->progW * s->progH;
+    const int tilesX = div_up(s->progW, kTileW);
+    const size_t slots = (size_t)tilesX * div_up(s->progH, kTileH) * 32, pixels = (size_t)s->progW * s->progH;
     CU_TRY(s->d_adN.grow(slots, st));
     CU_TRY(s->d_adStat.grow(slots, st));
     CU_TRY(s->d_adFlags.grow(slots, st));
