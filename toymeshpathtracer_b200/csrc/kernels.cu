@@ -26,6 +26,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "build_logic.cuh"
@@ -145,7 +146,7 @@ struct tmpt_scene {
     float4* d_hitdata = nullptr;   // per original triangle: vertices + precomputed normal
     uint32_t* d_parent = nullptr;  // per wide node: parent index (refit)
     uint32_t* d_pending = nullptr; // per wide node: inner children not yet refitted (refit scratch)
-    uint32_t* d_bounds = nullptr;  // scene bounds as ordered uints (refit scratch)
+    uint32_t* d_bounds = nullptr;  // scene bounds as ordered uints (written by build and refit)
     DevBuf<uint32_t> d_status;     // [0] status bits
     // render scratch
     DevBuf<uint32_t> d_tileCounter;
@@ -1435,6 +1436,79 @@ float bvh_far_limit(const tmpt_scene_info& info) {
     return 16.0f * m;
 }
 
+// The geometry step of build and refit, from s->d_tris9: the scene bounds as ordered uints into s->d_bounds, and the hit payload.
+int launch_scene_geometry(tmpt_scene* s, cudaStream_t st) {
+    const int n = s->triCount, B = 256, G = div_up(n, B);
+    const uint32_t initBounds[6] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0u, 0u, 0u};
+    CU_TRY(cudaMemcpyAsync(s->d_bounds, initBounds, sizeof initBounds, cudaMemcpyHostToDevice, st));
+    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9.p, n, s->d_bounds);
+    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9.p, n, s->d_hitdata);
+    return TMPT_OK;
+}
+// hb = the host copy of s->d_bounds: the scene bounds the info reports, and the far-ray limit that follows from them
+void set_scene_bounds(tmpt_scene* s, const uint32_t hb[6]) {
+    for (int k = 0; k < 3; ++k) {
+        s->info.bounds_min[k] = bld::ordered_to_float(hb[k]);
+        s->info.bounds_max[k] = bld::ordered_to_float(hb[3 + k]);
+    }
+    s->view.farLimit = bvh_far_limit(s->info);
+}
+// -DTMPT_QNODES=1: the walk reads a quantised copy of the wide nodes, remade whenever they change
+int quantize_nodes(tmpt_scene* s, uint32_t nodes, cudaStream_t st) {
+#if TMPT_QNODES
+    CU_TRY(s->d_qnodes.grow((size_t)nodes * bvh::QNODE_STRIDE, st));
+    LAUNCH(k_quantize_nodes, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, s->d_qnodes.p, nodes);
+#endif
+    return TMPT_OK;
+}
+
+// The build's scratch for n triangles, typed as the kernels take it.  Every array comes out of ONE allocation, at a 256-byte
+// boundary (a dozen cudaMalloc/cudaFree pairs cost more than the kernels).
+struct BuildScratch {
+    bld::BinTree t;                     // either builder's binary tree (keys = keysA)
+    uint32_t *primA, *primB;            // triangle order, double-buffered; the final order ends in primA
+    uint32_t *counters, *qCount;        // bld::WideOut::counters; the queue counters (three rotate in the cooperative kernels)
+    float* sah;                         // bld::WideOut::sahAccum
+    uint64_t *keysA, *keysB;            // LBVH: Morton keys, double-buffered by the radix sort
+    float4 *pLo, *pHi;                  // SAH: padded triangle boxes
+    uint32_t *primFinal, *nodeCounter;  // SAH: the final order in each leaf's range; binary nodes allocated
+    SahTask *tqA, *tqB;                 // SAH: task queues of one level and the next
+    bld::WorkItem *qA, *qB;             // collapse: work queues of one level and the next
+};
+// Lays the scratch out at `base` and returns its size in bytes (base == nullptr: only the size).
+size_t lay_out_build_scratch(char* base, int n, BuildScratch* b) {
+    const size_t N = (size_t)n;
+    size_t off = 0;
+    auto carve = [&](auto*& p, size_t count) {
+        p = reinterpret_cast<std::decay_t<decltype(p)>>(reinterpret_cast<uintptr_t>(base) + off);
+        off += (count * sizeof *p + 255) & ~(size_t)255;
+    };
+    carve(b->primA, N); carve(b->primB, N); carve(b->t.visits, N); carve(b->counters, 4); carve(b->qCount, 4);
+    carve(b->keysA, N); carve(b->keysB, N);
+    carve(b->t.left, 2 * N); carve(b->t.right, 2 * N); carve(b->t.parent, 2 * N); carve(b->t.first, 2 * N); carve(b->t.lo, 2 * N); carve(b->t.hi, 2 * N);
+    carve(b->sah, 2); carve(b->qA, N); carve(b->qB, N);
+    carve(b->pLo, N); carve(b->pHi, N); carve(b->primFinal, N); carve(b->nodeCounter, 1); carve(b->tqA, N); carve(b->tqB, N);
+    b->t.n = n;
+    b->t.keys = b->keysA;
+    return off;
+}
+
+// The level loop of k_sah_build or k_collapse_all in one cooperative launch: its three rotating task counters `counts` start at
+// {1, 0, 0}, and as many CTAs run as fit co-resident, at most maxGrid.  *ran = false when the device refuses the launch (e.g. it
+// is shared and the grid cannot be co-resident).  That is not an error: nothing has run, and the caller's per-level loop does the
+// same work.
+int launch_level_loop(tmpt_scene* s, const void* kernel, int threads, int maxGrid, uint32_t* counts, void** args, bool* ran) {
+    const uint32_t counts0[3] = {1u, 0u, 0u};
+    CU_TRY(cudaMemcpyAsync(counts, counts0, sizeof counts0, cudaMemcpyHostToDevice, s->stream));
+    int perSM = 0;
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kernel, threads, 0));
+    const int grid = std::max(1, std::min(s->smCount * std::max(perSM, 1), maxGrid));
+    *ran = cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(threads), args, 0, s->stream) == cudaSuccess;
+    if (*ran) tmpt::count_launch();
+    else cudaGetLastError();
+    return TMPT_OK;
+}
+
 constexpr int kTreeTooDeep = -100;  // internal: tmpt_scene_create falls back to the depth-bounded default builder
 
 int build_bvh(tmpt_scene* s, unsigned flags) {
@@ -1449,23 +1523,10 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
     const bool coop = coopAttr != 0 && !(getenv("TMPT_BUILD_HOSTLOOP") && atoi(getenv("TMPT_BUILD_HOSTLOOP")) != 0);
     const int maxLeaf = getenv("TMPT_SAH_MAXLEAF") ? std::max(1, std::min(bvh::MAX_LEAF_TRIS, atoi(getenv("TMPT_SAH_MAXLEAF")))) : bvh::MAX_LEAF_TRIS;
 
-    // every build scratch array comes out of ONE allocation (a dozen cudaMalloc/cudaFree pairs cost more than the kernels)
-    struct Arr { void* p = nullptr; };
-    Arr bounds, primA, primB, visits, counters, qCount, keysA, keysB, left, right, parent, first, lo, hi, sah, qA, qB, pLo, pHi, primFinal, nodeCounter, tqA, tqB;
+    BuildScratch b;
     DevBuf<char> arena;
-    {
-        const size_t N = (size_t)n;
-        struct Req { Arr* a; size_t bytes; };
-        const Req reqs[] = {{&bounds, 6 * 4}, {&primA, N * 4}, {&primB, N * 4}, {&visits, N * 4}, {&counters, 4 * 4}, {&qCount, 4 * 4}, {&keysA, N * 8},
-                            {&keysB, N * 8}, {&left, 2 * N * 4}, {&right, 2 * N * 4}, {&parent, 2 * N * 4}, {&first, 2 * N * 4}, {&lo, 2 * N * 16},
-                            {&hi, 2 * N * 16}, {&sah, 2 * 4}, {&qA, N * sizeof(bld::WorkItem)}, {&qB, N * sizeof(bld::WorkItem)}, {&pLo, N * 16},
-                            {&pHi, N * 16}, {&primFinal, N * 4}, {&nodeCounter, 4}, {&tqA, N * sizeof(SahTask)}, {&tqB, N * sizeof(SahTask)}};
-        size_t total = 0;
-        for (const Req& r : reqs) total += (r.bytes + 255) & ~(size_t)255;
-        CU_TRY(arena.grow(total, st));
-        size_t off = 0;
-        for (const Req& r : reqs) { r.a->p = arena.p + off; off += (r.bytes + 255) & ~(size_t)255; }
-    }
+    CU_TRY(arena.grow(lay_out_build_scratch(nullptr, n, &b), st));
+    lay_out_build_scratch(arena.p, n, &b);
     // nodes, slots and hit payload share one allocation (each cudaMalloc costs as much as a build kernel)
     CU_TRY(s->d_nodes.grow((size_t)n * (bvh::NODE_F4 + 3 + 3) + div_up((long long)n * 2 + 8, sizeof(float4) / sizeof(uint32_t)), st));
     s->d_tris = s->d_nodes.p + (size_t)n * bvh::NODE_F4;
@@ -1474,82 +1535,50 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
     s->d_pending = s->d_parent + n;
     s->d_bounds = s->d_pending + n;
     CU_TRY(cudaMemsetAsync(s->d_parent, 0, sizeof(uint32_t), st));  // the root is its own parent
-
-    uint32_t* const d_bounds = (uint32_t*)bounds.p; uint32_t* const d_primA = (uint32_t*)primA.p; uint32_t* const d_primB = (uint32_t*)primB.p;
-    uint32_t* const d_visits = (uint32_t*)visits.p; uint32_t* const d_counters = (uint32_t*)counters.p; uint32_t* const d_qCount = (uint32_t*)qCount.p;
-    uint64_t* const d_keysA = (uint64_t*)keysA.p; uint64_t* const d_keysB = (uint64_t*)keysB.p;
-    int* const d_left = (int*)left.p; int* const d_right = (int*)right.p; int* const d_parent = (int*)parent.p; int* const d_first = (int*)first.p;
-    float4* const d_lo = (float4*)lo.p; float4* const d_hi = (float4*)hi.p; float* const d_sah = (float*)sah.p;
-    bld::WorkItem* const d_qA = (bld::WorkItem*)qA.p; bld::WorkItem* const d_qB = (bld::WorkItem*)qB.p;
-    const uint32_t initBounds[6] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0u, 0u, 0u};
-    CU_TRY(cudaMemcpyAsync(d_bounds, initBounds, sizeof initBounds, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemsetAsync(d_visits, 0, (size_t)n * sizeof(uint32_t), st));
-    CU_TRY(cudaMemsetAsync(d_counters, 0, 4 * sizeof(uint32_t), st));
-    CU_TRY(cudaMemsetAsync(d_sah, 0, 2 * sizeof(float), st));
-    CU_TRY(cudaMemsetAsync(d_parent, 0xFF, 2 * (size_t)n * sizeof(int), st));
+    CU_TRY(cudaMemsetAsync(b.t.visits, 0, (size_t)n * sizeof(uint32_t), st));
+    CU_TRY(cudaMemsetAsync(b.counters, 0, 4 * sizeof(uint32_t), st));
+    CU_TRY(cudaMemsetAsync(b.sah, 0, 2 * sizeof(float), st));
+    CU_TRY(cudaMemsetAsync(b.t.parent, 0xFF, 2 * (size_t)n * sizeof(int), st));
+    TRY(launch_scene_geometry(s, st));
 
     const int B = 256, G = div_up(n, B);
-    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9.p, n, d_bounds);
-    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9.p, n, s->d_hitdata);
-    bld::BinTree t{n, d_keysA, d_left, d_right, d_parent, d_lo, d_hi, d_first, d_visits};
+    const uint32_t one = 1, zero = 0;
     bld::SahParams sp{cInner, cTri, maxLeaf};
-    const uint32_t* primOrder = d_primA;
     int rootIsLeaf = (n == 1);
     if (flags & TMPT_BUILD_LBVH) {
-        LAUNCH(k_morton, G, B, 0, st, s->d_tris9.p, n, d_bounds, d_keysA, d_primA);
+        LAUNCH(k_morton, G, B, 0, st, s->d_tris9.p, n, s->d_bounds, b.keysA, b.primA);
         const int passes = 16;  // 63-bit keys, 4 bits per pass; an even count leaves the result in A
         const int sortSmem = 16 * SORT_THREADS * (int)sizeof(uint32_t);
         CU_TRY(cudaFuncSetAttribute(k_radix_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, sortSmem));
-        LAUNCH(k_radix_sort, 1, SORT_THREADS, sortSmem, st, d_keysA, d_primA, d_keysB, d_primB, n, passes);
-        LAUNCH(k_leaf_boxes, G, B, 0, st, s->d_tris9.p, d_primA, n, d_bounds, cTri, d_lo, d_hi, d_first);
+        LAUNCH(k_radix_sort, 1, SORT_THREADS, sortSmem, st, b.keysA, b.primA, b.keysB, b.primB, n, passes);
+        LAUNCH(k_leaf_boxes, G, B, 0, st, s->d_tris9.p, b.primA, n, s->d_bounds, cTri, b.t.lo, b.t.hi, b.t.first);
         if (n > 1) {
-            LAUNCH(k_karras, div_up(n - 1, B), B, 0, st, t);
-            LAUNCH(k_refit, G, B, 0, st, t, sp);
+            LAUNCH(k_karras, div_up(n - 1, B), B, 0, st, b.t);
+            LAUNCH(k_refit, G, B, 0, st, b.t, sp);
         }
         s->info.builder = TMPT_BUILD_LBVH;
     } else {
-        // binned SAH, level by level; tasks double-buffer in the collapse queues' memory
-        float4* const d_pLo = (float4*)pLo.p; float4* const d_pHi = (float4*)pHi.p;
-        uint32_t* const d_primFinal = (uint32_t*)primFinal.p; uint32_t* const d_nodeCounter = (uint32_t*)nodeCounter.p;
-        SahTask* const d_tqA = (SahTask*)tqA.p; SahTask* const d_tqB = (SahTask*)tqB.p;
-        LAUNCH(k_prim_boxes, G, B, 0, st, s->d_tris9.p, n, d_bounds, d_pLo, d_pHi, d_primA);
+        // binned SAH, level by level
+        LAUNCH(k_prim_boxes, G, B, 0, st, s->d_tris9.p, n, s->d_bounds, b.pLo, b.pHi, b.primA);
         const SahTask rootTask{0, 0, n, 0};
-        const uint32_t one = 1, zero = 0;
-        CU_TRY(cudaMemcpyAsync(d_tqA, &rootTask, sizeof rootTask, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(d_nodeCounter, &one, 4, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(b.tqA, &rootTask, sizeof rootTask, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(b.nodeCounter, &one, 4, cudaMemcpyHostToDevice, st));
         bool sahDone = false;
         if (coop) {
-            // one cooperative launch for all levels (k_sah_build); d_qCount = three rotating task counters
-            const uint32_t counts0[3] = {1u, 0u, 0u};
-            CU_TRY(cudaMemcpyAsync(d_qCount, counts0, sizeof counts0, cudaMemcpyHostToDevice, st));
-            int perSM = 0;
-            CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_sah_build, SAH_THREADS, 0));
-            const int grid = std::max(1, std::min(s->smCount * std::max(perSM, 1), n));
-            uint32_t* idxA = d_primA; uint32_t* idxB = d_primB;
-            SahTask* qA = d_tqA; SahTask* qB = d_tqB;
-            uint32_t* countsP = d_qCount; uint32_t* nodeCounterP = d_nodeCounter; uint32_t* primFinalP = d_primFinal;
-            const float4* pLoP = d_pLo; const float4* pHiP = d_pHi;
             int maxLevels = 4096;
             uint32_t* statusP = s->d_status.p + 1;
-            void* args[] = {&t, &pLoP, &pHiP, &idxA, &idxB, &primFinalP, &qA, &qB, &countsP, &nodeCounterP, &sp, &maxLevels, &statusP};
-            // (a refused cooperative launch -- e.g. the device is shared and the grid cannot be co-resident -- is not an error:
-            //  nothing has run yet, the per-level loop below does the same work)
-            if (cudaLaunchCooperativeKernel((void*)k_sah_build, dim3(grid), dim3(SAH_THREADS), args, 0, st) == cudaSuccess) {
-                tmpt::count_launch();
-                sahDone = true;
-            } else {
-                cudaGetLastError();
-            }
+            void* args[] = {&b.t, &b.pLo, &b.pHi, &b.primA, &b.primB, &b.primFinal, &b.tqA, &b.tqB, &b.qCount, &b.nodeCounter, &sp, &maxLevels, &statusP};
+            TRY(launch_level_loop(s, (const void*)k_sah_build, SAH_THREADS, n, b.qCount, args, &sahDone));
         }
         if (!sahDone) {
-            uint32_t* idxIn = d_primA; uint32_t* idxOut = d_primB;
-            SahTask* qin = d_tqA; SahTask* qout = d_tqB;
+            uint32_t* idxIn = b.primA; uint32_t* idxOut = b.primB;
+            SahTask* qin = b.tqA; SahTask* qout = b.tqB;
             uint32_t count = 1;
             int levels = 0;
             while (count > 0) {
-                CU_TRY(cudaMemcpyAsync(d_qCount, &zero, 4, cudaMemcpyHostToDevice, st));
-                LAUNCH(k_sah_level, count, SAH_THREADS, 0, st, t, d_pLo, d_pHi, idxIn, idxOut, d_primFinal, qin, qout, d_qCount, d_nodeCounter, sp);
-                CU_TRY(cudaMemcpyAsync(&count, d_qCount, 4, cudaMemcpyDeviceToHost, st));
+                CU_TRY(cudaMemcpyAsync(b.qCount, &zero, 4, cudaMemcpyHostToDevice, st));
+                LAUNCH(k_sah_level, count, SAH_THREADS, 0, st, b.t, b.pLo, b.pHi, idxIn, idxOut, b.primFinal, qin, qout, b.qCount, b.nodeCounter, sp);
+                CU_TRY(cudaMemcpyAsync(&count, b.qCount, 4, cudaMemcpyDeviceToHost, st));
                 CU_TRY(cudaStreamSynchronize(st));
                 std::swap(idxIn, idxOut);
                 std::swap(qin, qout);
@@ -1557,14 +1586,14 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
             }
         }
         // the final order lives in primFinal; keep it in primA for the collapse (same stream, device copy)
-        CU_TRY(cudaMemcpyAsync(d_primA, d_primFinal, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+        CU_TRY(cudaMemcpyAsync(b.primA, b.primFinal, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
         s->info.builder = TMPT_BUILD_DEFAULT;
     }
-    bld::WideOut w{s->d_nodes.p, s->d_tris, s->d_tris9.p, primOrder, d_counters, d_sah, s->d_parent};
+    bld::WideOut w{s->d_nodes.p, s->d_tris, s->d_tris9.p, b.primA, b.counters, b.sah, s->d_parent};
     if (n > 1) {
         float4 rootHi;
         uint32_t bst = 0;
-        CU_TRY(cudaMemcpyAsync(&rootHi, d_hi, sizeof rootHi, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaMemcpyAsync(&rootHi, b.t.hi, sizeof rootHi, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaMemcpyAsync(&bst, s->d_status.p + 1, 4, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         if (bst & 2u) return tmpt::fail(TMPT_ERR_CUDA, "SAH build did not terminate");
@@ -1572,41 +1601,26 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         rootIsLeaf = c < 0;
     }
     if (rootIsLeaf) {
-        const uint32_t one = 1;
-        CU_TRY(cudaMemcpyAsync(d_counters, &one, 4, cudaMemcpyHostToDevice, st));
-        LAUNCH(k_collapse_root_leaf, 1, 1, 0, st, t, w, 0);
+        CU_TRY(cudaMemcpyAsync(b.counters, &one, 4, cudaMemcpyHostToDevice, st));
+        LAUNCH(k_collapse_root_leaf, 1, 1, 0, st, b.t, w, 0);
     } else {
         const bld::WorkItem root{0, 0u, 0};
-        const uint32_t one = 1, zero = 0;
-        CU_TRY(cudaMemcpyAsync(d_qA, &root, sizeof root, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(d_counters, &one, 4, cudaMemcpyHostToDevice, st));   // wide node 0 is taken
-        CU_TRY(cudaMemcpyAsync(d_qCount, &one, 4, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(b.qA, &root, sizeof root, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(b.counters, &one, 4, cudaMemcpyHostToDevice, st));   // wide node 0 is taken
         bool collapseDone = false;
         if (coop) {
-            const uint32_t counts0[3] = {1u, 0u, 0u};
-            CU_TRY(cudaMemcpyAsync(d_qCount, counts0, sizeof counts0, cudaMemcpyHostToDevice, st));
-            int perSM = 0;
-            CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_collapse_all, 128, 0));
-            const int grid = std::max(1, std::min(s->smCount * std::max(perSM, 1), div_up(n, 128)));
-            bld::WorkItem* qA = d_qA; bld::WorkItem* qB = d_qB;
-            uint32_t* countsP = d_qCount;
-            void* args[] = {&t, &w, &qA, &qB, &countsP};
-            if (cudaLaunchCooperativeKernel((void*)k_collapse_all, dim3(grid), dim3(128), args, 0, st) == cudaSuccess) {
-                tmpt::count_launch();
-                collapseDone = true;
-            } else {
-                cudaGetLastError();
-            }
+            void* args[] = {&b.t, &w, &b.qA, &b.qB, &b.qCount};
+            TRY(launch_level_loop(s, (const void*)k_collapse_all, 128, div_up(n, 128), b.qCount, args, &collapseDone));
         }
         if (!collapseDone) {
-            CU_TRY(cudaMemcpyAsync(d_qCount, &one, 4, cudaMemcpyHostToDevice, st));
-            bld::WorkItem* qin = d_qA; bld::WorkItem* qout = d_qB;
+            CU_TRY(cudaMemcpyAsync(b.qCount, &one, 4, cudaMemcpyHostToDevice, st));
+            bld::WorkItem* qin = b.qA; bld::WorkItem* qout = b.qB;
             int cin = 0;
             uint32_t count = 1;
             while (count > 0) {
-                CU_TRY(cudaMemcpyAsync(d_qCount + (1 - cin), &zero, 4, cudaMemcpyHostToDevice, st));
-                LAUNCH(k_collapse, div_up(count, 128), 128, 0, st, t, w, qin, d_qCount + cin, qout, d_qCount + (1 - cin));
-                CU_TRY(cudaMemcpyAsync(&count, d_qCount + (1 - cin), 4, cudaMemcpyDeviceToHost, st));
+                CU_TRY(cudaMemcpyAsync(b.qCount + (1 - cin), &zero, 4, cudaMemcpyHostToDevice, st));
+                LAUNCH(k_collapse, div_up(count, 128), 128, 0, st, b.t, w, qin, b.qCount + cin, qout, b.qCount + (1 - cin));
+                CU_TRY(cudaMemcpyAsync(&count, b.qCount + (1 - cin), 4, cudaMemcpyDeviceToHost, st));
                 CU_TRY(cudaStreamSynchronize(st));
                 cin = 1 - cin;
                 bld::WorkItem* tq = qin; qin = qout; qout = tq;
@@ -1614,19 +1628,16 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         }
     }
     uint32_t hc[4]; float hs[2]; uint32_t hb[6];
-    CU_TRY(cudaMemcpyAsync(hc, d_counters, sizeof hc, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(hs, d_sah, sizeof hs, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(hb, d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(hc, b.counters, sizeof hc, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(hs, b.sah, sizeof hs, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(hb, s->d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     CU_TRY(cudaGetLastError());
     s->info.node_count = (int)hc[0];
     s->info.leaf_count = (int)hc[2];
     s->info.max_depth = (int)hc[3] + 1;
     s->info.max_leaf_tris = bvh::MAX_LEAF_TRIS;
-    for (int k = 0; k < 3; ++k) {
-        s->info.bounds_min[k] = bld::ordered_to_float(hb[k]);
-        s->info.bounds_max[k] = bld::ordered_to_float(hb[3 + k]);
-    }
+    set_scene_bounds(s, hb);
     {
         const float dx = s->info.bounds_max[0] - s->info.bounds_min[0], dy = s->info.bounds_max[1] - s->info.bounds_min[1],
                     dz = s->info.bounds_max[2] - s->info.bounds_min[2];
@@ -1634,10 +1645,7 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
         s->info.sah_cost = rootArea > 0.0f ? (cInner * hs[0] + cTri * hs[1]) / rootArea : 0.0f;
     }
     if ((int)hc[1] != n) return tmpt::fail(TMPT_ERR_CUDA, "BVH build lost triangles: %u slots for %d triangles", hc[1], n);
-#if TMPT_QNODES
-    CU_TRY(s->d_qnodes.grow((size_t)hc[0] * bvh::QNODE_STRIDE, st));
-    LAUNCH(k_quantize_nodes, div_up((int)hc[0], 128), 128, 0, st, s->d_nodes.p, s->d_qnodes.p, hc[0]);
-#endif
+    TRY(quantize_nodes(s, hc[0], st));
     // the traversal stack holds at most 3 entries per level (bvh::wide_node_step): refuse what it could not hold.  The default
     // builder cannot get here (bld::sah_must_halve bounds its depth for any input); a Morton tree over many coincident centres can.
     if (3 * s->info.max_depth + 4 > bvh::STACK_SIZE) {
@@ -1654,7 +1662,6 @@ int build_bvh(tmpt_scene* s, unsigned flags) {
     s->view.rootRef = 0u;
     s->view.triCount = n;
     s->view.status = s->d_status.p;
-    s->view.farLimit = bvh_far_limit(s->info);
     return TMPT_OK;
 }
 
@@ -1728,6 +1735,19 @@ struct DeviceGuard {
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 }  // namespace
+
+// The end of a timed window that began with s->ev0 on `st`: records s->ev1, then (outside the window) copies the device counter
+// `countDev` to *count if given, waits for the stream and returns the window's length in *seconds.
+static int end_timed_window(tmpt_scene* s, cudaStream_t st, double* seconds, const unsigned long long* countDev = nullptr,
+                            unsigned long long* count = nullptr) {
+    CU_TRY(cudaEventRecord(s->ev1, st));
+    if (countDev) CU_TRY(cudaMemcpyAsync(count, countDev, sizeof *count, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    float ms = 0.0f;
+    CU_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    if (seconds) *seconds = (double)ms * 1.0e-3;
+    return TMPT_OK;
+}
 
 // ------------------------------------------------------------------------------------------
 // C ABI: scene
@@ -1809,38 +1829,22 @@ extern "C" int tmpt_scene_refit(tmpt_scene* s, const float* tris9, int triCount,
     DeviceGuard guard(s->device);
     if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "tmpt_scene_refit: cudaSetDevice(%d) failed", s->device);
     cudaStream_t st = s->stream;
-    const int n = triCount, B = 256, G = div_up(n, B), nodes = s->info.node_count;
+    const int n = triCount, nodes = s->info.node_count;
     CU_TRY(cudaEventRecord(s->ev0, st));
     CU_TRY(cudaMemcpyAsync(s->d_tris9.p, tris9, (size_t)n * 9 * sizeof(float), cudaMemcpyHostToDevice, st));
-    const uint32_t initBounds[6] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0u, 0u, 0u};
-    CU_TRY(cudaMemcpyAsync(s->d_bounds, initBounds, sizeof initBounds, cudaMemcpyHostToDevice, st));
-    LAUNCH(k_prim_bounds, G, B, 0, st, s->d_tris9.p, n, s->d_bounds);
-    LAUNCH(k_hitdata, G, B, 0, st, s->d_tris9.p, n, s->d_hitdata);
+    TRY(launch_scene_geometry(s, st));
     LAUNCH(k_refit_pending, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, (uint32_t)nodes, s->d_pending);
     LAUNCH(k_refit_wide, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, s->d_tris, s->d_tris9.p, s->d_parent, s->d_pending, (uint32_t)nodes, s->d_bounds);
-#if TMPT_QNODES
-    LAUNCH(k_quantize_nodes, div_up(nodes, 128), 128, 0, st, s->d_nodes.p, s->d_qnodes.p, (uint32_t)nodes);
-#endif
+    TRY(quantize_nodes(s, (uint32_t)nodes, st));
     uint32_t hb[6];
     CU_TRY(cudaMemcpyAsync(hb, s->d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     CU_TRY(cudaGetLastError());
-    for (int k = 0; k < 3; ++k) {
-        s->info.bounds_min[k] = bld::ordered_to_float(hb[k]);
-        s->info.bounds_max[k] = bld::ordered_to_float(hb[3 + k]);
-    }
-    {  // the shadow rays' grid is rebuilt for the new positions and bounds (inside the timed window)
-        const int grc = build_sun_grid(s, n, st);
-        if (grc != TMPT_OK) return grc;
-    }
-    CU_TRY(cudaEventRecord(s->ev1, st));
-    CU_TRY(cudaStreamSynchronize(st));
+    set_scene_bounds(s, hb);
+    TRY(build_sun_grid(s, n, st));  // the shadow rays' grid, rebuilt for the new positions and bounds (inside the timed window)
+    TRY(end_timed_window(s, st, seconds));
     CU_TRY(cudaGetLastError());
-    s->view.farLimit = bvh_far_limit(s->info);
     s->probeW = 0;  // moved geometry: the next frame probes again (k_probe_paths)
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    if (seconds) *seconds = ms * 1e-3;
     return TMPT_OK;
 }
 
@@ -1872,6 +1876,18 @@ static int check_status(const tmpt_scene* s, cudaStream_t st) {
 // ------------------------------------------------------------------------------------------
 // C ABI: HitScene
 // ------------------------------------------------------------------------------------------
+using HitKernel = void (*)(bvh::SceneView, const float*, long long, float, float, int*, float*, float*, float*, unsigned long long*);
+// The k_hit_scene instantiation of a checked query mode; stats: the instrumented one (CLOSEST, ANY and SUN only)
+static HitKernel hit_kernel(int mode, bool stats) {
+    if (mode == TMPT_HIT_CLOSEST) return stats ? k_hit_scene<TMPT_HIT_CLOSEST, true> : k_hit_scene<TMPT_HIT_CLOSEST, false>;
+    if (mode == TMPT_HIT_ANY) return stats ? k_hit_scene<TMPT_HIT_ANY, true> : k_hit_scene<TMPT_HIT_ANY, false>;
+    if (mode == TMPT_HIT_SUN) return stats ? k_hit_scene<TMPT_HIT_SUN, true> : k_hit_scene<TMPT_HIT_SUN, false>;
+    return k_hit_scene<TMPT_HIT_BRUTE, false>;
+}
+constexpr int kHitThreads = 128;
+// the rays in a grid-stride loop: at most 64 CTAs per SM
+static int hit_grid(const tmpt_scene* s, int64_t nRays) { return (int)std::min<long long>(div_up(nRays, kHitThreads), (long long)s->smCount * 64); }
+
 extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t nRays, float tMin, float tMax, int mode, int mem,
                               int32_t* outID, float* outT, float* outPos3, float* outNormal3, void* stream) {
     if (!s || nRays < 0 || (nRays > 0 && (!rays6 || !outID))) return tmpt::fail(TMPT_ERR_ARG, "tmpt_hit_scene: NULL scene / rays / outID");
@@ -1905,8 +1921,6 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
         dRays = (const float*)d; dID = (int*)(d + offID);
         dT = outT ? (float*)(d + offT) : nullptr; dPos = outPos3 ? (float*)(d + offPos) : nullptr; dNrm = outNormal3 ? (float*)(d + offNrm) : nullptr;
     }
-    const int B = 128;
-    const int G = (int)std::min<long long>(div_up(nRays, B), (long long)s->smCount * 64);
     if (getenv("TMPT_HIT_KERNEL") && atoi(getenv("TMPT_HIT_KERNEL")) > 0)
         return tmpt::fail(TMPT_ERR_ARG, "TMPT_HIT_KERNEL: the experimental HitScene kernels of round 1 were removed (see profiles/r1_hit_scene_variants_ncu.txt)");
 #if TMPT_EXPERIMENTS
@@ -1916,9 +1930,9 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
         int perSM = 0;
 #define REFILL_CASE(M, GT)                                                                                                     \
         if (mode == M && refillGate == GT) {                                                                                   \
-            CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_hit_scene_refill<M, GT>, B, 0));                    \
-            const int GP = (int)std::min<long long>(div_up(nRays, B), (long long)s->smCount * std::max(perSM, 1));            \
-            LAUNCH((k_hit_scene_refill<M, GT>), GP, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, s->d_fetchCounter.p); \
+            CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_hit_scene_refill<M, GT>, kHitThreads, 0));          \
+            const int GP = (int)std::min<long long>(div_up(nRays, kHitThreads), (long long)s->smCount * std::max(perSM, 1));  \
+            LAUNCH((k_hit_scene_refill<M, GT>), GP, kHitThreads, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, s->d_fetchCounter.p); \
         } else
         REFILL_CASE(TMPT_HIT_CLOSEST, 1) REFILL_CASE(TMPT_HIT_CLOSEST, 4) REFILL_CASE(TMPT_HIT_CLOSEST, 8) REFILL_CASE(TMPT_HIT_CLOSEST, 16)
         REFILL_CASE(TMPT_HIT_ANY, 1) REFILL_CASE(TMPT_HIT_ANY, 4) REFILL_CASE(TMPT_HIT_ANY, 8) REFILL_CASE(TMPT_HIT_ANY, 16)
@@ -1926,10 +1940,7 @@ extern "C" int tmpt_hit_scene(const tmpt_scene* s, const float* rays6, int64_t n
         return tmpt::fail(TMPT_ERR_ARG, "TMPT_HIT_REFILL=%d: gates are 1, 4, 8, 16", refillGate);
     } else
 #endif
-    if (mode == TMPT_HIT_CLOSEST) LAUNCH((k_hit_scene<TMPT_HIT_CLOSEST, false>), G, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
-    else if (mode == TMPT_HIT_ANY) LAUNCH((k_hit_scene<TMPT_HIT_ANY, false>), G, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
-    else if (mode == TMPT_HIT_SUN) LAUNCH((k_hit_scene<TMPT_HIT_SUN, false>), G, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
-    else LAUNCH((k_hit_scene<TMPT_HIT_BRUTE, false>), G, B, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
+    LAUNCH(hit_kernel(mode, false), hit_grid(s, nRays), kHitThreads, 0, st, s->view, dRays, (long long)nRays, tMin, tMax, dID, dT, dPos, dNrm, nullptr);
     CU_TRY(cudaGetLastError());
     if (mem == TMPT_HOST) {
         const char* d = s->d_stage.p; char* h = s->h_stage.p;
@@ -2309,19 +2320,6 @@ struct Staging {
     }
 };
 
-// The end of a timed window that began with s->ev0 on `st`: records s->ev1, then (outside the window) copies the device counter
-// `countDev` to *count if given, waits for the stream and returns the window's length in *seconds.
-static int end_timed_window(tmpt_scene* s, cudaStream_t st, double* seconds, const unsigned long long* countDev = nullptr,
-                            unsigned long long* count = nullptr) {
-    CU_TRY(cudaEventRecord(s->ev1, st));
-    if (countDev) CU_TRY(cudaMemcpyAsync(count, countDev, sizeof *count, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    if (seconds) *seconds = (double)ms * 1.0e-3;
-    return TMPT_OK;
-}
-
 // One single-GPU frame (prog == nullptr) or progressive pass into the buffers `out` names: with TMPT_HOST each requested buffer is
 // staged in the scene's device scratch and copied out inside the timed window; the kernels always write an RGBA frame (the scene's
 // scratch frame when the caller asks for none).  An adaptive pass reports into *adOut.  The caller holds hostCallMutex and the device.
@@ -2683,11 +2681,7 @@ extern "C" int tmpt_hit_scene_stats(const tmpt_scene* s, const float* rays6Dev, 
     CU_TRY(stats.grow(TMPT_STATS_COUNT, st));
     CU_TRY(ids.grow((size_t)nRays, st));
     CU_TRY(cudaMemsetAsync(stats.p, 0, TMPT_STATS_COUNT * sizeof(unsigned long long), st));
-    const int B = 128;
-    const int G = (int)std::min<long long>(div_up(nRays, B), (long long)s->smCount * 64);
-    if (mode == TMPT_HIT_CLOSEST) LAUNCH((k_hit_scene<TMPT_HIT_CLOSEST, true>), G, B, 0, st, s->view, rays6Dev, (long long)nRays, tMin, tMax, ids.p, nullptr, nullptr, nullptr, stats.p);
-    else if (mode == TMPT_HIT_SUN) LAUNCH((k_hit_scene<TMPT_HIT_SUN, true>), G, B, 0, st, s->view, rays6Dev, (long long)nRays, tMin, tMax, ids.p, nullptr, nullptr, nullptr, stats.p);
-    else LAUNCH((k_hit_scene<TMPT_HIT_ANY, true>), G, B, 0, st, s->view, rays6Dev, (long long)nRays, tMin, tMax, ids.p, nullptr, nullptr, nullptr, stats.p);
+    LAUNCH(hit_kernel(mode, true), hit_grid(s, nRays), kHitThreads, 0, st, s->view, rays6Dev, (long long)nRays, tMin, tMax, ids.p, nullptr, nullptr, nullptr, stats.p);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaMemcpyAsync(outStats, stats.p, TMPT_STATS_COUNT * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
