@@ -2108,9 +2108,11 @@ static RenderKernel shipped_render_kernel(bool paths, int cfg, bool far) {
     return {k_render<false, 256, 4, kSStack, false, MODE>, 256, 256 * b};
 }
 // The shipped render instantiation of a launch: k_render_paths (configurations 1 = 256 x 4 and 3 = 1024 x 1) or k_render
-// (1, 2 = 512 x 2, 3, and the far-camera one at 256 x 4) in the launch's output mode, or the instrumented pass (frame mode only).
+// (1, 2 = 512 x 2, 3, and the far-camera one at 256 x 4) in the launch's output mode, or the instrumented pass (frame mode only;
+// a far camera gets its FAR form too, so that it traces the rays the frame traces and counts the same rays).
 static RenderKernel render_kernel(OutMode mode, bool paths, int cfg, bool far, bool stats) {
-    if (stats) return {k_render<true, 256, 4, kSStack>, 256, 256 * kSStack * sizeof(unsigned long long)};
+    constexpr size_t sb = 256 * kSStack * sizeof(unsigned long long);
+    if (stats) return far ? RenderKernel{k_render<true, 256, 4, kSStack, true>, 256, sb} : RenderKernel{k_render<true, 256, 4, kSStack>, 256, sb};
     switch (mode) {
         case OutMode::Aov: return shipped_render_kernel<OutMode::Aov>(paths, cfg, far);
         case OutMode::List: return shipped_render_kernel<OutMode::List>(paths, cfg, far);
