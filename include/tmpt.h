@@ -156,6 +156,27 @@ typedef struct tmpt_outputs {
 int tmpt_render_outputs(const tmpt_scene* scene, const tmpt_camera* camera, int width, int height, int spp, int mem,
                         const tmpt_outputs* out, uint64_t* rayCount, double* seconds, void* stream);
 
+/* Beyond the reference: nViews frames of one size, one camera each, in one call (orbits, cube-map faces, stereo pairs,
+ * light-field grids).  The views share one work queue and one launch sequence, so small views keep the GPU busy.
+ *   cameras    a HOST array of nViews cameras (as tmpt_render's camera is a host pointer); the call uploads it into scratch
+ *              owned by the scene.
+ *   out        as tmpt_render_outputs, every buffer view-major: [nViews][height][width] with the per-pixel layout of
+ *              tmpt_render_outputs, row 0 = the bottom of each view.  View v of a buffer starts at v * width * height pixels,
+ *              so tmpt_denoise can run on one view of a batch through plain pointer offsets.
+ *   rayCount   the sum of the counts of the nViews single frames below.
+ *   mem / stream / seconds   as tmpt_render_outputs; with TMPT_HOST the buffers are staged in the scene's scratch, sized for
+ *              the whole batch.  A batch uses the scene's scratch like a frame does (calls take turns).
+ * Equality: view v of every buffer equals tmpt_render_outputs(cameras[v], width, height, spp) with the same outputs: bytes for
+ * rgba and triangle, bits for radiance, normal and depth, NaN included.
+ * RNG: every view uses the pixel streams of a single frame, seeded from (chunk, pixel index in its view).  Two views with the
+ * same camera are therefore identical, and the noise of different views is correlated.  This is deliberate: it is the price
+ * of the equality above.
+ * Errors, before any device work: TMPT_ERR_ARG for a NULL scene or cameras, nViews outside 1..65536, nViews * width * height
+ * above 10^8 (the reference's largest single frame), the range checks of tmpt_render, or the checks of tmpt_render_outputs'
+ * `out` and `mem`.  Single GPU; no progressive or adaptive form. */
+int tmpt_render_views(const tmpt_scene* scene, const tmpt_camera* cameras, int nViews, int width, int height, int spp,
+                      int mem, const tmpt_outputs* out, uint64_t* rayCount, double* seconds, void* stream);
+
 /* Progressive rendering (beyond the reference, SURVEY.md 8(f) rank 4): the frame converges over calls.
  * tmpt_progressive_begin fixes the frame size and clears the running per-pixel sums kept with the scene; every
  * tmpt_progressive_pass traces `nChunks` (1..128) more chunks of 8 samples per pixel with the SAME camera, adds them to

@@ -9,6 +9,8 @@ drive it through; it mirrors the reference's own interface names:
     Scene.HitScene(rays, tMin, tMax) Scene::HitScene, batched        (scene.h:36-37)
     Scene.render(camera, w, h, spp)  TraceImageBody over all rows    (main.cpp:180-246, 329-331)
     Scene.render_outputs(...)        the same frame plus linear radiance and first-hit AOVs (beyond the reference)
+    Scene.render_views(cams, ...)    a batch of views, one camera each, in one call: view v = render_outputs(cams[v])
+                                     (beyond the reference)
     Scene.denoise(...)               an a-trous filter over the radiance, guided by the AOVs (beyond the reference)
     load_scene(path)                 LoadScene                       (main.cpp:122-170)
     camera_for_scene(...)            camera placement of main()      (main.cpp:296-307)
@@ -42,6 +44,7 @@ ABI_SYMBOLS = [
     "tmpt_frame_alloc", "tmpt_frame_open", "tmpt_frame_close", "tmpt_frame_free", "tmpt_render_multi",
     "tmpt_scene_refit", "tmpt_progressive_begin", "tmpt_progressive_pass", "tmpt_render_kernel_choice",
     "tmpt_render_outputs", "tmpt_progressive_pass_outputs", "tmpt_progressive_pass_adaptive", "tmpt_denoise",
+    "tmpt_render_views",
 ]
 
 
@@ -57,6 +60,14 @@ OUTPUTS = ("rgba", "radiance", "normal", "depth", "triangle")  # the members of 
 class Outputs(C.Structure):
     """tmpt_outputs: one pointer per buffer, NULL = not produced."""
     _fields_ = [(name, C.c_void_p) for name in OUTPUTS]
+
+
+def _cameras(cameras) -> np.ndarray:
+    """A batch of cameras as the C ABI takes it: float32 [N, 22], C order."""
+    cams = _f32(cameras)
+    if cams.ndim != 2 or cams.shape[1] != 22:
+        raise ValueError(f"cameras must be an array [N, 22] (one camera_make result per view), not {cams.shape}")
+    return cams
 
 
 def _output_arrays(names, width: int, height: int) -> dict:
@@ -119,6 +130,7 @@ def lib() -> C.CDLL:
     L.tmpt_hit_scene.argtypes = [vp, vp, i64, f32, f32, i32, i32, vp, vp, vp, vp, vp]
     L.tmpt_render.argtypes = [vp, vp, i32, i32, i32, i32, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
     L.tmpt_render_outputs.argtypes = [vp, vp, i32, i32, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
+    L.tmpt_render_views.argtypes = [vp, vp, i32, i32, i32, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double), vp]
     L.tmpt_progressive_pass_outputs.argtypes = [vp, vp, i32, i32, C.POINTER(Outputs), C.POINTER(C.c_uint64), C.POINTER(C.c_double),
                                                 C.POINTER(i32), vp]
     L.tmpt_progressive_pass_adaptive.argtypes = [vp, vp, i32, C.POINTER(Adaptive), i32, C.POINTER(Outputs), vp, C.POINTER(C.c_uint64),
@@ -331,6 +343,29 @@ class Scene:
         rays, sec = C.c_uint64(0), C.c_double(0.0)
         _check(lib().tmpt_render_outputs(self._h, _ptr(cam), width, height, spp, DEVICE, C.byref(out), C.byref(rays), C.byref(sec),
                                          stream or None))
+        return rays.value, sec.value
+
+    def render_views(self, cameras, width: int, height: int, spp: int, outputs=OUTPUTS):
+        """nViews frames of one size in one call (tmpt_render_views): `cameras` is array-like [N, 22], e.g. np.stack of camera_make
+        results -> ({name: host array [N, h, w, ...]}, rayCount, seconds).  View v of every array equals render_outputs(cameras[v],
+        width, height, spp) byte for byte; rayCount is the sum of those frames' counts."""
+        cams = _cameras(cameras)
+        n = cams.shape[0]
+        arrays = _output_arrays(outputs, width, n * height)
+        out = Outputs(**{k: a.ctypes.data for k, a in arrays.items()})
+        rays, sec = C.c_uint64(0), C.c_double(0.0)
+        _check(lib().tmpt_render_views(self._h, _ptr(cams), n, width, height, spp, HOST, C.byref(out), C.byref(rays), C.byref(sec), None))
+        return {k: a.reshape((n, height) + a.shape[1:]) for k, a in arrays.items()}, rays.value, sec.value
+
+    def render_views_device(self, cameras, width: int, height: int, spp: int, rgba_ptr: int = 0, radiance_ptr: int = 0, normal_ptr: int = 0,
+                            depth_ptr: int = 0, triangle_ptr: int = 0, stream: int = 0):
+        """tmpt_render_views into view-major device buffers [N, h, w, ...] (raw addresses, e.g. torch ``data_ptr()``; 0 = not
+        produced) -> (rayCount, seconds)."""
+        cams = _cameras(cameras)
+        out = Outputs(rgba_ptr or None, radiance_ptr or None, normal_ptr or None, depth_ptr or None, triangle_ptr or None)
+        rays, sec = C.c_uint64(0), C.c_double(0.0)
+        _check(lib().tmpt_render_views(self._h, _ptr(cams), cams.shape[0], width, height, spp, DEVICE, C.byref(out), C.byref(rays),
+                                       C.byref(sec), stream or None))
         return rays.value, sec.value
 
     def progressive_begin(self, width: int, height: int):

@@ -18,6 +18,7 @@
 
 #include <atomic>
 #include <chrono>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -156,6 +157,7 @@ struct tmpt_scene {
     // and tmpt_denoise(TMPT_HOST); [0] is also the frame of a call that asks for none, and tmpt_render_multi's frame
     DevBuf<char> staged[5];
     DevBuf<float4> d_accum;        // chunk sums of the band being rendered
+    DevBuf<integ::Camera> d_viewCams;  // tmpt_render_views: the batch's cameras
     DevBuf<float4> d_sum;          // progressive render: running per-pixel sums
     int progW = 0, progH = 0, progChunks = -1;  // -1: no progressive render begun
     int progAdaptive = -1;         // the session's kind, fixed by its first pass: -1 none yet, 0 uniform, 1 adaptive
@@ -726,6 +728,10 @@ struct RenderParams {
     unsigned long long* stats;  // instrumented pass only
     const uint2* list;   // LIST kernels (adaptive passes): the band's entries of the active list, {x | y << 16, first chunk n_i}
     int listLen;         // entries in the band
+    // VIEWS kernels (tmpt_render_views): `height` counts the stacked rows of all views; stacked row R is row R % viewHeight of
+    // view R / viewHeight, seen by cams[R / viewHeight] (device memory).  `cam` is not read.
+    const integ::Camera* cams;
+    int viewHeight;
 };
 
 // The 8x4-pixel tile, a warp's pixels in the render kernels and in the adaptive list: lane = (x & 7) + 8 (y & 3), tiles in
@@ -805,8 +811,9 @@ struct WorkItem {
     int chunk;      // the accumulation plane
     int gchunk;     // the chunk of the pixel's samples (progressive passes continue the numbering)
     int spp, len;   // integ::chunk_start's sample range arguments
+    int view, vy;   // VIEWS: the view of stacked row y and the row in it
 };
-template <bool LIST>
+template <bool LIST, bool VIEWS = false>
 __device__ __forceinline__ bool decode_item(const RenderParams& p, uint32_t w, uint32_t lane, WorkItem& it) {
     const uint32_t chunk = w / (uint32_t)p.numTiles, tile = w - chunk * (uint32_t)p.numTiles;
     if (LIST) {
@@ -820,7 +827,12 @@ __device__ __forceinline__ bool decode_item(const RenderParams& p, uint32_t w, u
     it.spp = p.spp; it.len = p.chunkLen;
     tile_pixel(tile, lane, p.tilesX, it.xl, it.rb);
     it.r = p.bandRow0 + it.rb;
-    return it.xl < p.localWidth && it.r < p.ownedRows && local_to_global(it.xl, it.r, p.stripeRows, p.rank, p.world, p.width, it.x, it.y);
+    const bool in = it.xl < p.localWidth && it.r < p.ownedRows && local_to_global(it.xl, it.r, p.stripeRows, p.rank, p.world, p.width, it.x, it.y);
+    if (VIEWS && in) {
+        it.view = it.y / p.viewHeight;
+        it.vy = it.y - it.view * p.viewHeight;
+    }
+    return in;
 }
 
 // The chunk sums of a band (RenderParams::accum): chunk-major float4 planes [plane][bandRows][localWidth], so that a warp's stores
@@ -859,7 +871,9 @@ __device__ __forceinline__ void flush_rays(const RenderParams& p, unsigned long 
 // FAR = the camera stands beyond the scene's far limit (bvh.cuh: ray_is_far): rays are checked and, if far, answered by the
 // exact all-triangle scan.  Only the 256-thread configuration has that instantiation (a camera sixteen scene sizes away sees
 // a few pixels of scene).
-template <bool STATS, int THREADS, int MINB, int SSTACK, bool FAR = false, OutMode MODE = OutMode::Frame>
+// VIEWS = a batch of views (RenderParams::cams): each lane traces its pixel in its own view, with that view's camera, row and
+// height, and stores it at its stacked row (Frame and Aov modes only).
+template <bool STATS, int THREADS, int MINB, int SSTACK, bool FAR = false, OutMode MODE = OutMode::Frame, bool VIEWS = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_render(const RenderParams p) {
     constexpr bool AOV = MODE == OutMode::Aov, LIST = MODE == OutMode::List;
     const int lane = threadIdx.x & 31;
@@ -872,9 +886,12 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render(const RenderParams p) 
         item = __shfl_sync(0xffffffffu, item, 0);
         if (item >= (uint32_t)p.numTiles * (uint32_t)p.chunks) break;
         WorkItem it;
-        if (decode_item<LIST>(p, item, (uint32_t)lane, it)) {
+        if (decode_item<LIST, VIEWS>(p, item, (uint32_t)lane, it)) {
             integ::AovSums aov;
-            const ex::V3 sum = integ::render_chunk<STATS, FAR, AOV>(stack, p.sc, p.cam, it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len, p.lightDir, rays, &ts, &aov);
+            const ex::V3 sum = VIEWS ? integ::render_chunk<STATS, FAR, AOV>(stack, p.sc, p.cams[it.view], it.x, it.vy, it.gchunk, p.width, p.viewHeight, it.spp,
+                                                                          it.len, p.lightDir, rays, &ts, &aov)
+                                     : integ::render_chunk<STATS, FAR, AOV>(stack, p.sc, p.cam, it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len,
+                                                                          p.lightDir, rays, &ts, &aov);
             if (AOV && p.triangle && p.chunk0 + it.chunk == 0) p.triangle[(size_t)it.y * p.width + it.x] = aov.id0;
             store_chunk<MODE>(p, it, sum, &aov);
         }
@@ -1006,7 +1023,9 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_regen(const RenderPara
 // whole tile.  The per-lane arithmetic and its order are those of integ::render_chunk: the frame is byte-identical to k_render's.
 // AOV (as in k_render): the camera ray's hit of each sample is added to nsum / tsum and counted in cl's top byte.
 // LIST (as in k_render): loc holds the list entry.
-template <int THREADS, int MINB, int GATE, OutMode MODE = OutMode::Frame>
+// VIEWS (as in k_render): pix holds the row in the view; the stacked row is bandRow0 + rb, so a views band has fewer than 2^16
+// rows (plan_render).
+template <int THREADS, int MINB, int GATE, OutMode MODE = OutMode::Frame, bool VIEWS = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderParams p) {
     constexpr bool AOV = MODE == OutMode::Aov, LIST = MODE == OutMode::List;
     constexpr unsigned FULL = 0xffffffffu;
@@ -1023,7 +1042,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
     int depth = 0;
     ex::V3 sum = ex::v3(0.0f, 0.0f, 0.0f), o = sum, d = sum, nsum = sum;
     float tsum = 0.0f;
-    const float invW = ex::divf(1.0f, (float)p.width), invH = ex::divf(1.0f, (float)p.height);
+    const float invW = ex::divf(1.0f, (float)p.width), invH = ex::divf(1.0f, (float)(VIEWS ? p.viewHeight : p.height));
     const unsigned long long totalItems = (unsigned long long)p.numTiles * (unsigned long long)p.chunks * 32ull;
     for (;;) {
         // ---- regeneration: lanes without a path get their item's next sample, or a new item
@@ -1034,7 +1053,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             bool wantItem = !havePath && !done && (cl & 0xFFu) == 0u;
             if (wantItem && hasItem) {
                 const int rb = (int)(loc >> 16);
-                const WorkItem it = {(int)(pix & 0xFFFFu), (int)(pix >> 16), (int)(LIST ? loc : loc & 0xFFFFu), rb, p.bandRow0 + rb,
+                const WorkItem it = {(int)(pix & 0xFFFFu), VIEWS ? p.bandRow0 + rb : (int)(pix >> 16), (int)(LIST ? loc : loc & 0xFFFFu), rb, p.bandRow0 + rb,
                                      (int)(AOV ? (cl >> 8) & 0xFFFFu : cl >> 8)};
                 const integ::AovSums aov = {nsum, tsum, (float)(cl >> 24), 0};
                 store_chunk<MODE>(p, it, sum, &aov);
@@ -1053,9 +1072,10 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
                     if (item >= totalItems) { done = true; wantItem = false; }
                     else {
                         WorkItem it;
-                        if (decode_item<LIST>(p, (uint32_t)(item >> 5), (uint32_t)item & 31u, it)) {
+                        if (decode_item<LIST, VIEWS>(p, (uint32_t)(item >> 5), (uint32_t)item & 31u, it)) {
                             int s0, s1;
-                            rng = integ::chunk_start(it.x, it.y, it.gchunk, p.width, p.height, it.spp, it.len, s0, s1);
+                            if (VIEWS) it.y = it.vy;  // (the pixel in its view: the stacked row follows from rb)
+                            rng = integ::chunk_start(it.x, it.y, it.gchunk, p.width, VIEWS ? p.viewHeight : p.height, it.spp, it.len, s0, s1);
                             pix = (uint32_t)it.x | ((uint32_t)it.y << 16);
                             loc = (uint32_t)it.xl | ((uint32_t)it.rb << 16);
                             cl = ((uint32_t)it.chunk << 8) | (uint32_t)(s1 - s0);
@@ -1069,7 +1089,8 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             }
             // (b) the next camera ray of every lane that has an item and no path
             if (!havePath && !done && (cl & 0xFFu) != 0u) {
-                integ::primary_ray(p.cam, (int)(pix & 0xFFFFu), (int)(pix >> 16), invW, invH, rng, o, d);
+                integ::primary_ray(VIEWS ? p.cams[(p.bandRow0 + (int)(loc >> 16)) / p.viewHeight] : p.cam, (int)(pix & 0xFFFFu), (int)(pix >> 16), invW,
+                                   invH, rng, o, d);
                 depth = 0;
                 havePath = true;
             }
@@ -1097,7 +1118,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_render_paths(const RenderPara
             ex::V3 color = ex::v3(0.0f, 0.0f, 0.0f);
             if (AOV && depth == 0) {  // the sample's camera ray (integ::render_chunk's AovSums, in the same order)
                 if (p.triangle && p.chunk0 == 0 && cl == (uint32_t)min(p.chunkLen, p.spp))  // chunk 0's first sample
-                    p.triangle[(size_t)(pix >> 16) * p.width + (pix & 0xFFFFu)] = h.id;
+                    p.triangle[(size_t)(VIEWS ? p.bandRow0 + (int)(loc >> 16) : (int)(pix >> 16)) * p.width + (pix & 0xFFFFu)] = h.id;
                 if (hit) { nsum = ex::add(nsum, normal); tsum = ex::add(tsum, h.t); cl += 1u << 24; }
             }
             if (hit) {
@@ -2018,8 +2039,12 @@ struct RenderPlan {
     int granule;        // bands are multiples of it: 4 rows (a tile row), or 32 list entries (a list tile)
     int units;          // what is banded: owned rows, or the entries of an adaptive pass's active list
     int unitWidth;      // pixels per unit: the local width, or 1
+    int maxBand;        // the most units a band may have, a multiple of the granule
 };
-static RenderPlan plan_render(int localWidth, int ownedRows, int spp, const ProgressivePass* prog, const FrameOutputs* outs, int listLen) {
+// A batch of views (tmpt_render_views) has up to 10^8 stacked rows; k_render_paths packs a band's row into 16 bits.
+constexpr int kMaxViewBandRows = 65536 - kTileH;
+static RenderPlan plan_render(int localWidth, int ownedRows, int spp, const ProgressivePass* prog, const FrameOutputs* outs, int listLen,
+                              bool views = false) {
     RenderPlan pl;
     pl.mode = prog && prog->adaptive ? OutMode::List : outs && outs->aov() ? OutMode::Aov : OutMode::Frame;
     pl.chunks = prog ? prog->nChunks : host_chunk_count(spp);
@@ -2032,17 +2057,18 @@ static RenderPlan plan_render(int localWidth, int ownedRows, int spp, const Prog
     pl.granule = list ? 32 : kTileH;
     pl.units = list ? listLen : ownedRows;
     pl.unitWidth = list ? 1 : localWidth;
+    pl.maxBand = views ? kMaxViewBandRows : INT_MAX;
     return pl;
 }
 
 // The accumulation buffer of a plan: the chunk sums of one band of units, the band sized so that the buffer stays within a fixed
-// budget (a whole 1080p x 64 spp frame, 32 chunks per pixel, is 1.06 GB; the budget is 4 GB).  Allocation happens here so that
-// callers can do it before their timed window starts.
+// budget (a whole 1080p x 64 spp frame, 32 chunks per pixel, is 1.06 GB; the budget is 4 GB) and has at most pl.maxBand units.
+// Allocation happens here so that callers can do it before their timed window starts.
 static int prepare_accum(tmpt_scene* s, const RenderPlan& pl, cudaStream_t st, int* outBandUnits) {
-    int band = pl.units;
+    int band = std::min(pl.units, pl.maxBand);
     if (pl.useAccum && pl.units > 0) {
         const size_t unitBytes = (size_t)pl.unitWidth * pl.chunks * pl.planes * sizeof(float4), budget = (size_t)4 << 30;
-        band = (int)std::min<size_t>((size_t)pl.units, std::max<size_t>(pl.granule, (budget / unitBytes) & ~(size_t)(pl.granule - 1)));
+        band = (int)std::min<size_t>((size_t)band, std::max<size_t>(pl.granule, (budget / unitBytes) & ~(size_t)(pl.granule - 1)));
         const size_t need = (size_t)band * unitBytes;
         CU_TRY(s->d_accum.grow(need / sizeof(float4), st));
     }
@@ -2098,21 +2124,24 @@ struct RenderKernel {
     int threads;
     size_t smem;  // dynamic shared memory: k_render's traversal stacks, kSStack entries x 8 bytes per thread
 };
-template <OutMode MODE>
+template <OutMode MODE, bool VIEWS = false>
 static RenderKernel shipped_render_kernel(bool paths, int cfg, bool far) {
     constexpr size_t b = kSStack * sizeof(unsigned long long);
-    if (paths) return cfg == 3 ? RenderKernel{k_render_paths<1024, 1, 8, MODE>, 1024, 0} : RenderKernel{k_render_paths<256, 4, 8, MODE>, 256, 0};
-    if (far) return {k_render<false, 256, 4, kSStack, true, MODE>, 256, 256 * b};
-    if (cfg == 3) return {k_render<false, 1024, 1, kSStack, false, MODE>, 1024, 1024 * b};
-    if (cfg == 2) return {k_render<false, 512, 2, kSStack, false, MODE>, 512, 512 * b};
-    return {k_render<false, 256, 4, kSStack, false, MODE>, 256, 256 * b};
+    if (paths)
+        return cfg == 3 ? RenderKernel{k_render_paths<1024, 1, 8, MODE, VIEWS>, 1024, 0} : RenderKernel{k_render_paths<256, 4, 8, MODE, VIEWS>, 256, 0};
+    if (far) return {k_render<false, 256, 4, kSStack, true, MODE, VIEWS>, 256, 256 * b};
+    if (cfg == 3) return {k_render<false, 1024, 1, kSStack, false, MODE, VIEWS>, 1024, 1024 * b};
+    if (cfg == 2) return {k_render<false, 512, 2, kSStack, false, MODE, VIEWS>, 512, 512 * b};
+    return {k_render<false, 256, 4, kSStack, false, MODE, VIEWS>, 256, 256 * b};
 }
 // The shipped render instantiation of a launch: k_render_paths (configurations 1 = 256 x 4 and 3 = 1024 x 1) or k_render
 // (1, 2 = 512 x 2, 3, and the far-camera one at 256 x 4) in the launch's output mode, or the instrumented pass (frame mode only;
-// a far camera gets its FAR form too, so that it traces the rays the frame traces and counts the same rays).
-static RenderKernel render_kernel(OutMode mode, bool paths, int cfg, bool far, bool stats) {
+// a far camera gets its FAR form too, so that it traces the rays the frame traces and counts the same rays).  views: the VIEWS
+// forms of the Frame and Aov modes (a batch of views has no instrumented or List form).
+static RenderKernel render_kernel(OutMode mode, bool paths, int cfg, bool far, bool stats, bool views) {
     constexpr size_t sb = 256 * kSStack * sizeof(unsigned long long);
     if (stats) return far ? RenderKernel{k_render<true, 256, 4, kSStack, true>, 256, sb} : RenderKernel{k_render<true, 256, 4, kSStack>, 256, sb};
+    if (views) return mode == OutMode::Aov ? shipped_render_kernel<OutMode::Aov, true>(paths, cfg, far) : shipped_render_kernel<OutMode::Frame, true>(paths, cfg, far);
     switch (mode) {
         case OutMode::Aov: return shipped_render_kernel<OutMode::Aov>(paths, cfg, far);
         case OutMode::List: return shipped_render_kernel<OutMode::List>(paths, cfg, far);
@@ -2129,10 +2158,26 @@ static int render_blocks_per_sm(const RenderKernel& k, int* perSM) {
     return TMPT_OK;
 }
 
+// A batch of views of one size (tmpt_render_views): the frame of a launch is their stacked rows.
+struct ViewBatch {
+    const tmpt_camera* cameras;  // host: camera v sees view v
+    const integ::Camera* dev;    // their device copy (RenderParams::cams)
+    int n, height;               // views, rows per view
+};
+
+// A camera beyond the scene's far limit: its frame needs the FAR instantiations (lens offsets are at most lensRadius from the
+// origin: the test adds it).
+static bool far_camera(const tmpt_scene* s, const tmpt_camera* camera) {
+    return s->view.farLimit > 0.0f &&
+           std::max(std::max(std::fabs(camera->origin[0]), std::fabs(camera->origin[1])), std::fabs(camera->origin[2])) + std::fabs(camera->lensRadius) >
+               0.5f * s->view.farLimit;
+}
+
+// views: `height` is the batch's stacked rows, `camera` its first camera.
 static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int width, int height, int spp, int stripeRows, int rank, int world,
                          uint8_t* outStripes, uint8_t* frame, unsigned long long* rayCountDev, cudaStream_t st,
                          unsigned long long* statsDev = nullptr, const ProgressivePass* prog = nullptr, const FrameOutputs* outs = nullptr,
-                         int listLen = 0) {
+                         int listLen = 0, const ViewBatch* views = nullptr) {
     tmpt_scene* s = const_cast<tmpt_scene*>(cs);  // scratch buffers only; the scene data is immutable
     RenderParams p;
     p.sc = s->view;
@@ -2144,8 +2189,10 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
     p.ownedRows = tmpt_stripe_rows(height, stripeRows, rank, world);
     p.localWidth = tmpt_local_width(width, stripeRows, world);
     p.tilesX = div_up(p.localWidth, kTileW);
-    const RenderPlan pl = plan_render(p.localWidth, p.ownedRows, spp, prog, outs, listLen);
+    const RenderPlan pl = plan_render(p.localWidth, p.ownedRows, spp, prog, outs, listLen, views != nullptr);
     p.spp = pl.spp; p.chunks = pl.chunks; p.chunk0 = pl.chunk0; p.chunkLen = pl.chunkLen; p.useAccum = pl.useAccum ? 1 : 0;
+    p.cams = views ? views->dev : nullptr;
+    p.viewHeight = views ? views->height : height;
     p.radiance = outs ? outs->radiance : nullptr;
     p.normal = outs ? outs->normal : nullptr;
     p.depth = outs ? outs->depth : nullptr;
@@ -2178,12 +2225,13 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         return tmpt::fail(TMPT_ERR_ARG, "render: AOV outputs need the shipped render kernels (no instrumented pass, TMPT_RENDER_KERNEL or tuning configuration)");
     if (pl.mode == OutMode::List && (rk > 0 || (TMPT_TUNE_CFG && cfgEnv >= 4)))
         return tmpt::fail(TMPT_ERR_ARG, "render: adaptive passes need the shipped render kernels (no TMPT_RENDER_KERNEL or tuning configuration)");
-    // (lens offsets are at most lensRadius from the origin: add it to the test)
-    const bool farCamera = s->view.farLimit > 0.0f &&
-        std::max(std::max(std::fabs(camera->origin[0]), std::fabs(camera->origin[1])), std::fabs(camera->origin[2])) + std::fabs(camera->lensRadius) >
-            0.5f * s->view.farLimit;
-    bool usePaths = false;  // (the instrumented pass and far cameras stay with k_render)
-    if (!statsDev && !farCamera && rk == 0 && cfgEnv == 0) TRY(choose_render_kernel(s, camera, p.cam, width, height, st, &usePaths));
+    if (views && (statsDev || prog || rk > 0 || (TMPT_TUNE_CFG && cfgEnv >= 4)))
+        return tmpt::fail(TMPT_ERR_ARG, "render: batches of views need the shipped render kernels (no instrumented pass, passes, TMPT_RENDER_KERNEL or tuning configuration)");
+    bool farCamera = far_camera(s, camera);  // (a batch with one far camera takes the FAR instantiation for all its views)
+    for (int v = 1; views && v < views->n && !farCamera; ++v) farCamera = far_camera(s, &views->cameras[v]);
+    bool usePaths = false;  // (the instrumented pass and far cameras stay with k_render; a batch probes its first view)
+    if (!statsDev && !farCamera && rk == 0 && cfgEnv == 0)
+        TRY(choose_render_kernel(s, camera, p.cam, width, views ? views->height : height, st, &usePaths));
     if (!statsDev) s->lastUsedPaths = usePaths ? 1 : 0;
     int perSM[4] = {-1, -1, -1, -1};  // CTAs per SM of configuration 1..3's kernel, queried when a band first needs it
     for (int b0 = 0; b0 < pl.units; b0 += band) {
@@ -2235,12 +2283,12 @@ static int launch_render(const tmpt_scene* cs, const tmpt_camera* camera, int wi
         {
             int cfg = (statsDev || rk > 0 || farCamera) ? 1 : cfgEnv;
             if (cfg <= 0) {
-                TRY(render_blocks_per_sm(render_kernel(pl.mode, usePaths, 3, false, false), &perSM[3]));
+                TRY(render_blocks_per_sm(render_kernel(pl.mode, usePaths, 3, false, false, views != nullptr), &perSM[3]));
                 cfg = items >= (long long)s->smCount * 32 * 8 && perSM[3] > 0 ? 3 : 1;
             } else if (cfg != 2 && cfg != 3) {
                 cfg = 1;
             }
-            const RenderKernel k = render_kernel(pl.mode, usePaths, cfg, farCamera, statsDev != nullptr);
+            const RenderKernel k = render_kernel(pl.mode, usePaths, cfg, farCamera, statsDev != nullptr, views != nullptr);
             TRY(render_blocks_per_sm(k, &perSM[cfg]));
             if (usePaths) CU_TRY(cudaMemsetAsync(s->d_fetchCounter.p, 0, sizeof(unsigned long long), st));  // one (pixel, chunk) item per lane
             // every SM's resident CTAs, or fewer when a warp per (tile, chunk) item (k_render) or a lane per (pixel, chunk) item
@@ -2324,9 +2372,11 @@ struct Staging {
 
 // One single-GPU frame (prog == nullptr) or progressive pass into the buffers `out` names: with TMPT_HOST each requested buffer is
 // staged in the scene's device scratch and copied out inside the timed window; the kernels always write an RGBA frame (the scene's
-// scratch frame when the caller asks for none).  An adaptive pass reports into *adOut.  The caller holds hostCallMutex and the device.
+// scratch frame when the caller asks for none).  An adaptive pass reports into *adOut.  A batch of views (views != nullptr) is
+// rendered as one frame of its stacked rows (`height`).  The caller holds hostCallMutex and the device.
 static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int height, int spp, int mem, const tmpt_outputs* out,
-                        const ProgressivePass* prog, cudaStream_t st, uint64_t* rayCount, double* seconds, AdaptiveResult* adOut = nullptr) {
+                        const ProgressivePass* prog, cudaStream_t st, uint64_t* rayCount, double* seconds, AdaptiveResult* adOut = nullptr,
+                        const ViewBatch* views = nullptr) {
     const size_t pixels = (size_t)width * height;
     Staging g{{out->rgba, out->radiance, out->normal, out->depth, out->triangle}};
     TRY(g.stage(s, pixels, mem, true, st));
@@ -2339,7 +2389,7 @@ static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int
         samples = s->d_samples.p;
     }
     // (scratch allocation stays outside the timed window; an adaptive pass allocates for a list of every pixel)
-    TRY(prepare_accum(s, plan_render(width, height, spp, prog, &f, (int)pixels), st, nullptr));
+    TRY(prepare_accum(s, plan_render(width, height, spp, prog, &f, (int)pixels, views != nullptr), st, nullptr));
     CU_TRY(cudaEventRecord(s->ev0, st));
     CU_TRY(cudaMemsetAsync(s->d_rayCount.p, 0, sizeof(unsigned long long), st));
     uint32_t listLen = 0;
@@ -2357,7 +2407,8 @@ static int render_frame(tmpt_scene* s, const tmpt_camera* camera, int width, int
         CU_TRY(cudaMemcpyAsync(&listLen, s->d_adTotals.p + nBlocks, sizeof listLen, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
     }
-    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, (uint8_t*)g.dev[0], s->d_rayCount.p, st, nullptr, prog, &f, (int)listLen));
+    TRY(launch_render(s, camera, width, height, spp, height, 0, 1, nullptr, (uint8_t*)g.dev[0], s->d_rayCount.p, st, nullptr, prog, &f, (int)listLen,
+                      views));
     if (ad) LAUNCH(k_adaptive_write, div_up((long long)pixels, 256), 256, 0, st, prog->sum, s->d_adN.p, (long long)pixels, (uchar4*)g.dev[0], f.radiance,
                    samples);
     TRY(g.copy(mem, cudaMemcpyDeviceToHost, st));
@@ -2391,6 +2442,30 @@ extern "C" int tmpt_render(const tmpt_scene* cs, const tmpt_camera* camera, int 
     tmpt_outputs out{};
     out.rgba = rgba;
     return tmpt_render_outputs(cs, camera, width, height, spp, mem, &out, rayCount, seconds, stream);
+}
+
+// A batch of views (beyond the reference): one frame of nViews * height stacked rows, one camera per view (include/tmpt.h).
+constexpr int kMaxViews = 65536;
+constexpr long long kMaxBatchPixels = 100000000;  // the reference's largest single frame, 10000 x 10000
+extern "C" int tmpt_render_views(const tmpt_scene* cs, const tmpt_camera* cameras, int nViews, int width, int height, int spp, int mem,
+                                 const tmpt_outputs* out, uint64_t* rayCount, double* seconds, void* stream) {
+    static const char* fn = "tmpt_render_views";
+    if (!cs || !cameras) return tmpt::fail(TMPT_ERR_ARG, "%s: NULL scene / cameras", fn);
+    if (nViews < 1 || nViews > kMaxViews) return tmpt::fail(TMPT_ERR_ARG, "%s: nViews %d out of range 1..%d", fn, nViews, kMaxViews);
+    TRY(check_render_args(cs, cameras, width, height, spp));
+    if ((long long)nViews * width * height > kMaxBatchPixels)
+        return tmpt::fail(TMPT_ERR_ARG, "%s: %d views of %d x %d are more than %lld pixels", fn, nViews, width, height, kMaxBatchPixels);
+    TRY(check_outputs(fn, out, mem));
+    tmpt_scene* s = const_cast<tmpt_scene*>(cs);  // scratch buffers only; the scene data is immutable
+    std::lock_guard<std::mutex> lock(s->hostCallMutex);
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return tmpt::fail(TMPT_ERR_CUDA, "%s: cudaSetDevice(%d) failed", fn, s->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    CU_TRY(s->d_viewCams.grow((size_t)nViews, st));
+    CU_TRY(cudaMemcpyAsync(s->d_viewCams.p, cameras, (size_t)nViews * sizeof(tmpt_camera), cudaMemcpyHostToDevice, st));
+    const ViewBatch views{cameras, s->d_viewCams.p, nViews, height};
+    TRY(render_frame(s, cameras, width, nViews * height, spp, mem, out, nullptr, st, rayCount, seconds, nullptr, &views));
+    return check_status(s, st);
 }
 
 // Progressive rendering (beyond the reference): the running per-pixel sums live with the scene.
